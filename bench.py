@@ -301,6 +301,11 @@ def main():
     ap.add_argument("--no-msm-sweep", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="headline line only (profiling runs)")
     ap.add_argument("--msm-log2", type=int, default=20)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (verdict, 576-byte GT, this "
+                         "rank's 576-byte partial) to DIR/<name>.npy as float64, one value per byte, so that two builds "
+                         "can be compared output for output; DIR/inputs.json records the seed and the RLC chunk count "
+                         "(pin --chunks when the hosts differ)")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -345,6 +350,7 @@ def main():
     gt = (C.c_uint8 * 576)()
     launches = [0]
     stage_acc = {}
+    last_rc = [None]
 
     def step(src_ptr, n=S, first_=first, total_=total, chunks_=chunks, expect=1):
         # one collective: the 576-byte partial carries the share's verdict too (a flagged share seals it as zero)
@@ -357,6 +363,7 @@ def main():
         else:
             rc = L.blsgpu_finalize_dev(h, C.c_void_p(d_partial.data_ptr()), 1, None, gt)
         launches[0] += L.blsgpu_last_launches(h)
+        last_rc[0] = rc
         assert rc == expect, f"batch verdict {rc}, expected {expect}: {cache.last_error()}"
         ms = (C.c_float * 16)()
         k = L.blsgpu_last_stage_ms(h, ms, 16)
@@ -424,6 +431,18 @@ def main():
         th.start()
     ms_total = timed(resident, args.steps)
     stop.set()
+    if args.dump_outputs and rank == 0:
+        # the batch is the seeded device-generated workload, so with the same arguments and rlc_chunks these are
+        # the same bytes on every run; the GT and the partial are copied before any later call overwrites them
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        dumps = {"verdict": [last_rc[0]], "gt": bytes(gt), "partial": d_partial.cpu().numpy().tobytes()}
+        for name, v in dumps.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), np.array(list(v), dtype=np.float64))
+        # the GT and the partial depend on the RLC chunk count, which defaults to the host's thread count: pass --chunks
+        # to compare dumps taken on different hosts
+        with open(os.path.join(args.dump_outputs, "inputs.json"), "w") as f:
+            json.dump({"seed": SEED, "sets_per_gpu": S, "world": world, "rlc_chunks": chunks, "srb": srb.hex()}, f)
     n_launch = launches[0]
     stages = {k: v / args.steps for k, v in stage_acc.items()}
     e2e_extra = {}

@@ -689,3 +689,71 @@ def batch_verify(sets, srb, chunks=0, scalars=None):
     gtsig = miller_loop(G1_GEN, S) if any_sig else F12_ONE
     out = final_exp(f12_mul(f12_conj(gtsig), gt))
     return out == F12_ONE, f12_to_bytes(out)
+
+
+# ----------------------------------------------------------------------------
+# PublicKey / Signature fromBytes (bls_sig_io.nim:42-122 over blst_p1/p2_uncompress and _deserialize, e1.c / e2.c):
+# returns (BLST_ERROR, affine point in memory layout, all zero on error).
+#   0 SUCCESS, 1 BAD_ENCODING, 2 POINT_NOT_ON_CURVE, 3 POINT_NOT_IN_GROUP, 6 PK_IS_INFINITY
+def _fp_from_be48(b, flags):
+    v = int.from_bytes((bytes([b[0] & 0x1f]) + b[1:48]) if flags else b[:48], "big")
+    return v if v < P else None
+
+
+def _f2_largest(y):
+    return y[1] > (P - 1) // 2 if y[1] else y[0] > (P - 1) // 2
+
+
+def _point_from_bytes(raw, g2):
+    size = 96 if g2 else 48                                   # compressed length
+    b0 = raw[0]
+    if len(raw) == 2 * size and b0 & 0xe0 == 0:               # uncompressed x || y
+        c = [_fp_from_be48(raw[48 * k:48 * k + 48], k == 0) for k in range(len(raw) // 48)]
+        if None in c:
+            return 1, None
+        pt = ((c[1], c[0]), (c[3], c[2])) if g2 else (c[0], c[1])
+        if not (g2_on_curve(pt) if g2 else g1_on_curve(pt)):
+            return 2, None
+        return (3 if not g2 and pt[0] == 0 else 0), pt
+    if b0 & 0x80:
+        if b0 & 0x40:
+            return (0 if b0 & 0x3f == 0 and not any(raw[1:size]) else 1), None
+        if g2:
+            c1, c0 = _fp_from_be48(raw[:48], True), _fp_from_be48(raw[48:96], False)
+            if c1 is None or c0 is None:
+                return 1, None
+            x = (c0, c1)
+            y = f2_sqrt(f2_add(f2_mul(f2_sqr(x), x), B2))
+            if y is None:
+                return 2, None
+            if _f2_largest(y) != bool(b0 & 0x20):
+                y = f2_neg(y)
+            return 0, (x, y)
+        x = _fp_from_be48(raw[:48], True)
+        if x is None:
+            return 1, None
+        y = fp_sqrt((x ** 3 + B1) % P)
+        if y is None:
+            return 2, None
+        if (y > (P - 1) // 2) != bool(b0 & 0x20):
+            y = (P - y) % P
+        return (3 if x == 0 else 0), (x, y)
+    if len(raw) == 2 * size and b0 & 0x40 and b0 & 0x3f == 0 and not any(raw[1:]):
+        return 0, None
+    return 1, None
+
+
+def pubkey_from_bytes(raw, group_check=True):
+    err, pt = _point_from_bytes(raw, False)
+    if err == 0 and pt is None:
+        err = 6
+    if err == 0 and group_check and g1_mul(pt, R_ORDER) is not None:
+        err = 3
+    return err, g1_to_mem(pt if err == 0 else None)
+
+
+def signature_from_bytes(raw, group_check=True):
+    err, pt = _point_from_bytes(raw, True)
+    if err == 0 and group_check and g2_mul(pt, R_ORDER) is not None:
+        err = 3
+    return err, g2_to_mem(pt if err == 0 else None)

@@ -133,9 +133,11 @@ def test_api_mirror(cache, br, srb):
 
 
 @pytest.mark.parametrize("n,chunks", [(10, 0), (10, 4), (3, 8), (257, 16), (1000, 7)])
-def test_rlc_scalars(cache, br, srb, n, chunks):
+def test_rlc_scalars(cache, srb, n, chunks):
+    """Against pyref's restatement of the derivation (pinned to BLST's scalars by tests/test_oracle_golden.py)."""
     import nim_blscurve_b200 as bg
-    assert bg.rlcScalars(cache, srb, n, chunks) == br.rlc_scalars(srb, n, chunks)
+    from oracle import pyref as pr
+    assert bg.rlcScalars(cache, srb, n, chunks) == pr.rlc_scalars(srb, n, chunks)
 
 
 def test_device_generated_sets_verify(cache, br, srb):

@@ -139,3 +139,45 @@ def test_blst_hash_to_g2_rfc_vectors():
         x = tuple(int(t, 16) for t in v["P"]["x"].split(","))
         y = tuple(int(t, 16) for t in v["P"]["y"].split(","))
         assert pr.g2_from_mem(aff) == (x, y)
+
+
+# ---- the stand-in used when oracle/_ref is not built: its stored answers against pyref --------------------------
+def test_replay_table_matches_pyref(monkeypatch):
+    """A sample of every kind of entry in tests/golden/oracle_answers.json.gz, on the inputs the GPU tests make (here
+    rebuilt with pyref instead of the library), recomputed with pyref."""
+    import random
+    from oracle import replay as rp
+    monkeypatch.setattr(rp, "INPUTS_ON_DEVICE", False)
+    srb = hashlib.sha256(b"Mr F was here").digest()
+
+    def same(name, args, ref):
+        assert rp._answer(name, args, None) == ref, name
+    for n, chunks in ((1, 0), (2, 4)):                                   # test_valid_batches
+        sets = rp.make_sets(0, n, b"msg")
+        same("batch_verify", (sets, srb, chunks, None), rp._ref_batch_verify(sets, srb, chunks, None))
+    s1, s2 = rp.make_set(1, b"msg1"), rp.make_set(2, b"msg2")            # test_wrong_signature
+    bad = s1 + s2[:128] + s1[128:]
+    same("batch_verify", (bad, srb, 0, None), rp._ref_batch_verify(bad, srb, 0, None))
+    pts, sc = rp.msm_points(0xFACADE, 3)                                 # test_msm_g1_255[3]
+    same("msm_g1", (pts, sc, 255), rp._ref_msm(pts, sc, 255, False))
+    sets = rp.make_sets(3, 2)                                            # test_msm_g2[2-64]
+    g2 = b"".join(sets[i * 320 + 128:(i + 1) * 320] for i in range(2))
+    rng = random.Random(2 * 1000 + 64)
+    sc2 = b"".join(rng.getrandbits(64).to_bytes(8, "little") for _ in range(2))
+    same("msm_g2", (g2, sc2, 64), rp._ref_msm(g2, sc2, 64, True))
+    dst = pr.DST_ETH2                                                    # test_hash_to_g2_eth2_dst
+    msgs = b"".join(hashlib.sha256(b"m%d" % i).digest() for i in range(300))
+    same("hash_to_g2", (msgs, 32, dst), rp._ref_hash_to_g2(msgs, 32, dst))
+    sets = [rp.make_set(i, b"same message") for i in range(2)]           # test_combine_same_message[2]
+    pks, sigs = b"".join(s[:96] for s in sets), b"".join(s[128:] for s in sets)
+    same("combine", (srb, pks, sigs), rp._ref_combine(srb, pks, sigs))
+    rng = random.Random(1)                                               # test_aggregate_verify[1]
+    m = [bytes(rng.randrange(256) for _ in range(rng.choice([0, 1, 31, 32, 33, 55, 56, 64, 101])))]
+    pk, sig = rp.sign(900, m[0])
+    agg = rp.aggregate_g2(sig)[1]
+    for args in ((pk, m, agg, dst), (bytes(96), m, agg, dst), (pk, m, bytes(192), dst)):
+        same("aggregate_verify", args, rp._ref_aggregate_verify(*args))
+    h = hashlib.sha256(b"sync committee 2").digest()                     # test_fast_aggregate_verify[2]
+    member, aset = rp.fast_aggregate_set(3000, 2, h)
+    for args in ((member, h, aset[128:], dst), (member[:-96], h, aset[128:], dst)):
+        same("fast_aggregate_verify", args, rp._ref_fast_aggregate_verify(*args))
