@@ -13,6 +13,7 @@
 #include "kernels.cuh"
 #include "msm.cuh"
 #include "fpprog.hpp"
+#include "route.hpp"
 
 using namespace bls;
 
@@ -21,6 +22,22 @@ static const char *STAGE_NAMES[ST_COUNT] = {"rlc_scalars", "g2_mul64", "g2_sum",
                                             "miller_lines", "miller_acc", "gt_product", "partial", "final_exp"};
 // Miller-loop tiling: at most LINES_TILE pairs have their 68 x 288-byte line triples resident at once
 static const size_t LINES_TILE = (size_t)1 << 18;
+static_assert(route::ACC_BLOCK == BLS_ACC_BS && ST_ACC == ST_LINES + 1 && ST_GTPROD == ST_LINES + 2 && ST_PARTIAL == ST_LINES + 3,
+              "route.hpp / miller_ws layout");
+
+// Buffers, stream and stage events of one multi-Miller loop (run_miller)
+struct miller_ws {
+    uint32_t *lines = nullptr;    // 68 x 72 words x lines_cap
+    size_t lines_cap = 0;         // pairs per tile
+    fp12 *F = nullptr;            // per-segment block products, nseg rows
+    size_t f_cap = 0;
+    fp12 *F2 = nullptr;           // second-level block products
+    size_t f2_cap = 0;
+    fp12 *seg = nullptr;          // 64 segment products
+    fp *small_lines = nullptr;    // 68 x 6 field elements per pair (small-batch route), allocated on first use
+    cudaStream_t stream = nullptr;
+    cudaEvent_t *ev = nullptr;    // begin/end pairs of miller_lines, miller_acc, gt_product, partial
+};
 
 struct blsgpu_ctx {
     int device = 0;
@@ -34,14 +51,11 @@ struct blsgpu_ctx {
     g2_aff *d_Q = nullptr;
     g1_aff *d_P = nullptr;
     g2_jac *d_S = nullptr;
-    fp12 *d_F = nullptr;          // per-segment block products, nseg rows
-    size_t f_cap = 0;
-    fp12 *d_F2 = nullptr;         // second-level block products
-    size_t f2_cap = 0;
-    fp12 *d_seg = nullptr;        // 64 segment products
+    miller_ws ml;                 // the Miller loop over the batch's pairs: on `stream`, events of ST_LINES..ST_PARTIAL
+    // the one-pair Miller loop of (S, -G1) when it runs on the side stream beside the main loop (run_partial_impl):
+    // buffers allocated on first use, events in ev_scratch
+    miller_ws ml_sig;
     bool acc_team = true;         // six-lane team accumulation (acc_team.cuh) vs one thread per group
-    uint32_t *d_lines = nullptr;  // 68 x 72 words x lines_stride
-    size_t lines_cap = 0;         // pairs per tile
     fp12 *d_partials = nullptr;   // 64 slots
     uint8_t *d_gtb = nullptr;     // 576 canonical GT bytes
     int *d_flags = nullptr;       // [0] pk infinity, [1] is_one
@@ -52,11 +66,7 @@ struct blsgpu_ctx {
     uint8_t *h_pinned = nullptr;  // 4 KiB pinned for small D2H results
     cudaEvent_t ev[2 * ST_COUNT + 5];                        // stage begin/end pairs + fork/join/G1-ready
     bool ev_valid[2 * ST_COUNT + 5];
-    // buffers of the one-pair Miller loop of (S, -G1) when it runs on the side stream beside the big loop (run_partial_impl)
-    uint32_t *sig_lines = nullptr;
-    fp12 *sig_F = nullptr, *sig_F2 = nullptr, *sig_seg = nullptr;
-    fp *sig_small_lines = nullptr;
-    cudaEvent_t ev_scratch[8];                               // event window of the deferred signature-pair Miller loop
+    cudaEvent_t ev_scratch[8];                               // stage events of ml_sig
     bool ev_scratch_valid = false;
     cudaStream_t side2 = nullptr;                            // small batches: [r_i] pk_i beside both the hash and the signature work
     cudaStream_t side = nullptr;                             // the signature-side MSM runs beside the per-set stages
@@ -68,7 +78,6 @@ struct blsgpu_ctx {
     // warp-cooperative tail programs (fpprog.hpp), compiled on first use and kept on the device
     struct dev_prog { uint32_t *d = nullptr; int nslots = 0, nrounds = 0, version = 1; };
     std::map<int, dev_prog> combine_progs, final_progs, norm_progs, set_progs, prod_progs;   // keyed by segment count / partial count
-    fp *d_small_lines = nullptr;                             // 68 x 6 field elements per pair (small-batch route)
     fp *d_small = nullptr;                                   // per-set program inputs/outputs of the small-batch route
     fp *d_norm = nullptr;                                    // [0] Fp norm taken out of the final exponentiation, [1] its inverse
     fp *d_consts = nullptr;                                  // Frobenius coefficients (fpprog::CONST_*)
@@ -81,7 +90,6 @@ struct blsgpu_ctx {
     cudaStream_t copy_stream = nullptr, slice_stream[4] = {nullptr, nullptr, nullptr, nullptr};
     cudaEvent_t ev_copy[4], ev_slice[4];
     bool slices_ready = false;
-    bool chain_hogged = false;                               // the last scalar launch reserved an SM (k_wait_started applies)
     bool chain_smem_raised = false;                          // k_rlc_scalars allowed to reserve a whole SM's shared memory
     // multi-device context (blsgpu_create_multi): this context is the leader (share 0 + the one final exponentiation),
     // peers[k-1] owns share k on its own device; the 576-byte partials and the flags are gathered into the leader
@@ -135,7 +143,7 @@ extern "C" void blsgpu_destroy(blsgpu_ctx *ctx) {
     ctx->peers.clear();
     cudaSetDevice(ctx->device);
     cudaFree(ctx->d_gather); cudaFree(ctx->d_gather_flags); cudaFree(ctx->d_srb);
-    cudaFree(ctx->sig_lines); cudaFree(ctx->sig_F); cudaFree(ctx->sig_F2); cudaFree(ctx->sig_seg); cudaFree(ctx->sig_small_lines);
+    for (miller_ws *w : {&ctx->ml, &ctx->ml_sig}) { cudaFree(w->lines); cudaFree(w->F); cudaFree(w->F2); cudaFree(w->seg); cudaFree(w->small_lines); }
     for (auto &g : ctx->graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
     if (ctx->ev_share) cudaEventDestroy(ctx->ev_share);
     if (ctx->slices_ready) {
@@ -144,14 +152,14 @@ extern "C" void blsgpu_destroy(blsgpu_ctx *ctx) {
     }
     if (ctx->ev_scratch_valid) for (int i = 0; i < 8; i++) cudaEventDestroy(ctx->ev_scratch[i]);
     cudaFree(ctx->d_sets); cudaFree(ctx->d_r); cudaFree(ctx->d_H); cudaFree(ctx->d_Pj); cudaFree(ctx->d_Q);
-    cudaFree(ctx->d_P); cudaFree(ctx->d_S); cudaFree(ctx->d_F); cudaFree(ctx->d_partials); cudaFree(ctx->d_gtb);
+    cudaFree(ctx->d_P); cudaFree(ctx->d_S); cudaFree(ctx->d_partials); cudaFree(ctx->d_gtb);
     cudaFree(ctx->d_flags); cudaFree(ctx->d_dbg); cudaFree(ctx->d_misc); cudaFree(ctx->d_misc2); cudaFree(ctx->d_consts); cudaFree(ctx->d_gt);
     for (auto &kv : ctx->combine_progs) cudaFree(kv.second.d);
     for (auto &kv : ctx->final_progs) cudaFree(kv.second.d);
     for (auto &kv : ctx->norm_progs) cudaFree(kv.second.d);
     for (auto &kv : ctx->set_progs) cudaFree(kv.second.d);
     for (auto &kv : ctx->prod_progs) cudaFree(kv.second.d);
-    cudaFree(ctx->d_norm); cudaFree(ctx->d_small); cudaFree(ctx->d_small_lines); cudaFree(ctx->d_seg); cudaFree(ctx->d_lines); cudaFree(ctx->d_F2);
+    cudaFree(ctx->d_norm); cudaFree(ctx->d_small);
     msm_free(ctx->msm);
     if (ctx->h_pinned) cudaFreeHost(ctx->h_pinned);
     for (int i = 0; i < 2 * ST_COUNT + 5; i++) if (ctx->ev_valid[i]) cudaEventDestroy(ctx->ev[i]);
@@ -180,7 +188,7 @@ extern "C" blsgpu_ctx *blsgpu_create(int device, size_t max_sets) {
     };
     if (e != cudaSuccess) return bad("cudaSetDevice", e);
     if ((e = cudaStreamCreateWithFlags(&ctx->own_stream, cudaStreamNonBlocking)) != cudaSuccess) return bad("cudaStreamCreate", e);
-    ctx->stream = ctx->own_stream;
+    ctx->stream = ctx->ml.stream = ctx->own_stream;
     { int sms = 0; if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) == cudaSuccess && sms > 0) ctx->msm.sms = sms; }
     size_t n = max_sets;
 #define ALLOC(ptr, bytes) if ((e = cudaMalloc((void **)&(ptr), (bytes))) != cudaSuccess) return bad("cudaMalloc " #ptr, e)
@@ -191,14 +199,16 @@ extern "C" blsgpu_ctx *blsgpu_create(int device, size_t max_sets) {
     ALLOC(ctx->d_Q, (n + 1) * sizeof(g2_aff));            // + the signature-side pair
     ALLOC(ctx->d_P, (n + 1) * sizeof(g1_aff));
     ALLOC(ctx->d_S, n * sizeof(g2_jac));
-    ctx->lines_cap = ((n + 1 < LINES_TILE ? n + 1 : LINES_TILE) + 31) & ~(size_t)31;
-    ALLOC(ctx->d_lines, (size_t)ML_NLINES * ML_LINE_WORDS * 4 * ctx->lines_cap);
+    miller_ws &ml = ctx->ml;
+    ml.lines_cap = ((n + 1 < LINES_TILE ? n + 1 : LINES_TILE) + 31) & ~(size_t)31;
+    ALLOC(ml.lines, (size_t)ML_NLINES * ML_LINE_WORDS * 4 * ml.lines_cap);
     // block products: <= 64 segments x (blocks per tile + 1) x tiles
-    ctx->f_cap = (n + 1) / 2 + 40000 + 64 * ((n + 1) / LINES_TILE + 2);   // >= nseg * groups for every miller_shape
-    ALLOC(ctx->d_F, ctx->f_cap * sizeof(fp12));
-    ctx->f2_cap = ctx->f_cap / 8 + 4096;                      // level-1 output of the 8-way product trees (+ padding)
-    ALLOC(ctx->d_F2, ctx->f2_cap * sizeof(fp12));
-    ALLOC(ctx->d_seg, 64 * sizeof(fp12));
+    ml.f_cap = (n + 1) / 2 + 40000 + 64 * ((n + 1) / LINES_TILE + 2);   // >= nseg * groups for every miller_shape
+    ALLOC(ml.F, ml.f_cap * sizeof(fp12));
+    ml.f2_cap = ml.f_cap / 8 + 4096;                          // level-1 output of the 8-way product trees (+ padding)
+    ALLOC(ml.F2, ml.f2_cap * sizeof(fp12));
+    ALLOC(ml.seg, 64 * sizeof(fp12));
+    ml.ev = ctx->ev + 2 * ST_LINES;
     ALLOC(ctx->d_partials, 64 * sizeof(fp12));
     ALLOC(ctx->d_gtb, 576);
     ALLOC(ctx->d_gt, sizeof(fp12));
@@ -234,6 +244,11 @@ extern "C" blsgpu_ctx *blsgpu_create(int device, size_t max_sets) {
     if ((e = cudaEventCreateWithFlags(&ctx->ev_share, cudaEventDisableTiming)) != cudaSuccess) return bad("cudaEventCreate", e);
     for (int i = 0; i < 8; i++) if ((e = cudaEventCreate(&ctx->ev_scratch[i])) != cudaSuccess) return bad("cudaEventCreate", e);
     ctx->ev_scratch_valid = true;
+    ctx->ml_sig.lines_cap = 32;
+    ctx->ml_sig.f_cap = 2048;
+    ctx->ml_sig.f2_cap = 512;
+    ctx->ml_sig.stream = ctx->side;
+    ctx->ml_sig.ev = ctx->ev_scratch;
     return ctx;
 }
 
@@ -273,7 +288,7 @@ extern "C" int blsgpu_device_span(const blsgpu_ctx *ctx) { return ctx ? 1 + (int
 
 extern "C" int blsgpu_set_stream(blsgpu_ctx *ctx, void *cuda_stream) {
     if (!ctx) return BLSGPU_ERR_ARG;
-    ctx->stream = cuda_stream ? (cudaStream_t)cuda_stream : ctx->own_stream;
+    ctx->stream = ctx->ml.stream = cuda_stream ? (cudaStream_t)cuda_stream : ctx->own_stream;
     return 0;
 }
 
@@ -311,36 +326,37 @@ static_assert(fpprog::CONST_COUNT == fpprog_const_count && fpprog::CONST_FROB1 =
 #define EV_SC (2 * ST_COUNT + 3)
 #define EV_HASHED (2 * ST_COUNT + 4)
 
-// scalars for global indices [first, first+n) into d_r
+// the route thresholds, read from the environment once per process (route.hpp)
+static const route::thresholds &thr() {
+    static const route::thresholds t = route::read_thresholds();
+    return t;
+}
+static route::batch_plan batch_plan_of(const blsgpu_ctx *ctx, size_t n, size_t total_n, uint32_t chunks, bool host_src, bool scalars) {
+    return route::plan_batch(thr(), {ctx->use_side, ctx->acc_team, ctx->serial_tail, ctx->use_graph}, n, total_n, chunks, host_src,
+                             scalars);
+}
+
+// scalars for global indices [first, first+n) into d_r; hog: the block of chains reserves an SM (route::chain_hog)
 static int launch_scalars(blsgpu_ctx *ctx, const uint8_t srb[32], size_t n, size_t first, size_t total_n,
-                          uint32_t chunks, const uint64_t *scalars, cudaStream_t s) {
+                          uint32_t chunks, const uint64_t *scalars, bool hog, cudaStream_t s) {
     if (scalars) {
         for (size_t i = 0; i < n; i++) if (scalars[i] == 0) return fail(ctx, BLSGPU_ERR_ARG, "explicit RLC scalar is zero");
         CK(cudaMemcpyAsync(ctx->d_r, scalars, n * 8, cudaMemcpyHostToDevice, s));
         return 0;
     }
     if (!srb) return fail(ctx, BLSGPU_ERR_ARG, "secureRandomBytes is NULL");
-    size_t nb = chunks == 0 ? 1 : (total_n < chunks ? total_n : (size_t)chunks);
-    // Long chains (thousands of sequential SHA-256 blocks per reference chunk) are pure single-warp latency, and every
-    // consumer of the scalars waits for them.  Sharing an SM with the hash kernel's 16 warps costs the chain warp half
-    // of its issue slots (measured: 24-31 ms instead of 13 ms for 8 192 blocks per chain), so a block of chains asks for
-    // the whole shared memory of an SM and therefore gets one to itself: 32 chains per block, one SM per 32 chunks.
-    size_t hog = 0;
-    static const size_t hog_min = getenv("BLSGPU_CHAIN_HOG_MIN") ? (size_t)atoll(getenv("BLSGPU_CHAIN_HOG_MIN")) : 1024;
-    if (total_n / nb >= hog_min) {
-        hog = 227 * 1024;
-        if (!ctx->chain_smem_raised) {
-            CK(cudaFuncSetAttribute(k_rlc_scalars, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hog));
-            ctx->chain_smem_raised = true;
-        }
+    const size_t nb = route::rlc_chains(total_n, chunks);
+    const size_t smem = hog ? 227 * 1024 : 0;
+    if (hog && !ctx->chain_smem_raised) {
+        CK(cudaFuncSetAttribute(k_rlc_scalars, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        ctx->chain_smem_raised = true;
     }
     // d_flags[3]: "the block of chains is resident" (cleared with the other flags at the start of the call)
     volatile int *started = hog && ctx->use_side ? ctx->d_flags + 3 : nullptr;
-    ctx->chain_hogged = started != nullptr;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)nblk(nb, 32));
     cfg.blockDim = dim3(32);
-    cfg.dynamicSmemBytes = hog;
+    cfg.dynamicSmemBytes = smem;
     cfg.stream = s;
     const uint32_t *d_srb = nullptr;
     words8 w8 = words8();
@@ -361,8 +377,9 @@ enum { SETPROG_COFACTOR = 0, SETPROG_G2MUL64 = 1, SETPROG_LINES = 2 };
 
 // Compile (once) and fetch a tail program; kind 0 = combine over `key` segments, 1 = final exponentiation of `key`
 // partials with the Fp inversion supplied in IN1, 2 = the norm that inversion applies to (fpprog.hpp build_final),
-// 3 = per-set G2 program `key` (SETPROG_*), 4 = product tree over `key` Fp12 values
-static int get_prog(blsgpu_ctx *ctx, int kind, int key, blsgpu_ctx::dev_prog &out) {
+// 3 = per-set G2 program `key` (SETPROG_*), 4 = product tree over `key` Fp12 values.  A first use uploads the program
+// on stream st and waits for it.
+static int get_prog(blsgpu_ctx *ctx, int kind, int key, blsgpu_ctx::dev_prog &out, cudaStream_t st) {
     std::map<int, blsgpu_ctx::dev_prog> &cache = kind == 0 ? ctx->combine_progs : (kind == 1 ? ctx->final_progs : (kind == 2 ? ctx->norm_progs : (kind == 3 ? ctx->set_progs : ctx->prod_progs)));
     auto it = cache.find(key);
     if (it != cache.end()) { out = it->second; return 0; }
@@ -385,249 +402,151 @@ static int get_prog(blsgpu_ctx *ctx, int kind, int key, blsgpu_ctx::dev_prog &ou
     dp.version = P.version;
     CK(cudaMalloc((void **)&dp.d, P.words.size() * 4));
     // stream-ordered upload, completed before the host vector goes away (first use only)
-    CK(cudaMemcpyAsync(dp.d, P.words.data(), P.words.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
+    CK(cudaMemcpyAsync(dp.d, P.words.data(), P.words.size() * 4, cudaMemcpyHostToDevice, st));
+    CK(cudaStreamSynchronize(st));
     cache[key] = dp;
     out = dp;
     return 0;
 }
 
-static int launch_prog(blsgpu_ctx *ctx, const blsgpu_ctx::dev_prog &p, const fp *in0, fp *out0, const fp *in1 = nullptr) {
-    size_t smem = (size_t)p.nslots * sizeof(fp);
-    if (smem > 48 * 1024) {
-        // per context, not per process: the attribute belongs to the function on ONE device
-        if (!ctx->prog_smem_raised) {
-            CK(cudaFuncSetAttribute(k_fp_program, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-            CK(cudaFuncSetAttribute(k_fp_program2, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-            ctx->prog_smem_raised = true;
-        }
-    }
-    if (p.version == 2) k_fp_program2<<<1, 32, smem, ctx->stream>>>(p.d, in0, in1, ctx->d_consts, out0, 0, 0, 0);
-    else k_fp_program<<<1, 32, smem, ctx->stream>>>(p.d, in0, in1, ctx->d_consts, out0, 0, 0, 0);
-    ctx->launches++;
-    return 0;
-}
-
-// one warp per instance: n instances of a per-set program on stream st, strides in field elements
-static int launch_prog_many(blsgpu_ctx *ctx, const blsgpu_ctx::dev_prog &p, cudaStream_t st, size_t n, const fp *in0, size_t s_in0,
-                            const fp *in1, size_t s_in1, fp *out0, size_t s_out, bool stream_outputs = false) {
+// one warp per instance: n instances of a program (format 1 or 2, fpprog.hpp) on stream st, strides in field elements
+static void launch_prog_many(blsgpu_ctx *ctx, const blsgpu_ctx::dev_prog &p, cudaStream_t st, size_t n, const fp *in0, size_t s_in0,
+                             const fp *in1, size_t s_in1, fp *out0, size_t s_out, bool stream_outputs = false) {
     const size_t smem = (size_t)p.nslots * sizeof(fp);
-    if (p.version == 2) {
-        if (stream_outputs) k_fp_program2_stream<<<(unsigned)n, 32, smem, st>>>(p.d, in0, in1, ctx->d_consts, out0, s_in0, s_in1, s_out);
-        else k_fp_program2<<<(unsigned)n, 32, smem, st>>>(p.d, in0, in1, ctx->d_consts, out0, s_in0, s_in1, s_out);
-    } else if (stream_outputs)
-        k_fp_program_stream<<<(unsigned)n, 32, smem, st>>>(p.d, in0, in1, ctx->d_consts, out0, s_in0, s_in1, s_out);
-    else
-        k_fp_program<<<(unsigned)n, 32, smem, st>>>(p.d, in0, in1, ctx->d_consts, out0, s_in0, s_in1, s_out);
+    auto k = p.version == 2 ? (stream_outputs ? k_fp_program2_stream : k_fp_program2) : (stream_outputs ? k_fp_program_stream : k_fp_program);
+    k<<<(unsigned)n, 32, smem, st>>>(p.d, in0, in1, ctx->d_consts, out0, s_in0, s_in1, s_out);
     ctx->launches++;
+}
+
+// one warp per (row, group of m columns): rows of `in` (stride in_stride Fp12) -> rows of `out` (stride out_stride)
+static void launch_prog_rows(blsgpu_ctx *ctx, const blsgpu_ctx::dev_prog &p, cudaStream_t st, size_t blocks, const fp12 *in,
+                             fp12 *out, unsigned m, size_t in_stride, size_t out_stride) {
+    auto k = p.version == 2 ? k_fp_program2_rows : k_fp_program_rows;
+    k<<<(unsigned)blocks, 32, (size_t)p.nslots * sizeof(fp), st>>>(p.d, (const fp *)in, ctx->d_consts, (fp *)out, m, in_stride, out_stride);
+    ctx->launches++;
+}
+
+// one instance, which may use up to 64 KiB of shared memory
+static int launch_prog(blsgpu_ctx *ctx, const blsgpu_ctx::dev_prog &p, cudaStream_t st, const fp *in0, fp *out0, const fp *in1 = nullptr) {
+    if ((size_t)p.nslots * sizeof(fp) > 48 * 1024 && !ctx->prog_smem_raised) {
+        // per context, not per process: the attribute belongs to the function on ONE device
+        CK(cudaFuncSetAttribute(k_fp_program, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+        CK(cudaFuncSetAttribute(k_fp_program2, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+        ctx->prog_smem_raised = true;
+    }
+    launch_prog_many(ctx, p, st, 1, in0, 0, in1, 0, out0, 0);
     return 0;
 }
 
-// Largest batches that take the warp-per-set programs: the cofactor / [r]sig programs (5-6 KB of shared memory per
-// warp, 32 warps per SM) up to SMALL_ROUTE_MAX sets, the lines program (33 KB per warp, 6 per SM) up to SMALL_LINES_MAX
-// pairs; beyond that a thread per set fills the machine better (tools/probe.py, profiles/).
-#define SMALL_ROUTE_CAP 4096
-static size_t small_route_max() {
-    static const size_t v = getenv("BLSGPU_SMALL_MAX") ? (size_t)atoll(getenv("BLSGPU_SMALL_MAX")) : 4096;
-    return v > SMALL_ROUTE_CAP ? SMALL_ROUTE_CAP : v;
-}
-static size_t small_lines_max() {
-    static const size_t v = getenv("BLSGPU_SMALL_LINES_MAX") ? (size_t)atoll(getenv("BLSGPU_SMALL_LINES_MAX")) : 1025;
-    return v > 16385 ? 16385 : v;
-}
-#define SMALL_ROUTE_MAX SMALL_ROUTE_CAP   /* buffer strides */
-// Two lanes per set for H(m_i) and the line evaluations (fp2h.cuh).  Introduced for mid-size batches, where a thread per
-// set leaves the machine under-filled; measured again at the end of round 2 (profiles/r2/r2_probe_routes_large.log) it
-// also wins for large ones: a block of lane pairs runs half as long as a block of threads, so the grid ends on a finer
-// wave boundary (81 920 sets: 43.1 -> 36.3 ms, 114 688: 52.6 -> 49.0), and the halved stacks stay in L2.  Lines: lane
-// pairs up to 180 000 pairs; hash: up to 125 000 sets (at 131 072 the thread-per-set hash with its 1.73 waves is the
-// quicker one: 55.0 ms against 55.4 with lane pairs for both and 55.8 with threads for both); beyond, threads.
-static size_t pair_hash_min() { static const size_t v = getenv("BLSGPU_PAIR_HASH_MIN") ? (size_t)atoll(getenv("BLSGPU_PAIR_HASH_MIN")) : 2049; return v; }
-static size_t pair_hash_max() { static const size_t v = getenv("BLSGPU_PAIR_HASH_MAX") ? (size_t)atoll(getenv("BLSGPU_PAIR_HASH_MAX")) : 125000; return v; }
-static size_t pair_lines_max() { static const size_t v = getenv("BLSGPU_PAIR_LINES_MAX") ? (size_t)atoll(getenv("BLSGPU_PAIR_LINES_MAX")) : 180000; return v; }
 #define SMALL_FP_PER_SET (6 + 6 + 6 + 6 + 64)
 
-// Work decomposition of the accumulation: G pairs per group (they share the Fp12 squarings) and nseg loop segments,
-// chosen so that groups x segments gives every SM several warps even for small batches.
-static void miller_shape(size_t np, bool team, int &G, int &nseg) {
-    if (team && np <= 8192) {
-        // Latency regime (the machine is not full).  Measured on B200 (tools/gpu_small_sweep.sh): a team spends ~7.5 us
-        // per (squaring or line) step while all teams are resident (~12k of them), the product over groups is one
-        // block-wide tree (0.59 ms) up to 128 groups and two launches (1.16 ms) beyond (0.084 ms per tree level); up to 64 groups it is a pair of product-tree programs,
-        // one warp per row (0.04-0.08 ms), the segment Horner program costs
-        // 0.22 ms + 7.4 us per segment.
-        double best = 0.0;
-        G = 1; nseg = 32;
-        for (int g = 1; g <= 64; g *= 2)
-            for (int ns = 4; ns <= 32; ns *= 2) {
-                const size_t ngroups = (np + g - 1) / g;
-                if (ngroups * ns > 32768) continue;             // d_F holds at least 40 000 (group, segment) products
-                const double waves = (double)((ngroups * ns + 11999) / 12000);
-                const double acc = waves * (double)((63 + ns - 1) / ns) * (1 + g) * (g <= 16 ? 7.5e-3 : 9.5e-3);
-                int levels = 0;                                 // product trees of eight (k_fp_program_rows), ~0.03 ms a level
-                for (size_t m = ngroups; m > 1; m = (m + 7) / 8) levels++;
-                static const int old_gtp = getenv("BLSGPU_ACC_OLD_RULE") ? atoi(getenv("BLSGPU_ACC_OLD_RULE")) : 0;
-                int depth = 0;
-                while (((size_t)1 << depth) < ngroups) depth++;
-                const double gtp = old_gtp ? (ngroups <= 8 ? 0.04 : (ngroups <= 64 ? 0.08 : (ngroups <= 128 ? 0.084 * depth : 1.16)))
-                                           : 0.01 + 0.03 * levels;
-                const double cost = acc + gtp + 0.22 + 7.4e-3 * ns;
-                if (best == 0.0 || cost < best) { best = cost; G = g; nseg = ns; }
-            }
-    } else if (team) {
-        // Throughput regime.  The Fp12 squarings of a step are shared by the G pairs of a group (work per pair ~ 884 + 756 / G
-        // multiplications), and short segments keep the tail of the grid short: swept on B200 (profiles/r2): 16 384 sets
-        // G = 8 / 16 segments (2.14 -> 1.82 ms), 32 768 and 65 536: G = 16 / 16 (3.79 -> 3.51, 7.08 -> 6.59), 131 072:
-        // G = 24 / 8 (14.3 -> 13.1 ms); past ~65 000 teams the product trees and the segment Horner eat the gain.
-        static const int old_rule = getenv("BLSGPU_ACC_OLD_RULE") ? atoi(getenv("BLSGPU_ACC_OLD_RULE")) : 0;
-        if (old_rule) {
-            G = 1;
-            while (G < 16 && np / (size_t)(2 * G) >= 4096) G *= 2;
-            size_t ngroups = (np + G - 1) / G;
-            size_t want = ((size_t)1 << 15) / ngroups;
-            nseg = want < 1 ? 1 : (want > 32 ? 32 : (int)want);
-        } else {
-            G = np < 24576 ? 8 : (np < 98304 ? 16 : 24);
-            const size_t ngroups = (np + G - 1) / G;
-            nseg = 16;
-            while (nseg > 4 && ngroups * (size_t)nseg > 65536) nseg -= 4;
-        }
-    } else {
-        G = 1;
-        while (G < 8 && np / (size_t)(2 * G) >= 8192) G *= 2;
-        size_t ngroups = (np + G - 1) / G;
-        size_t want = ((size_t)1 << 17) / ngroups;
-        nseg = want < 1 ? 1 : (want > 32 ? 32 : (int)want);
-    }
-    if (const char *e = getenv("BLSGPU_MILLER_G")) G = atoi(e);
-    if (const char *e = getenv("BLSGPU_MILLER_NSEG")) nseg = atoi(e);
-    if (G < 1) G = 1;
-    if (nseg < 1) nseg = 1;
-    if (nseg > 63) nseg = 63;
-}
-
-// Multi-Miller loop over the np pairs (d_Q[pair0 + i], d_P[pair0 + i]) + reductions; leaves conj(prod ML) in d_partials[slot]
-static int run_miller(blsgpu_ctx *ctx, size_t np, int slot, size_t pair0 = 0) {
-    cudaStream_t s = ctx->stream;
+// Multi-Miller loop over the np pairs (d_Q[pair0 + i], d_P[pair0 + i]) + reductions, on the buffers, stream and stage
+// events of workspace ws; leaves conj(prod ML) in d_partials[slot]
+static int run_miller(blsgpu_ctx *ctx, miller_ws &ws, size_t np, int slot, size_t pair0 = 0) {
+#define WBEGIN(stage) CK(cudaEventRecord(ws.ev[2 * ((stage) - ST_LINES)], s))
+#define WEND(stage) CK(cudaEventRecord(ws.ev[2 * ((stage) - ST_LINES) + 1], s))
+    cudaStream_t s = ws.stream;
     int rc;
     // tile by tile: lines, then per-(group, segment) accumulation
     const bool team = ctx->acc_team;
-    int G, nseg;
-    miller_shape(np < ctx->lines_cap ? np : ctx->lines_cap, team, G, nseg);
-    size_t ncols = 0;                                       // entries per segment row of d_F
-    for (size_t off = 0; off < np; off += ctx->lines_cap) {
-        size_t t = np - off < ctx->lines_cap ? np - off : ctx->lines_cap;
-        size_t ngroups = (t + G - 1) / G;
-        ncols += team ? ngroups : (ngroups + BLS_ACC_BS - 1) / BLS_ACC_BS;
-    }
+    const route::miller_plan mp = route::plan_miller(thr(), np, ws.lines_cap, team, ctx->serial_tail);
+    const int G = mp.G, nseg = mp.nseg;
+    const size_t ncols = mp.ncols;                          // entries per segment row of F
     // small batches: the GT product of each segment row runs as product-tree programs over groups of 8 columns, so
-    // the rows of d_F are padded to a multiple of 8 with ones
-    static const int gt_env = getenv("BLSGPU_SMALL_ROUTE") ? atoi(getenv("BLSGPU_SMALL_ROUTE")) : 15;   // bit 3: GT product
-    static const size_t gt_prog_max = getenv("BLSGPU_GT_PROG_MAX") ? (size_t)atoll(getenv("BLSGPU_GT_PROG_MAX")) : ((size_t)1 << 20);
-    const bool gt_prog = (gt_env & 8) && team && np <= ctx->lines_cap && ncols <= gt_prog_max && !ctx->serial_tail;
-    const size_t row_stride = gt_prog && ncols > 8 ? ((ncols + 7) & ~(size_t)7) : ncols;
-    const size_t ncols2 = gt_prog ? ((((ncols + 7) / 8) + 7) & ~(size_t)7) : (ncols + BLS_ACC_BS - 1) / BLS_ACC_BS;
-    if ((size_t)nseg * row_stride > ctx->f_cap || (size_t)nseg * ncols2 > ctx->f2_cap)
+    // the rows of F are padded to a multiple of 8 with ones
+    const size_t row_stride = mp.gt_prog && ncols > 8 ? ((ncols + 7) & ~(size_t)7) : ncols;
+    const size_t ncols2 = mp.gt_prog ? ((((ncols + 7) / 8) + 7) & ~(size_t)7) : (ncols + BLS_ACC_BS - 1) / BLS_ACC_BS;
+    if ((size_t)nseg * row_stride > ws.f_cap || (size_t)nseg * ncols2 > ws.f2_cap)
         return fail(ctx, BLSGPU_ERR_CAPACITY, "segment product buffer too small");
     size_t col = 0;
-    BEGIN(ST_LINES, s);
-    bool single = np <= ctx->lines_cap;
-    for (size_t off = 0; off < np; off += ctx->lines_cap) {
-        size_t t = np - off < ctx->lines_cap ? np - off : ctx->lines_cap;
-        size_t stride = ctx->lines_cap;
-        static const int small_env = getenv("BLSGPU_SMALL_ROUTE") ? atoi(getenv("BLSGPU_SMALL_ROUTE")) : 15;   // bit 2: lines
-        if ((small_env & 4) && single && np <= small_lines_max() && !ctx->serial_tail) {
-            // one warp per pair runs the 68 line evaluations as a dataflow program (two multiplication levels per
-            // tangent instead of ~20 dependent products), then a scatter into the accumulation's layout
+    WBEGIN(ST_LINES);
+    bool single = np <= ws.lines_cap;
+    for (size_t off = 0; off < np; off += ws.lines_cap) {
+        size_t t = np - off < ws.lines_cap ? np - off : ws.lines_cap;
+        size_t stride = ws.lines_cap;
+        const int lines = off + t < np ? mp.lines : mp.lines_last;
+        if (lines == route::LINES_PROGRAM) {
+            // one warp per pair runs the 68 line evaluations as a dataflow program, then a scatter into the
+            // accumulation's layout
             blsgpu_ctx::dev_prog lp;
-            rc = get_prog(ctx, 3, SETPROG_LINES, lp);
+            rc = get_prog(ctx, 3, SETPROG_LINES, lp, s);
             if (rc) return rc;
             const size_t per = (size_t)ML_NLINES * 6;
-            if (!ctx->d_small_lines) CK(cudaMalloc((void **)&ctx->d_small_lines, small_lines_max() * per * sizeof(fp)));
-            launch_prog_many(ctx, lp, s, t, (const fp *)(ctx->d_Q + pair0), 4, (const fp *)(ctx->d_P + pair0), 2, ctx->d_small_lines, per, true);
-            k_lines_from_prog<<<nblk(t * ML_NLINES * ML_LINE_WORDS, 256), 256, 0, s>>>((const uint32_t *)ctx->d_small_lines, ctx->d_Q + pair0, ctx->d_P + pair0, t,
-                                                                                      ctx->d_lines, stride);
+            if (!ws.small_lines) CK(cudaMalloc((void **)&ws.small_lines, thr().small_lines_max * per * sizeof(fp)));
+            launch_prog_many(ctx, lp, s, t, (const fp *)(ctx->d_Q + pair0), 4, (const fp *)(ctx->d_P + pair0), 2, ws.small_lines, per, true);
+            k_lines_from_prog<<<nblk(t * ML_NLINES * ML_LINE_WORDS, 256), 256, 0, s>>>((const uint32_t *)ws.small_lines, ctx->d_Q + pair0, ctx->d_P + pair0, t,
+                                                                                      ws.lines, stride);
             ctx->launches++;
-        } else if (t <= pair_lines_max()) {
-            k_miller_lines_lanes2<<<nblk(2 * t), 128, 0, s>>>(ctx->d_Q + pair0 + off, ctx->d_P + pair0 + off, t, ctx->d_lines, stride);
+        } else if (lines == route::LINES_LANES2) {
+            k_miller_lines_lanes2<<<nblk(2 * t), 128, 0, s>>>(ctx->d_Q + pair0 + off, ctx->d_P + pair0 + off, t, ws.lines, stride);
         } else {
-            k_miller_lines<<<nblk(t), 128, 0, s>>>(ctx->d_Q + pair0 + off, ctx->d_P + pair0 + off, t, ctx->d_lines, stride);
+            k_miller_lines<<<nblk(t), 128, 0, s>>>(ctx->d_Q + pair0 + off, ctx->d_P + pair0 + off, t, ws.lines, stride);
         }
-        if (single) { END(ST_LINES, s); BEGIN(ST_ACC, s); }
+        if (single) { WEND(ST_LINES); WBEGIN(ST_ACC); }
         size_t ngroups = (t + G - 1) / G;
         if (team) {
             dim3 grid(nblk(ngroups, ACC_TPB), nseg);
-            k_miller_acc_team<<<grid, ACC_BS, 0, s>>>(ctx->d_lines, stride, t, ngroups, G, nseg, ctx->d_F, row_stride, col);
+            k_miller_acc_team<<<grid, ACC_BS, 0, s>>>(ws.lines, stride, t, ngroups, G, nseg, ws.F, row_stride, col);
             col += ngroups;
         } else {
             dim3 grid(nblk(ngroups, BLS_ACC_BS), nseg);
-            k_miller_acc<<<grid, BLS_ACC_BS, 0, s>>>(ctx->d_lines, stride, t, ngroups, G, nseg, ctx->d_F, ncols, col);
+            k_miller_acc<<<grid, BLS_ACC_BS, 0, s>>>(ws.lines, stride, t, ngroups, G, nseg, ws.F, ncols, col);
             col += grid.x;
         }
         ctx->launches += 2;
     }
-    if (!single) { END(ST_LINES, s); BEGIN(ST_ACC, s); }    // multi-tile: lines+acc are reported together under miller_lines
-    END(ST_ACC, s);
-    BEGIN(ST_GTPROD, s);
+    if (!single) { WEND(ST_LINES); WBEGIN(ST_ACC); }        // multi-tile: lines+acc are reported together under miller_lines
+    WEND(ST_ACC);
+    WBEGIN(ST_GTPROD);
     if (ncols == 1) {                                       // one group: the segment values are the products already
-        CK(cudaMemcpy2DAsync(ctx->d_seg, sizeof(fp12), ctx->d_F, row_stride * sizeof(fp12), sizeof(fp12), (size_t)nseg,
+        CK(cudaMemcpy2DAsync(ws.seg, sizeof(fp12), ws.F, row_stride * sizeof(fp12), sizeof(fp12), (size_t)nseg,
                              cudaMemcpyDeviceToDevice, s));
-    } else if (gt_prog) {
+    } else if (mp.gt_prog) {
         // product trees of eight as dataflow programs, one warp per (segment row, group of 8 columns), level after level
-        // (the 54 multiplications of a tree node spread over the 32 lanes); the rows ping-pong between d_F and d_F2 and
+        // (the 54 multiplications of a tree node spread over the 32 lanes); the rows ping-pong between F and F2 and
         // every level's rows are padded with ones to a multiple of 8
         blsgpu_ctx::dev_prog p8, pm;
-        fp12 *cur = ctx->d_F, *other = ctx->d_F2;
+        fp12 *cur = ws.F, *other = ws.F2;
         size_t cols = ncols, stride = row_stride;
         while (cols > 8) {
             const size_t m = (cols + 7) / 8, m_stride = m > 8 ? ((m + 7) & ~(size_t)7) : m;
-            rc = get_prog(ctx, 4, 8, p8);
+            rc = get_prog(ctx, 4, 8, p8, s);
             if (rc) return rc;
             if (cols & 7) { k_fp12_pad_one<<<nseg, 32, 0, s>>>(cur, stride, cols); ctx->launches++; }
-            if (p8.version == 2)
-                k_fp_program2_rows<<<(unsigned)((size_t)nseg * m), 32, (size_t)p8.nslots * sizeof(fp), s>>>(
-                    p8.d, (const fp *)cur, ctx->d_consts, (fp *)other, (unsigned)m, stride, m_stride);
-            else
-                k_fp_program_rows<<<(unsigned)((size_t)nseg * m), 32, (size_t)p8.nslots * sizeof(fp), s>>>(
-                    p8.d, (const fp *)cur, ctx->d_consts, (fp *)other, (unsigned)m, stride, m_stride);
-            ctx->launches++;
+            launch_prog_rows(ctx, p8, s, (size_t)nseg * m, cur, other, (unsigned)m, stride, m_stride);
             fp12 *t = cur; cur = other; other = t;
             cols = m;
             stride = m_stride;
         }
-        rc = get_prog(ctx, 4, (int)cols, pm);
+        rc = get_prog(ctx, 4, (int)cols, pm, s);
         if (rc) return rc;
-        if (pm.version == 2)
-            k_fp_program2_rows<<<(unsigned)nseg, 32, (size_t)pm.nslots * sizeof(fp), s>>>(pm.d, (const fp *)cur, ctx->d_consts,
-                                                                                         (fp *)ctx->d_seg, 1u, stride, 1);
-        else
-            k_fp_program_rows<<<(unsigned)nseg, 32, (size_t)pm.nslots * sizeof(fp), s>>>(pm.d, (const fp *)cur, ctx->d_consts,
-                                                                                        (fp *)ctx->d_seg, 1u, stride, 1);
-        ctx->launches++;
+        launch_prog_rows(ctx, pm, s, (size_t)nseg, cur, ws.seg, 1u, stride, 1);
     } else if (ncols > BLS_ACC_BS) {
         dim3 grid((unsigned)ncols2, nseg);
-        k_fp12_rows_step<<<grid, BLS_ACC_BS, 0, s>>>(ctx->d_F, ncols, ncols, ctx->d_F2, ncols2);
-        k_fp12_rows<<<nseg, BLS_ACC_BS, 0, s>>>(ctx->d_F2, ncols2, ncols2, ctx->d_seg);
+        k_fp12_rows_step<<<grid, BLS_ACC_BS, 0, s>>>(ws.F, ncols, ncols, ws.F2, ncols2);
+        k_fp12_rows<<<nseg, BLS_ACC_BS, 0, s>>>(ws.F2, ncols2, ncols2, ws.seg);
         ctx->launches++;
     } else {
-        k_fp12_rows<<<nseg, BLS_ACC_BS, 0, s>>>(ctx->d_F, ncols, ncols, ctx->d_seg);
+        k_fp12_rows<<<nseg, BLS_ACC_BS, 0, s>>>(ws.F, ncols, ncols, ws.seg);
     }
-    END(ST_GTPROD, s);
-    BEGIN(ST_PARTIAL, s);
+    WEND(ST_GTPROD);
+    WBEGIN(ST_PARTIAL);
     ctx->launches++;
     if (ctx->serial_tail) {
-        k_combine<<<1, 32, 0, s>>>(ctx->d_seg, nseg, ctx->d_partials + slot);
+        k_combine<<<1, 32, 0, s>>>(ws.seg, nseg, ctx->d_partials + slot);
         ctx->launches++;
     } else {
         blsgpu_ctx::dev_prog cp;
-        rc = get_prog(ctx, 0, nseg, cp);
+        rc = get_prog(ctx, 0, nseg, cp, s);
         if (rc) return rc;
-        rc = launch_prog(ctx, cp, (const fp *)ctx->d_seg, (fp *)(ctx->d_partials + slot));
+        rc = launch_prog(ctx, cp, s, (const fp *)ws.seg, (fp *)(ctx->d_partials + slot));
         if (rc) return rc;
     }
-    END(ST_PARTIAL, s);
+    WEND(ST_PARTIAL);
     CK(cudaGetLastError());
     return 0;
+#undef WBEGIN
+#undef WEND
 }
 
 static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, size_t first, size_t total_n,
@@ -663,13 +582,13 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
     cudaStream_t s = ctx->stream;
     ctx->launches = 0;
     if (!scalars && !srb) return fail(ctx, BLSGPU_ERR_ARG, "secureRandomBytes is NULL");
+    const route::batch_plan plan = batch_plan_of(ctx, n, total_n, chunks, ctx->h_src != nullptr, scalars != nullptr);
     // Host-buffer call (blsgpu_batch_verify): this function issues the H2D copy itself.  Small and mid-size batches: one
     // copy ahead of everything.  Large ones: H2D_SLICES pieces on a copy stream, each followed at once by the launch of
     // the hash kernel over that piece on its own stream, so the copy (and, for pageable memory, the host-side staging
     // that blocks the calling thread piece by piece) hides behind H(m_i) of the earlier pieces.
     enum { H2D_SLICES = 4 };
-    static const size_t slice_min = getenv("BLSGPU_H2D_SLICE_MIN") ? (size_t)atoll(getenv("BLSGPU_H2D_SLICE_MIN")) : 32768;
-    const bool sliced = ctx->h_src && (const void *)d_sets == (const void *)ctx->d_sets && n >= slice_min && n > small_route_max();
+    const bool sliced = plan.sliced;
     if (ctx->h_src && !sliced) CK(cudaMemcpyAsync(ctx->d_sets, ctx->h_src, n * sizeof(sigset), cudaMemcpyHostToDevice, s));
     if (sliced && !ctx->slices_ready) {
         CK(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
@@ -691,15 +610,14 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
         CK(cudaStreamWaitEvent(g, ctx->ev[EV_FORK], 0));
     }
     BEGIN(ST_SCALARS, cs);
-    int rc = launch_scalars(ctx, srb, n, first, total_n, chunks, scalars, cs);
+    int rc = launch_scalars(ctx, srb, n, first, total_n, chunks, scalars, plan.chain_hog, cs);
     if (rc) return rc;
     END(ST_SCALARS, cs);
     if (ctx->use_side) {
         CK(cudaEventRecord(ctx->ev[EV_SC], cs));
         CK(cudaStreamWaitEvent(g, ctx->ev[EV_SC], 0));
     }
-    static const int chain_wait = getenv("BLSGPU_CHAIN_WAIT") ? atoi(getenv("BLSGPU_CHAIN_WAIT")) : 1;
-    if (chain_wait && ctx->chain_hogged && !scalars) {
+    if (plan.chain_wait) {
         // the main stream (whose next kernel fills the machine) waits until the chains' block is placed: ~10 us when the
         // device is idle, at most 0.2 ms (400 000 cycles) when it is not
         k_wait_started<<<1, 32, 0, s>>>(ctx->d_flags + 3, 400000, ctx->d_dbg);
@@ -707,22 +625,18 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
     }
     // Small-batch route: the serial stretches of a set (cofactor clearing, [r_i] sig_i) run as per-set dataflow
     // programs, one warp per set (fpprog.hpp build_g2_clear_cofactor / build_g2_mul64)
-    static const int small_env = getenv("BLSGPU_SMALL_ROUTE") ? atoi(getenv("BLSGPU_SMALL_ROUTE")) : 15;   // bit 0 hash, bit 1 sig (bit 2: lines, bit 3: GT product, run_miller)
-    const bool small = small_env != 0 && n <= small_route_max() && !ctx->serial_tail;
-    const bool pair_hash = n >= pair_hash_min() && n <= pair_hash_max();
-    const bool small_hash = small && (small_env & 1) && !pair_hash, small_sig = small && (small_env & 2);
     blsgpu_ctx::dev_prog p_cof, p_mul;
     fp *sm_hash_in = nullptr, *sm_hash_out = nullptr, *sm_sig_in = nullptr, *sm_sig_out = nullptr, *sm_bits = nullptr;
-    if (small) {
-        if (!ctx->d_small) CK(cudaMalloc((void **)&ctx->d_small, (size_t)SMALL_ROUTE_MAX * SMALL_FP_PER_SET * sizeof(fp)));
-        rc = get_prog(ctx, 3, SETPROG_COFACTOR, p_cof);
-        if (!rc) rc = get_prog(ctx, 3, SETPROG_G2MUL64, p_mul);
+    if (plan.small) {
+        if (!ctx->d_small) CK(cudaMalloc((void **)&ctx->d_small, route::SMALL_ROUTE_CAP * SMALL_FP_PER_SET * sizeof(fp)));
+        rc = get_prog(ctx, 3, SETPROG_COFACTOR, p_cof, s);
+        if (!rc) rc = get_prog(ctx, 3, SETPROG_G2MUL64, p_mul, s);
         if (rc) return rc;
         sm_hash_in = ctx->d_small;
-        sm_hash_out = sm_hash_in + 6 * SMALL_ROUTE_MAX;
-        sm_sig_in = sm_hash_out + 6 * SMALL_ROUTE_MAX;
-        sm_sig_out = sm_sig_in + 6 * SMALL_ROUTE_MAX;
-        sm_bits = sm_sig_out + 6 * SMALL_ROUTE_MAX;
+        sm_hash_out = sm_hash_in + 6 * route::SMALL_ROUTE_CAP;
+        sm_sig_in = sm_hash_out + 6 * route::SMALL_ROUTE_CAP;
+        sm_sig_out = sm_sig_in + 6 * route::SMALL_ROUTE_CAP;
+        sm_bits = sm_sig_out + 6 * route::SMALL_ROUTE_CAP;
     }
     if (sliced) {
         if (!ctx->use_side) CK(cudaEventRecord(ctx->ev[EV_FORK], s));
@@ -738,7 +652,7 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
             CK(cudaEventRecord(ctx->ev_copy[k], ctx->copy_stream));
             cudaStream_t sk = ctx->slice_stream[k];
             CK(cudaStreamWaitEvent(sk, ctx->ev_copy[k], 0));
-            if (pair_hash) k_hash_sets_lanes2<<<nblk(2 * len), 128, 0, sk>>>(d_sets + off, len, ctx->d_H + off);
+            if (plan.hash == route::HASH_LANES2) k_hash_sets_lanes2<<<nblk(2 * len), 128, 0, sk>>>(d_sets + off, len, ctx->d_H + off);
             else k_hash_sets<<<nblk(len), 128, 0, sk>>>(d_sets + off, len, ctx->d_H + off);
             ctx->launches++;
             CK(cudaEventRecord(ctx->ev_slice[k], sk));
@@ -747,16 +661,7 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
         END(ST_HASH, s);
         CK(cudaStreamWaitEvent(g, ctx->ev_copy[H2D_SLICES - 1], 0));    // the signature-side MSM reads every set
     }
-    // Small batches are latency chains (one thread per set): [r_i]pk_i does not depend on H(m_i), so it leads the
-    // second stream instead of queueing behind the hash kernel.  Large batches: behind a scalar chain of several
-    // milliseconds it starts while the hash kernel is in its last wave and fills the slots that wave leaves empty.
-    // measured (profiles/r2): beside the hash up to 8 192 sets (4 096 sets: 7.4 -> 6.7 ms) and from 36 000 on (49 152:
-    // 25.5 -> 24.1 ms, 65 536: 31.7 -> 30.3, 98 304: 45.8 -> 43.8, 131 072: 56.2 -> 55.9); between, the chain is short,
-    // the two run side by side from the start and contend (9 000 sets: 8.4 -> 9.1 ms)
-    static const size_t g1_aside_max = getenv("BLSGPU_G1_ASIDE_MAX") ? (size_t)atoll(getenv("BLSGPU_G1_ASIDE_MAX")) : 8192;
-    static const size_t g1_aside_large = getenv("BLSGPU_G1_ASIDE_LARGE_MIN") ? (size_t)atoll(getenv("BLSGPU_G1_ASIDE_LARGE_MIN")) : 36000;
-    const bool g1_aside = ctx->use_side && (n <= g1_aside_max || n >= g1_aside_large);
-    if (g1_aside) {
+    if (plan.g1_aside) {
         cudaStream_t g1s = ctx->side2;
         CK(cudaStreamWaitEvent(g1s, ctx->ev[EV_SC], 0));
         if (sliced) CK(cudaStreamWaitEvent(g1s, ctx->ev_copy[H2D_SLICES - 1], 0));   // the keys of every slice are in place
@@ -769,36 +674,27 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
     auto launch_hash = [&]() -> int {
         if (sliced) return 0;
         BEGIN(ST_HASH, s);
-        if (small_hash) {
-            static const int map2 = getenv("BLSGPU_MAP_LANES2") ? atoi(getenv("BLSGPU_MAP_LANES2")) : 1;
-            if (map2) k_hash_map_lanes2<<<nblk(2 * n, 64), 64, 0, s>>>(d_sets, nullptr, nullptr, nullptr, 0, n, sm_hash_in);
+        if (plan.hash == route::HASH_PROGRAM) {
+            if (thr().map_lanes2) k_hash_map_lanes2<<<nblk(2 * n, 64), 64, 0, s>>>(d_sets, nullptr, nullptr, nullptr, 0, n, sm_hash_in);
             else k_hash_map_pair<<<nblk(2 * n), 128, 0, s>>>(d_sets, n, sm_hash_in);
             launch_prog_many(ctx, p_cof, s, n, sm_hash_in, 6, nullptr, 0, sm_hash_out, 6);
             k_g2_hom_to_jac<<<nblk(n), 128, 0, s>>>(sm_hash_out, n, ctx->d_H);
             ctx->launches += 2;
-        } else if (pair_hash) k_hash_sets_lanes2<<<nblk(2 * n), 128, 0, s>>>(d_sets, n, ctx->d_H);
-        else if (n <= 8192) k_hash_sets_pair<<<nblk(2 * n), 128, 0, s>>>(d_sets, n, ctx->d_H);
+        } else if (plan.hash == route::HASH_LANES2) k_hash_sets_lanes2<<<nblk(2 * n), 128, 0, s>>>(d_sets, n, ctx->d_H);
+        else if (plan.hash == route::HASH_PAIR) k_hash_sets_pair<<<nblk(2 * n), 128, 0, s>>>(d_sets, n, ctx->d_H);
         else k_hash_sets<<<nblk(n), 128, 0, s>>>(d_sets, n, ctx->d_H);
         END(ST_HASH, s);
         return 0;
     };
-    // BLSGPU_MSM_AFTER_HASH_MIN (off by default): the signature-side MSM waits for the hash kernel and runs beside
-    // [r_i]pk_i and the line evaluations instead.  Measured at 131 072 sets: hash 26.1 -> 24.0 ms (its time alone), [r_i]pk_i
-    // +0.9, lines +1.3, step 57.3 -> 57.1 ms whatever the length of the scalar chain — but the starved MSM then ends only
-    // 1-2 ms before the join, so the gain is not worth the exposure.
-    static const size_t msm_after_hash_min = getenv("BLSGPU_MSM_AFTER_HASH_MIN") ? (size_t)atoll(getenv("BLSGPU_MSM_AFTER_HASH_MIN")) : ~(size_t)0;
-    const bool msm_after_hash = ctx->use_side && n >= msm_after_hash_min;
-    if (msm_after_hash) {
+    if (plan.msm_after_hash) {
         rc = launch_hash();
         if (rc) return rc;
         CK(cudaEventRecord(ctx->ev[EV_HASHED], s));
         CK(cudaStreamWaitEvent(g, ctx->ev[EV_HASHED], 0));
     }
     BEGIN(ST_G2MUL, g);
-    // S = sum_i [r_i] sig_i : Pippenger over the signatures in place (stride 320) for batches that can fill the
-    // buckets, n independent 64-bit multiplications + tree below that
-    static const size_t g2_msm_min = getenv("BLSGPU_G2_MSM_MIN") ? (size_t)atoll(getenv("BLSGPU_G2_MSM_MIN")) : 2500;   // swept: 2 048 sets 6.54 -> 6.13 ms with the per-set programs, 2 600: 6.39 -> 6.33 with the MSM
-    if (n >= g2_msm_min) {
+    // S = sum_i [r_i] sig_i
+    if (plan.sig == route::SIG_MSM) {
         std::string err;
         rc = msm_run<fp2>(ctx->msm, (const uint8_t *)d_sets + offsetof(sigset, sig), sizeof(sigset), (const uint8_t *)ctx->d_r, 8,
                           n, 64, g, ctx->d_S, nullptr, &ctx->launches, err);
@@ -806,7 +702,7 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
         END(ST_G2MUL, g);
         BEGIN(ST_G2SUM, g);
     } else {
-        if (small_sig) {
+        if (plan.sig == route::SIG_PROGRAM) {
             k_g2_mul_prep<<<nblk(64 * n), 128, 0, g>>>(d_sets, ctx->d_r, n, sm_sig_in, sm_bits);
             launch_prog_many(ctx, p_mul, g, n, sm_sig_in, 6, sm_bits, 64, sm_sig_out, 6);
             k_g2_hom_to_jac<<<nblk(n), 128, 0, g>>>(sm_sig_out, n, ctx->d_S);
@@ -827,48 +723,27 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
     k_sig_pair<<<1, 32, 0, g>>>(ctx->d_S, n, ctx->d_Q, ctx->d_P);
     ctx->launches++;
     END(ST_G2SUM, g);
-    // From 4 500 sets on the n set pairs do not wait for the signature sum (scalar chain, then the signature-side MSM: 4 ms
-    // at 8 192 sets, tens of milliseconds behind the long chains of a large batch).  Pair number n = (S, -G1) gets its own
-    // one-pair Miller loop right here on the side stream, with buffers of its own, beside the big loop of the main stream;
-    // after the join the two values are multiplied (one Fp12 product program).  Same product of the same n + 1 Miller
-    // values, hence same GT.  Measured: 8 192 sets 8.10 -> 7.24 ms, 16 384: 11.1 -> 10.5, 32 768: 18.05 -> 17.2,
-    // 131 072: 57.7 -> 57.0; re-swept at the end of the round: it pays from ~4 500 sets on (4 800: 7.0 -> 6.87 ms, 6 000: 7.2 -> 7.0;
-    // 4 096: 6.55 -> 6.60, 3 000: 6.44 -> 6.51).
-    static const size_t defer_min = getenv("BLSGPU_DEFER_SIG_MIN") ? (size_t)atoll(getenv("BLSGPU_DEFER_SIG_MIN")) : 4500;
-    const bool defer_sig = ctx->use_side && !ctx->serial_tail && n >= defer_min && !scalars;
-    if (defer_sig) {
-        const size_t per = (size_t)ML_NLINES * 6;
-        if (!ctx->sig_lines) {
-            CK(cudaMalloc((void **)&ctx->sig_lines, (size_t)ML_NLINES * ML_LINE_WORDS * 4 * 32));
-            CK(cudaMalloc((void **)&ctx->sig_F, 2048 * sizeof(fp12)));
-            CK(cudaMalloc((void **)&ctx->sig_F2, 512 * sizeof(fp12)));
-            CK(cudaMalloc((void **)&ctx->sig_seg, 64 * sizeof(fp12)));
-            CK(cudaMalloc((void **)&ctx->sig_small_lines, 2 * per * sizeof(fp)));
+    // Deferred signature pair: pair number n = (S, -G1) gets its own one-pair Miller loop right here on the side stream,
+    // on its own workspace, beside the big loop of the main stream; after the join the two values are multiplied (one
+    // Fp12 product program).  Same product of the same n + 1 Miller values, hence same GT.
+    if (plan.defer_sig) {
+        miller_ws &ws = ctx->ml_sig;
+        if (!ws.lines) {
+            CK(cudaMalloc((void **)&ws.lines, (size_t)ML_NLINES * ML_LINE_WORDS * 4 * ws.lines_cap));
+            CK(cudaMalloc((void **)&ws.F, ws.f_cap * sizeof(fp12)));
+            CK(cudaMalloc((void **)&ws.F2, ws.f2_cap * sizeof(fp12)));
+            CK(cudaMalloc((void **)&ws.seg, 64 * sizeof(fp12)));
+            CK(cudaMalloc((void **)&ws.small_lines, 2 * (size_t)ML_NLINES * 6 * sizeof(fp)));
         }
-        // run_miller works on the context's buffers and stream: lend it the pair's own for this one call
-        struct swap_t {
-            blsgpu_ctx *c; uint32_t *lines; size_t lines_cap, f_cap, f2_cap; fp12 *F, *F2, *seg; fp *sl; cudaStream_t st; cudaEvent_t ev[8];
-            ~swap_t() {
-                c->d_lines = lines; c->lines_cap = lines_cap; c->f_cap = f_cap; c->f2_cap = f2_cap; c->d_F = F; c->d_F2 = F2;
-                c->d_seg = seg; c->d_small_lines = sl; c->stream = st;
-                const int ids[4] = {ST_LINES, ST_ACC, ST_GTPROD, ST_PARTIAL};
-                for (int k = 0; k < 4; k++) { c->ev[2 * ids[k]] = ev[2 * k]; c->ev[2 * ids[k] + 1] = ev[2 * k + 1]; }
-            }
-        } keep{ctx, ctx->d_lines, ctx->lines_cap, ctx->f_cap, ctx->f2_cap, ctx->d_F, ctx->d_F2, ctx->d_seg, ctx->d_small_lines, ctx->stream, {}};
-        const int ids[4] = {ST_LINES, ST_ACC, ST_GTPROD, ST_PARTIAL};
-        for (int k = 0; k < 4; k++) { keep.ev[2 * k] = ctx->ev[2 * ids[k]]; keep.ev[2 * k + 1] = ctx->ev[2 * ids[k] + 1]; }
-        for (int k = 0; k < 4; k++) { ctx->ev[2 * ids[k]] = ctx->ev_scratch[2 * k]; ctx->ev[2 * ids[k] + 1] = ctx->ev_scratch[2 * k + 1]; }
-        ctx->d_lines = ctx->sig_lines; ctx->lines_cap = 32; ctx->d_F = ctx->sig_F; ctx->f_cap = 2048; ctx->d_F2 = ctx->sig_F2;
-        ctx->f2_cap = 512; ctx->d_seg = ctx->sig_seg; ctx->d_small_lines = ctx->sig_small_lines; ctx->stream = g;
-        rc = run_miller(ctx, 1, slot + 1, n);
+        rc = run_miller(ctx, ws, 1, slot + 1, n);
         if (rc) return rc;
     }
     if (ctx->use_side) CK(cudaEventRecord(ctx->ev[EV_JOIN], g));
-    if (!msm_after_hash) {
+    if (!plan.msm_after_hash) {
         rc = launch_hash();
         if (rc) return rc;
     }
-    if (g1_aside) {
+    if (plan.g1_aside) {
         CK(cudaStreamWaitEvent(s, ctx->ev[EV_G1], 0));
     } else {
         if (ctx->use_side) CK(cudaStreamWaitEvent(s, ctx->ev[EV_SC], 0));
@@ -877,31 +752,28 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
         END(ST_G1MUL, s);
     }
     BEGIN(ST_AFFINE, s);
-    // small batches: one inversion per set is pure latency -> binary Euclid, one working lane per warp (it diverges
-    // across the lanes of a warp: sharing warps it is no quicker than the uniform Fermat chain, 0.53 vs 0.46 ms at 129)
-    static const size_t aff_block_min = getenv("BLSGPU_AFFINE_BLOCK_MIN") ? (size_t)atoll(getenv("BLSGPU_AFFINE_BLOCK_MIN")) : 1025;
-    if (n >= aff_block_min) {
+    if (plan.affine == route::AFFINE_BLOCK) {
         // one Euclid inversion per block of 128 threads, about 32 768 threads in flight: 1 set per thread up to 32 768
         // sets, up to AFF_B beyond
         int per = (int)((n + 32767) / 32768);
         if (per > AFF_B) per = AFF_B;
         k_pairs_affine<<<nblk((n + per - 1) / per), 128, 0, s>>>(ctx->d_H, ctx->d_Pj, n, ctx->d_Q, ctx->d_P, 2, 0, per);
-    } else if (small) k_pairs_affine<<<(unsigned)n, 32, 0, s>>>(ctx->d_H, ctx->d_Pj, n, ctx->d_Q, ctx->d_P, 1, 1, AFF_B);
+    } else if (plan.affine == route::AFFINE_WARP) k_pairs_affine<<<(unsigned)n, 32, 0, s>>>(ctx->d_H, ctx->d_Pj, n, ctx->d_Q, ctx->d_P, 1, 1, AFF_B);
     else k_pairs_affine<<<nblk((n + AFF_B - 1) / AFF_B), 128, 0, s>>>(ctx->d_H, ctx->d_Pj, n, ctx->d_Q, ctx->d_P, 0, 0, AFF_B);
     END(ST_AFFINE, s);
     ctx->launches += 3;
-    if (!defer_sig) {
+    if (!plan.defer_sig) {
         if (ctx->use_side) CK(cudaStreamWaitEvent(s, ctx->ev[EV_JOIN], 0));   // join: pair number n is in place
-        return run_miller(ctx, n + 1, slot);
+        return run_miller(ctx, ctx->ml, n + 1, slot);
     }
-    rc = run_miller(ctx, n, slot);                           // the n set pairs; (S, -G1) is being done on the side stream
+    rc = run_miller(ctx, ctx->ml, n, slot);                  // the n set pairs; (S, -G1) is being done on the side stream
     if (rc) return rc;
     CK(cudaStreamWaitEvent(s, ctx->ev[EV_JOIN], 0));
     blsgpu_ctx::dev_prog p2;
-    rc = get_prog(ctx, 4, 2, p2);
+    rc = get_prog(ctx, 4, 2, p2, s);
     if (rc) return rc;
     // in place: the program loads all 24 inputs into its slot file before the first round and stores at the end
-    rc = launch_prog(ctx, p2, (const fp *)(ctx->d_partials + slot), (fp *)(ctx->d_partials + slot));
+    rc = launch_prog(ctx, p2, s, (const fp *)(ctx->d_partials + slot), (fp *)(ctx->d_partials + slot));
     if (rc) return rc;
     END(ST_PARTIAL, s);
     CK(cudaGetLastError());
@@ -919,14 +791,14 @@ static int run_final_enqueue(blsgpu_ctx *ctx, int count, const fp12 *d_partials 
     } else {
         // norm program -> one-thread binary-Euclid inversion -> main program (fpprog.hpp build_final)
         blsgpu_ctx::dev_prog fpn, fpg;
-        int rc = get_prog(ctx, 2, count, fpn);
-        if (!rc) rc = get_prog(ctx, 1, count, fpg);
+        int rc = get_prog(ctx, 2, count, fpn, s);
+        if (!rc) rc = get_prog(ctx, 1, count, fpg, s);
         if (rc) return rc;
-        rc = launch_prog(ctx, fpn, (const fp *)parts, ctx->d_norm);
+        rc = launch_prog(ctx, fpn, s, (const fp *)parts, ctx->d_norm);
         if (rc) return rc;
         k_fp_inv_one<<<1, 32, 0, s>>>(ctx->d_norm, ctx->d_norm + 1);
         ctx->launches++;
-        rc = launch_prog(ctx, fpg, (const fp *)parts, (fp *)ctx->d_gt, ctx->d_norm + 1);
+        rc = launch_prog(ctx, fpg, s, (const fp *)parts, (fp *)ctx->d_gt, ctx->d_norm + 1);
         if (rc) return rc;
         k_final_out<<<1, 32, 0, s>>>(ctx->d_gt, count, d_rank_flags, ctx->d_gtb, ctx->d_flags + 1);
         ctx->launches++;
@@ -968,7 +840,7 @@ extern "C" int blsgpu_rlc_scalars(blsgpu_ctx *ctx, const uint8_t srb[32], size_t
     if (n == 0) return 0;
     if (n > ctx->cap) return fail(ctx, BLSGPU_ERR_CAPACITY, "batch larger than context capacity");
     CK(cudaSetDevice(ctx->device));
-    int rc = launch_scalars(ctx, srb, n, 0, n, chunks, nullptr, ctx->stream);
+    int rc = launch_scalars(ctx, srb, n, 0, n, chunks, nullptr, route::chain_hog(thr(), n, chunks), ctx->stream);
     if (rc) return rc;
     CK(cudaMemcpyAsync(out, ctx->d_r, n * 8, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
@@ -1032,8 +904,7 @@ extern "C" int blsgpu_batch_verify_dev(blsgpu_ctx *ctx, const void *d_sets, size
     if (n > ctx->cap) return fail(ctx, BLSGPU_ERR_CAPACITY, "batch larger than context capacity");
     CK(cudaSetDevice(ctx->device));
     int rc, pk_inf = 0;
-    static const size_t graph_max = getenv("BLSGPU_GRAPH_MAX") ? (size_t)atoll(getenv("BLSGPU_GRAPH_MAX")) : 8192;
-    if (ctx->use_graph && !scalars && srb && n <= graph_max && !ctx->serial_tail) {
+    if (srb && batch_plan_of(ctx, n, n, chunks, false, scalars != nullptr).graph) {
         bool done = false;
         rc = verify_graphed(ctx, d_sets, n, srb, chunks, done);
         if (rc) return rc;
@@ -1122,19 +993,13 @@ extern "C" int blsgpu_batch_verify(blsgpu_ctx *ctx, const void *sets, size_t n, 
     if (n == 0) return 0;
     if (!sets) return fail(ctx, BLSGPU_ERR_ARG, "sets is NULL");
     if (n > blsgpu_capacity(ctx)) return fail(ctx, BLSGPU_ERR_CAPACITY, "batch larger than context capacity");
-    if (!ctx->peers.empty()) {
-        if (!scalars && !srb) return fail(ctx, BLSGPU_ERR_ARG, "secureRandomBytes is NULL");
-        if (scalars)
-            for (size_t i = 0; i < n; i++) if (scalars[i] == 0) return fail(ctx, BLSGPU_ERR_ARG, "explicit RLC scalar is zero");
-        return batch_verify_multi(ctx, (const uint8_t *)sets, n, srb, chunks, scalars, gt_out);
-    }
     // argument errors are reported before the copy is queued: no transfer from the caller's buffer outlives the call
     if (!scalars && !srb) return fail(ctx, BLSGPU_ERR_ARG, "secureRandomBytes is NULL");
     if (scalars)
         for (size_t i = 0; i < n; i++) if (scalars[i] == 0) return fail(ctx, BLSGPU_ERR_ARG, "explicit RLC scalar is zero");
+    if (!ctx->peers.empty()) return batch_verify_multi(ctx, (const uint8_t *)sets, n, srb, chunks, scalars, gt_out);
     CK(cudaSetDevice(ctx->device));
-    static const size_t graph_max = getenv("BLSGPU_GRAPH_MAX") ? (size_t)atoll(getenv("BLSGPU_GRAPH_MAX")) : 8192;
-    if (n <= graph_max) {
+    if (batch_plan_of(ctx, n, n, chunks, true, scalars != nullptr).copy_ahead) {
         // small batches replay a captured graph that starts from ctx->d_sets: the copy stays outside of it
         CK(cudaMemcpyAsync(ctx->d_sets, sets, n * sizeof(sigset), cudaMemcpyHostToDevice, ctx->stream));
         return blsgpu_batch_verify_dev(ctx, ctx->d_sets, n, srb, chunks, scalars, gt_out);
@@ -1261,14 +1126,14 @@ extern "C" int blsgpu_hash_to_g2(blsgpu_ctx *ctx, const uint8_t *msgs, size_t n,
 // Test hook: the hash of the small-batch route up to (and including) the cofactor-clearing program.
 // out_in / out_out: n x 6 field elements each (homogeneous point before / after the program), host buffers.
 extern "C" int blsgpu_test_small_hash(blsgpu_ctx *ctx, const void *sets320, size_t n, uint8_t *out_in, uint8_t *out_out) {
-    if (!ctx || !sets320 || n == 0 || n > SMALL_ROUTE_MAX || n > ctx->cap) return BLSGPU_ERR_ARG;
+    if (!ctx || !sets320 || n == 0 || n > route::SMALL_ROUTE_CAP || n > ctx->cap) return BLSGPU_ERR_ARG;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->stream;
-    if (!ctx->d_small) CK(cudaMalloc((void **)&ctx->d_small, (size_t)SMALL_ROUTE_MAX * SMALL_FP_PER_SET * sizeof(fp)));
+    if (!ctx->d_small) CK(cudaMalloc((void **)&ctx->d_small, route::SMALL_ROUTE_CAP * SMALL_FP_PER_SET * sizeof(fp)));
     blsgpu_ctx::dev_prog p_cof;
-    int rc = get_prog(ctx, 3, SETPROG_COFACTOR, p_cof);
+    int rc = get_prog(ctx, 3, SETPROG_COFACTOR, p_cof, s);
     if (rc) return rc;
-    fp *hin = ctx->d_small, *hout = hin + 6 * SMALL_ROUTE_MAX;
+    fp *hin = ctx->d_small, *hout = hin + 6 * route::SMALL_ROUTE_CAP;
     CK(cudaMemcpyAsync(ctx->d_sets, sets320, n * 320, cudaMemcpyHostToDevice, s));
     k_hash_map_lanes2<<<nblk(2 * n, 64), 64, 0, s>>>(ctx->d_sets, nullptr, nullptr, nullptr, 0, n, hin);
     launch_prog_many(ctx, p_cof, s, n, hin, 6, nullptr, 0, hout, 6);
@@ -1374,16 +1239,14 @@ static int verify_pairs_dev(blsgpu_ctx *ctx, const g1_aff *d_pks, size_t n, cons
     ctx->launches = 0;
     CK(cudaMemsetAsync(ctx->d_flags, 0, 4 * sizeof(int), s));
     BEGIN(ST_HASH, s);
-    static const int small_env = getenv("BLSGPU_SMALL_ROUTE") ? atoi(getenv("BLSGPU_SMALL_ROUTE")) : 15;
-    if ((small_env & 1) && n <= small_route_max() && !ctx->serial_tail) {
+    if (route::program_hash(thr(), n, ctx->serial_tail)) {
         // small-batch route (see run_partial): two lanes per message, cofactor clearing as a per-message program
         blsgpu_ctx::dev_prog p_cof;
-        int rcp = get_prog(ctx, 3, SETPROG_COFACTOR, p_cof);
+        int rcp = get_prog(ctx, 3, SETPROG_COFACTOR, p_cof, s);
         if (rcp) return rcp;
-        if (!ctx->d_small) CK(cudaMalloc((void **)&ctx->d_small, (size_t)SMALL_ROUTE_MAX * SMALL_FP_PER_SET * sizeof(fp)));
-        fp *hin = ctx->d_small, *hout = hin + 6 * SMALL_ROUTE_MAX;
-        static const int map2 = getenv("BLSGPU_MAP_LANES2") ? atoi(getenv("BLSGPU_MAP_LANES2")) : 1;
-        if (map2) k_hash_map_lanes2<<<nblk(2 * n, 64), 64, 0, s>>>(nullptr, d_msgs, d_offs, d_dst, (uint32_t)dst_len, n, hin);
+        if (!ctx->d_small) CK(cudaMalloc((void **)&ctx->d_small, route::SMALL_ROUTE_CAP * SMALL_FP_PER_SET * sizeof(fp)));
+        fp *hin = ctx->d_small, *hout = hin + 6 * route::SMALL_ROUTE_CAP;
+        if (thr().map_lanes2) k_hash_map_lanes2<<<nblk(2 * n, 64), 64, 0, s>>>(nullptr, d_msgs, d_offs, d_dst, (uint32_t)dst_len, n, hin);
         else k_hash_map_pair_msgs<<<nblk(2 * n), 128, 0, s>>>(d_msgs, d_offs, d_dst, (uint32_t)dst_len, n, hin);
         launch_prog_many(ctx, p_cof, s, n, hin, 6, nullptr, 0, hout, 6);
         k_g2_hom_to_affine<<<(unsigned)n, 32, 0, s>>>(hout, n, ctx->d_Q);
@@ -1395,7 +1258,7 @@ static int verify_pairs_dev(blsgpu_ctx *ctx, const g1_aff *d_pks, size_t n, cons
     k_verify_pairs<<<nblk(n + 1), 128, 0, s>>>(d_pks, n, d_sig, ctx->d_Q, ctx->d_P, ctx->d_flags);
     ctx->launches += 2;
     CK(cudaGetLastError());
-    int rc = run_miller(ctx, n + 1, 0);
+    int rc = run_miller(ctx, ctx->ml, n + 1, 0);
     if (rc) return rc;
     int pk_inf = 0;
     rc = run_final(ctx, 1, gt_out, &pk_inf);

@@ -11,6 +11,7 @@
 #include "../../nim_blscurve_b200/csrc/io.cuh"
 #include "../../nim_blscurve_b200/csrc/fpprog.hpp"
 #include "../../nim_blscurve_b200/csrc/fplin.cuh"
+#include "../../nim_blscurve_b200/csrc/route.hpp"
 using namespace bls;
 
 // subtractAll as blsgpu.cu: subtract_all arranges it: pairwise tree over (elems..., -dst), negated root, to affine
@@ -287,4 +288,21 @@ int hs_pubkey_from_bytes(const uint8_t *in, int len, int group_check, g1_aff *ou
 int hs_signature_from_bytes(const uint8_t *in, int len, int group_check, g2_aff *out) { return signature_from_bytes(*out, in, len, group_check != 0); }
 void hs_g1_compress(const g1_aff *p, uint8_t *out) { g1_compress(out, *p); }
 void hs_miller_combine(const fp12 *seg, int nseg, fp12 *out) { miller_combine(*out, seg, nseg); }
+
+// ---- route.hpp: the plans of the batch pipeline, thresholds read from the environment at every call ----
+// out: the fields of route::batch_plan in declaration order
+void hs_plan_batch(size_t n, size_t total_n, uint32_t chunks, int host_src, int scalars, int use_side, int acc_team,
+                   int serial_tail, int use_graph, int *out) {
+    const route::switches sw = {use_side != 0, acc_team != 0, serial_tail != 0, use_graph != 0};
+    const route::batch_plan p = route::plan_batch(route::read_thresholds(), sw, n, total_n, chunks, host_src != 0, scalars != 0);
+    const int v[12] = {p.hash, p.sliced, p.small, p.sig, p.g1_aside, p.msm_after_hash, p.defer_sig, p.affine, p.chain_hog,
+                       p.chain_wait, p.graph, p.copy_ahead};
+    memcpy(out, v, sizeof v);
+}
+// out: G, nseg, lines, lines_last, ncols, gt_prog
+void hs_plan_miller(size_t np, size_t lines_cap, int team, int serial_tail, long long *out) {
+    const route::miller_plan p = route::plan_miller(route::read_thresholds(), np, lines_cap, team != 0, serial_tail != 0);
+    const long long v[6] = {p.G, p.nseg, p.lines, p.lines_last, (long long)p.ncols, p.gt_prog};
+    memcpy(out, v, sizeof v);
+}
 }

@@ -193,9 +193,10 @@ def test_epoch_batch_full_size_properties(br, srb):
 
 @pytest.mark.parametrize("n", [127, 128, 129, 1024, 1025, 2047, 2048, 2049, 2499, 2500, 4096, 4097, 4499, 4500, 6000, 8192, 8193, 9000])
 def test_route_boundaries_vs_blst(br, srb, n):
-    """The batch pipeline picks its kernels by batch size (warp-per-set programs up to 4 096 sets, two lanes per message
-    up to 8 192, a thread per set beyond; the G2 sum switches to Pippenger at 2 048): one batch just past each boundary,
-    valid and with one corrupted set, verdict and GT against BLST."""
+    """The batch pipeline picks its kernels by batch size (route.hpp; tests/test_hostsim.py::test_route_plans pins the
+    plans): per-set programs up to 4 096 sets, two lanes per message from 2 049, Pippenger for the G2 sum from 2 500,
+    the signature pair's own Miller loop from 4 500, graph replay up to 8 192.  One batch on each side of the
+    boundaries, valid and with one corrupted set, verdict and GT against BLST."""
     import nim_blscurve_b200 as bg
     c = bg.BatchedBLSVerifierCache(max_sets=n, device=0)
     try:

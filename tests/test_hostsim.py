@@ -447,3 +447,34 @@ def test_programs_in_the_lincomb_format_too(hs):
     assert bytes(r1) == bytes(r2)
     assert stats2[0] < 1100 and stats1[0] > 2 * stats2[0], (list(stats1), list(stats2))   # 2 408 -> 973 rounds
     assert stats2[1] == stats1[1]                                                           # same multiplication rounds
+
+
+def test_route_plans(hs, monkeypatch):
+    """route.hpp: the batch plan (hash route, host copy, small-route buffers, signature sum, streams, affine mode, scalar
+    chain, graph replay) and the Miller plan (G, segments, lines route of each tile, GT product) at the size boundaries of
+    the pipeline, with and without a host source, explicit scalars and the serial tail, under the default thresholds and
+    under non-default ones (clamps included).  tests/golden/route_plans.json holds the routes the batch pipeline took for
+    these inputs before its decisions moved into route.hpp."""
+    d = json.load(open(os.path.join(GOLD, "route_plans.json")))
+    names = {"hash": ["program", "lanes2", "pair", "thread"], "sig": ["program", "mul", "msm"],
+             "affine": ["default", "warp", "block"], "lines": ["program", "lanes2", "thread"]}
+    names["lines_last"] = names["lines"]
+    for k in [k for k in os.environ if k.startswith("BLSGPU_")]:
+        monkeypatch.delenv(k)
+    for cfg in d["configs"]:
+        for k, v in cfg["env"].items():
+            monkeypatch.setenv(k, v)
+        for inp, want in cfg["batch"]:
+            n, total, chunks, *flags = inp
+            o = (C.c_int * 12)()
+            hs.hs_plan_batch(C.c_size_t(n), C.c_size_t(total), C.c_uint32(chunks), *flags, o)
+            got = [names[f][v] if f in names else v for f, v in zip(d["batch_plan"], o)]
+            assert got == want, (cfg["env"], inp)
+        for inp, want in cfg["miller"]:
+            np_, cap, team, serial = inp
+            o = (C.c_longlong * 6)()
+            hs.hs_plan_miller(C.c_size_t(np_), C.c_size_t(cap), team, serial, o)
+            got = [names[f][v] if f in names else v for f, v in zip(d["miller_plan"], o)]
+            assert got == want, (cfg["env"], inp)
+        for k in cfg["env"]:
+            monkeypatch.delenv(k)
