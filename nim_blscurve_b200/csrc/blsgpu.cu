@@ -6,6 +6,7 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <functional>
 #include <string>
 #include <map>
 #include <vector>
@@ -24,6 +25,10 @@ static const char *STAGE_NAMES[ST_COUNT] = {"rlc_scalars", "g2_mul64", "g2_sum",
 static const size_t LINES_TILE = (size_t)1 << 18;
 static_assert(route::ACC_BLOCK == BLS_ACC_BS && ST_ACC == ST_LINES + 1 && ST_GTPROD == ST_LINES + 2 && ST_PARTIAL == ST_LINES + 3,
               "route.hpp / miller_ws layout");
+static_assert(route::LB_BLOCKS == BLS_LB_BLOCKS, "route.hpp plan_msm sizes the chunk grid for the BLS_LB occupancy");
+
+// device programs (fpprog.hpp) kept in blsgpu_ctx::progs, by kind and a key (see get_prog)
+enum prog_kind { PROG_COMBINE, PROG_FINAL, PROG_NORM, PROG_SET, PROG_PRODUCT, PROG_MSM_HORNER_G1, PROG_MSM_HORNER_G2 };
 
 // Buffers, stream and stage events of one multi-Miller loop (run_miller)
 struct miller_ws {
@@ -75,9 +80,9 @@ struct blsgpu_ctx {
     float stage_ms[ST_COUNT];
     int launches = 0;
     msm_state msm;
-    // warp-cooperative tail programs (fpprog.hpp), compiled on first use and kept on the device
+    // warp-cooperative dataflow programs (fpprog.hpp), compiled on first use and kept on the device
     struct dev_prog { uint32_t *d = nullptr; int nslots = 0, nrounds = 0, version = 1; };
-    std::map<int, dev_prog> combine_progs, final_progs, norm_progs, set_progs, prod_progs;   // keyed by segment count / partial count
+    std::map<std::pair<int, int>, dev_prog> progs;           // keyed by (prog_kind, key)
     fp *d_small = nullptr;                                   // per-set program inputs/outputs of the small-batch route
     fp *d_norm = nullptr;                                    // [0] Fp norm taken out of the final exponentiation, [1] its inverse
     fp *d_consts = nullptr;                                  // Frobenius coefficients (fpprog::CONST_*)
@@ -154,11 +159,7 @@ extern "C" void blsgpu_destroy(blsgpu_ctx *ctx) {
     cudaFree(ctx->d_sets); cudaFree(ctx->d_r); cudaFree(ctx->d_H); cudaFree(ctx->d_Pj); cudaFree(ctx->d_Q);
     cudaFree(ctx->d_P); cudaFree(ctx->d_S); cudaFree(ctx->d_partials); cudaFree(ctx->d_gtb);
     cudaFree(ctx->d_flags); cudaFree(ctx->d_dbg); cudaFree(ctx->d_misc); cudaFree(ctx->d_misc2); cudaFree(ctx->d_consts); cudaFree(ctx->d_gt);
-    for (auto &kv : ctx->combine_progs) cudaFree(kv.second.d);
-    for (auto &kv : ctx->final_progs) cudaFree(kv.second.d);
-    for (auto &kv : ctx->norm_progs) cudaFree(kv.second.d);
-    for (auto &kv : ctx->set_progs) cudaFree(kv.second.d);
-    for (auto &kv : ctx->prod_progs) cudaFree(kv.second.d);
+    for (auto &kv : ctx->progs) cudaFree(kv.second.d);
     cudaFree(ctx->d_norm); cudaFree(ctx->d_small);
     msm_free(ctx->msm);
     if (ctx->h_pinned) cudaFreeHost(ctx->h_pinned);
@@ -375,28 +376,37 @@ static int launch_scalars(blsgpu_ctx *ctx, const uint8_t srb[32], size_t n, size
 
 enum { SETPROG_COFACTOR = 0, SETPROG_G2MUL64 = 1, SETPROG_LINES = 2 };
 
-// Compile (once) and fetch a tail program; kind 0 = combine over `key` segments, 1 = final exponentiation of `key`
-// partials with the Fp inversion supplied in IN1, 2 = the norm that inversion applies to (fpprog.hpp build_final),
-// 3 = per-set G2 program `key` (SETPROG_*), 4 = product tree over `key` Fp12 values.  A first use uploads the program
-// on stream st and waits for it.
-static int get_prog(blsgpu_ctx *ctx, int kind, int key, blsgpu_ctx::dev_prog &out, cudaStream_t st) {
-    std::map<int, blsgpu_ctx::dev_prog> &cache = kind == 0 ? ctx->combine_progs : (kind == 1 ? ctx->final_progs : (kind == 2 ? ctx->norm_progs : (kind == 3 ? ctx->set_progs : ctx->prod_progs)));
-    auto it = cache.find(key);
-    if (it != cache.end()) { out = it->second; return 0; }
+// Compile (once) and fetch a program:
+//   PROG_COMBINE        combine over `key` segments
+//   PROG_FINAL          final exponentiation of `key` partials with the Fp inversion supplied in IN1
+//   PROG_NORM           the norm that inversion applies to (fpprog.hpp build_final)
+//   PROG_SET            per-set G2 program `key` (SETPROG_*)
+//   PROG_PRODUCT        product tree over `key` Fp12 values
+//   PROG_MSM_HORNER_G*  window Horner of an MSM, key = nwin * 64 + c (c < 64)
+// A first use uploads the program on stream st and waits for it.  A tail program that does not build fails the call;
+// a Horner program that does not build or needs more than 48 KiB of shared memory is cached as absent (out.d == nullptr),
+// and the MSM runs k_msm_horner instead.
+static int get_prog(blsgpu_ctx *ctx, prog_kind kind, int key, blsgpu_ctx::dev_prog &out, cudaStream_t st) {
+    auto it = ctx->progs.find({kind, key});
+    if (it != ctx->progs.end()) { out = it->second; return 0; }
     fpprog::Program P;
-    if (kind == 0) {
+    const bool horner = kind == PROG_MSM_HORNER_G1 || kind == PROG_MSM_HORNER_G2;
+    if (kind == PROG_COMBINE) {
         int len[64];
         for (int j = 0; j < key; j++) len[j] = ml_seg_hi(j, key) - ml_seg_lo(j, key) + 1;
         P = fpprog::build_combine(key, len);
-    } else if (kind == 4) {                              // product of `key` Fp12 values (GT product of a small batch)
+    } else if (kind == PROG_PRODUCT) {                   // product of `key` Fp12 values (GT product of a small batch)
         P = fpprog::build_fp12_product(key);
-    } else if (kind == 3) {                              // per-set programs of the small-batch route
+    } else if (kind == PROG_SET) {                       // per-set programs of the small-batch route
         P = key == SETPROG_COFACTOR ? fpprog::build_g2_clear_cofactor() : (key == SETPROG_G2MUL64 ? fpprog::build_g2_mul64() : fpprog::build_miller_lines());
+    } else if (horner) {
+        P = kind == PROG_MSM_HORNER_G1 ? fpprog::build_msm_horner_g1(key / 64, key % 64) : fpprog::build_msm_horner_g2(key / 64, key % 64);
     } else {
-        P = fpprog::build_final(key, kind == 1 ? fpprog::INV_EXTERNAL : fpprog::INV_EMIT_ARG);
+        P = fpprog::build_final(key, kind == PROG_FINAL ? fpprog::INV_EXTERNAL : fpprog::INV_EMIT_ARG);
     }
-    if (!P.ok) return fail(ctx, BLSGPU_ERR_ARG, "tail program does not fit the slot file");
     blsgpu_ctx::dev_prog dp;
+    if (horner && (!P.ok || (size_t)P.nslots * sizeof(fp) > 48 * 1024)) { ctx->progs[{kind, key}] = dp; out = dp; return 0; }
+    if (!P.ok) return fail(ctx, BLSGPU_ERR_ARG, "tail program does not fit the slot file");
     dp.nslots = P.nslots;
     dp.nrounds = P.nrounds;
     dp.version = P.version;
@@ -404,7 +414,7 @@ static int get_prog(blsgpu_ctx *ctx, int kind, int key, blsgpu_ctx::dev_prog &ou
     // stream-ordered upload, completed before the host vector goes away (first use only)
     CK(cudaMemcpyAsync(dp.d, P.words.data(), P.words.size() * 4, cudaMemcpyHostToDevice, st));
     CK(cudaStreamSynchronize(st));
-    cache[key] = dp;
+    ctx->progs[{kind, key}] = dp;
     out = dp;
     return 0;
 }
@@ -438,6 +448,25 @@ static int launch_prog(blsgpu_ctx *ctx, const blsgpu_ctx::dev_prog &p, cudaStrea
     return 0;
 }
 
+// sum_i [k_i] P_i on stream s (msm.cuh msm_run) in the shape route::plan_msm picks, the window Horner as a program when
+// the plan allows it and the program builds; a failure is reported into ctx
+template <class F>
+static int run_msm(blsgpu_ctx *ctx, const uint8_t *d_points, size_t pstride, const uint8_t *d_scalars, size_t sstride, size_t n,
+                   int nbits, cudaStream_t s, jac_t<F> *d_out_jac, aff_t<F> *d_out_aff) {
+    const route::msm_plan p = route::plan_msm(thr(), n, nbits, ctx->msm.sms);
+    blsgpu_ctx::dev_prog hp;
+    if (p.horner_prog) {
+        int rc = get_prog(ctx, std::is_same<F, fp>::value ? PROG_MSM_HORNER_G1 : PROG_MSM_HORNER_G2, p.nwin * 64 + p.c, hp, s);
+        if (rc) return rc;
+    }
+    std::function<void(cudaStream_t, const fp *, fp *)> horner;
+    if (hp.d) horner = [&](cudaStream_t ts, const fp *in, fp *out) { launch_prog_many(ctx, hp, ts, 1, in, 0, nullptr, 0, out, 0); };
+    std::string err;
+    int rc = msm_run<F>(ctx->msm, p, horner, d_points, pstride, d_scalars, sstride, n, nbits, s, d_out_jac, d_out_aff,
+                        &ctx->launches, err);
+    return rc ? fail(ctx, rc == -1 ? BLSGPU_ERR_CUDA : BLSGPU_ERR_ARG, err.c_str()) : 0;
+}
+
 #define SMALL_FP_PER_SET (6 + 6 + 6 + 6 + 64)
 
 // Multi-Miller loop over the np pairs (d_Q[pair0 + i], d_P[pair0 + i]) + reductions, on the buffers, stream and stage
@@ -469,7 +498,7 @@ static int run_miller(blsgpu_ctx *ctx, miller_ws &ws, size_t np, int slot, size_
             // one warp per pair runs the 68 line evaluations as a dataflow program, then a scatter into the
             // accumulation's layout
             blsgpu_ctx::dev_prog lp;
-            rc = get_prog(ctx, 3, SETPROG_LINES, lp, s);
+            rc = get_prog(ctx, PROG_SET, SETPROG_LINES, lp, s);
             if (rc) return rc;
             const size_t per = (size_t)ML_NLINES * 6;
             if (!ws.small_lines) CK(cudaMalloc((void **)&ws.small_lines, thr().small_lines_max * per * sizeof(fp)));
@@ -510,7 +539,7 @@ static int run_miller(blsgpu_ctx *ctx, miller_ws &ws, size_t np, int slot, size_
         size_t cols = ncols, stride = row_stride;
         while (cols > 8) {
             const size_t m = (cols + 7) / 8, m_stride = m > 8 ? ((m + 7) & ~(size_t)7) : m;
-            rc = get_prog(ctx, 4, 8, p8, s);
+            rc = get_prog(ctx, PROG_PRODUCT, 8, p8, s);
             if (rc) return rc;
             if (cols & 7) { k_fp12_pad_one<<<nseg, 32, 0, s>>>(cur, stride, cols); ctx->launches++; }
             launch_prog_rows(ctx, p8, s, (size_t)nseg * m, cur, other, (unsigned)m, stride, m_stride);
@@ -518,7 +547,7 @@ static int run_miller(blsgpu_ctx *ctx, miller_ws &ws, size_t np, int slot, size_
             cols = m;
             stride = m_stride;
         }
-        rc = get_prog(ctx, 4, (int)cols, pm, s);
+        rc = get_prog(ctx, PROG_PRODUCT, (int)cols, pm, s);
         if (rc) return rc;
         launch_prog_rows(ctx, pm, s, (size_t)nseg, cur, ws.seg, 1u, stride, 1);
     } else if (ncols > BLS_ACC_BS) {
@@ -537,7 +566,7 @@ static int run_miller(blsgpu_ctx *ctx, miller_ws &ws, size_t np, int slot, size_
         ctx->launches++;
     } else {
         blsgpu_ctx::dev_prog cp;
-        rc = get_prog(ctx, 0, nseg, cp, s);
+        rc = get_prog(ctx, PROG_COMBINE, nseg, cp, s);
         if (rc) return rc;
         rc = launch_prog(ctx, cp, s, (const fp *)ws.seg, (fp *)(ctx->d_partials + slot));
         if (rc) return rc;
@@ -629,8 +658,8 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
     fp *sm_hash_in = nullptr, *sm_hash_out = nullptr, *sm_sig_in = nullptr, *sm_sig_out = nullptr, *sm_bits = nullptr;
     if (plan.small) {
         if (!ctx->d_small) CK(cudaMalloc((void **)&ctx->d_small, route::SMALL_ROUTE_CAP * SMALL_FP_PER_SET * sizeof(fp)));
-        rc = get_prog(ctx, 3, SETPROG_COFACTOR, p_cof, s);
-        if (!rc) rc = get_prog(ctx, 3, SETPROG_G2MUL64, p_mul, s);
+        rc = get_prog(ctx, PROG_SET, SETPROG_COFACTOR, p_cof, s);
+        if (!rc) rc = get_prog(ctx, PROG_SET, SETPROG_G2MUL64, p_mul, s);
         if (rc) return rc;
         sm_hash_in = ctx->d_small;
         sm_hash_out = sm_hash_in + 6 * route::SMALL_ROUTE_CAP;
@@ -695,10 +724,9 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
     BEGIN(ST_G2MUL, g);
     // S = sum_i [r_i] sig_i
     if (plan.sig == route::SIG_MSM) {
-        std::string err;
-        rc = msm_run<fp2>(ctx->msm, (const uint8_t *)d_sets + offsetof(sigset, sig), sizeof(sigset), (const uint8_t *)ctx->d_r, 8,
-                          n, 64, g, ctx->d_S, nullptr, &ctx->launches, err);
-        if (rc) return fail(ctx, rc == -1 ? BLSGPU_ERR_CUDA : BLSGPU_ERR_ARG, err.c_str());
+        rc = run_msm<fp2>(ctx, (const uint8_t *)d_sets + offsetof(sigset, sig), sizeof(sigset), (const uint8_t *)ctx->d_r, 8, n, 64,
+                          g, ctx->d_S, nullptr);
+        if (rc) return rc;
         END(ST_G2MUL, g);
         BEGIN(ST_G2SUM, g);
     } else {
@@ -770,7 +798,7 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
     if (rc) return rc;
     CK(cudaStreamWaitEvent(s, ctx->ev[EV_JOIN], 0));
     blsgpu_ctx::dev_prog p2;
-    rc = get_prog(ctx, 4, 2, p2, s);
+    rc = get_prog(ctx, PROG_PRODUCT, 2, p2, s);
     if (rc) return rc;
     // in place: the program loads all 24 inputs into its slot file before the first round and stores at the end
     rc = launch_prog(ctx, p2, s, (const fp *)(ctx->d_partials + slot), (fp *)(ctx->d_partials + slot));
@@ -791,8 +819,8 @@ static int run_final_enqueue(blsgpu_ctx *ctx, int count, const fp12 *d_partials 
     } else {
         // norm program -> one-thread binary-Euclid inversion -> main program (fpprog.hpp build_final)
         blsgpu_ctx::dev_prog fpn, fpg;
-        int rc = get_prog(ctx, 2, count, fpn, s);
-        if (!rc) rc = get_prog(ctx, 1, count, fpg, s);
+        int rc = get_prog(ctx, PROG_NORM, count, fpn, s);
+        if (!rc) rc = get_prog(ctx, PROG_FINAL, count, fpg, s);
         if (rc) return rc;
         rc = launch_prog(ctx, fpn, s, (const fp *)parts, ctx->d_norm);
         if (rc) return rc;
@@ -1131,7 +1159,7 @@ extern "C" int blsgpu_test_small_hash(blsgpu_ctx *ctx, const void *sets320, size
     cudaStream_t s = ctx->stream;
     if (!ctx->d_small) CK(cudaMalloc((void **)&ctx->d_small, route::SMALL_ROUTE_CAP * SMALL_FP_PER_SET * sizeof(fp)));
     blsgpu_ctx::dev_prog p_cof;
-    int rc = get_prog(ctx, 3, SETPROG_COFACTOR, p_cof, s);
+    int rc = get_prog(ctx, PROG_SET, SETPROG_COFACTOR, p_cof, s);
     if (rc) return rc;
     fp *hin = ctx->d_small, *hout = hin + 6 * route::SMALL_ROUTE_CAP;
     CK(cudaMemcpyAsync(ctx->d_sets, sets320, n * 320, cudaMemcpyHostToDevice, s));
@@ -1242,7 +1270,7 @@ static int verify_pairs_dev(blsgpu_ctx *ctx, const g1_aff *d_pks, size_t n, cons
     if (route::program_hash(thr(), n, ctx->serial_tail)) {
         // small-batch route (see run_partial): two lanes per message, cofactor clearing as a per-message program
         blsgpu_ctx::dev_prog p_cof;
-        int rcp = get_prog(ctx, 3, SETPROG_COFACTOR, p_cof, s);
+        int rcp = get_prog(ctx, PROG_SET, SETPROG_COFACTOR, p_cof, s);
         if (rcp) return rcp;
         if (!ctx->d_small) CK(cudaMalloc((void **)&ctx->d_small, route::SMALL_ROUTE_CAP * SMALL_FP_PER_SET * sizeof(fp)));
         fp *hin = ctx->d_small, *hout = hin + 6 * route::SMALL_ROUTE_CAP;
@@ -1445,11 +1473,10 @@ static int msm_api_dev(blsgpu_ctx *ctx, const void *d_points, const void *d_scal
     CK(cudaSetDevice(ctx->device));
     int rc = ensure_misc2(ctx, 256);
     if (rc) return rc;
-    std::string err;
     ctx->launches = 0;
-    rc = msm_run<F>(ctx->msm, (const uint8_t *)d_points, pb, (const uint8_t *)d_scalars, (nbits + 7) / 8, n, (int)nbits,
-                    ctx->stream, nullptr, (aff_t<F> *)ctx->d_misc2, &ctx->launches, err);
-    if (rc) return fail(ctx, rc == -1 ? BLSGPU_ERR_CUDA : BLSGPU_ERR_ARG, err.c_str());
+    rc = run_msm<F>(ctx, (const uint8_t *)d_points, pb, (const uint8_t *)d_scalars, (nbits + 7) / 8, n, (int)nbits, ctx->stream,
+                    nullptr, (aff_t<F> *)ctx->d_misc2);
+    if (rc) return rc;
     CK(cudaMemcpyAsync(ctx->h_pinned, ctx->d_misc2, pb, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     memcpy(out, ctx->h_pinned, pb);
@@ -1509,11 +1536,9 @@ static int msm_api_multi(blsgpu_ctx *lead, const uint8_t *points, const uint8_t 
             break;
         }
         busy[k] = 1;
-        std::string err;
         ctx->launches = 0;
-        int r = msm_run<F>(ctx->msm, base, pb, base + len * pb, sb, len, (int)nbits, ctx->stream, nullptr, (aff_t<F> *)ctx->d_misc2,
-                           &ctx->launches, err);
-        if (r) { rc = fail(lead, r == -1 ? BLSGPU_ERR_CUDA : BLSGPU_ERR_ARG, err.c_str()); break; }
+        int r = run_msm<F>(ctx, base, pb, base + len * pb, sb, len, (int)nbits, ctx->stream, nullptr, (aff_t<F> *)ctx->d_misc2);
+        if (r) { rc = fail(lead, r, ctx->err.c_str()); break; }
         launches += ctx->launches;
         if ((e = cudaMemcpyAsync(ctx->h_pinned, ctx->d_misc2, pb, cudaMemcpyDeviceToHost, ctx->stream)) != cudaSuccess)
             rc = fail(lead, BLSGPU_ERR_CUDA, "cudaMemcpyAsync(msm partial)", e);
@@ -1567,12 +1592,11 @@ extern "C" int blsgpu_combine(blsgpu_ctx *ctx, const uint8_t srb[32], const void
     CK(cudaMemcpyAsync(d_sig, sigs192, n * 192, cudaMemcpyHostToDevice, s));
     ctx->launches = 1;
     k_combine_scalars<<<1, 32, 0, s>>>(words_of(srb), n, (uint64_t *)d_sc);
-    std::string err;
     g1_aff *o1 = (g1_aff *)ctx->d_misc2;
     g2_aff *o2 = (g2_aff *)((uint8_t *)ctx->d_misc2 + 256);
-    rc = msm_run<fp>(ctx->msm, d_pk, 96, d_sc, 8, n, 64, s, nullptr, o1, &ctx->launches, err);
-    if (!rc) rc = msm_run<fp2>(ctx->msm, d_sig, 192, d_sc, 8, n, 64, s, nullptr, o2, &ctx->launches, err);
-    if (rc) return fail(ctx, rc == -1 ? BLSGPU_ERR_CUDA : BLSGPU_ERR_ARG, err.c_str());
+    rc = run_msm<fp>(ctx, d_pk, 96, d_sc, 8, n, 64, s, nullptr, o1);
+    if (!rc) rc = run_msm<fp2>(ctx, d_sig, 192, d_sc, 8, n, 64, s, nullptr, o2);
+    if (rc) return rc;
     CK(cudaMemcpyAsync(ctx->h_pinned, o1, 96, cudaMemcpyDeviceToHost, s));
     CK(cudaMemcpyAsync(ctx->h_pinned + 256, o2, 192, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));

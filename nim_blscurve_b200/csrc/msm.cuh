@@ -20,12 +20,11 @@
 // multiplication at a time.
 // Scalars are NOT reduced mod r (as in the reference); the nbits low bits of each little-endian scalar are used.
 #pragma once
-#include <cstdlib>
-#include <map>
+#include <functional>
 #include <string>
 #include <type_traits>
 #include "kernels.cuh"
-#include "fpprog.hpp"
+#include "route.hpp"
 
 namespace bls {
 
@@ -35,8 +34,6 @@ struct msm_state {
     int sms = 148;                 // SM count of the device (B200: 148); set at context creation
     // window-group pipelining: the latency-bound tail of a group (combine, segment, tree, Horner) runs on this
     // higher-priority stream underneath the bucket accumulation of the next group
-    struct horner_prog { uint32_t *d = nullptr; int nslots = 0, version = 1; };
-    std::map<int, horner_prog> horner;      // window-Horner dataflow programs (fpprog.hpp), keyed by (nwin * 64 + c) * 2 + is_g2
     cudaStream_t tail = nullptr;
     cudaEvent_t ev_group[8] = {}, ev_done = nullptr;
     bool ev_ok = false;
@@ -45,8 +42,6 @@ struct msm_state {
 static inline void msm_free(msm_state &m) {
     if (m.ev_ok) { for (int i = 0; i < 8; i++) cudaEventDestroy(m.ev_group[i]); cudaEventDestroy(m.ev_done); m.ev_ok = false; }
     if (m.tail) { cudaStreamDestroy(m.tail); m.tail = nullptr; }
-    for (auto &kv : m.horner) cudaFree(kv.second.d);
-    m.horner.clear();
     if (m.buf) cudaFree(m.buf);
     m.buf = nullptr;
     m.bytes = 0;
@@ -433,101 +428,31 @@ __global__ void BLS_LB k_msm_make_inputs(uint64_t seed, size_t n, g1_aff *points
     scalars[32 * i + 31] &= 0x7f;
 }
 
-// Window width c and count.  Cost model per candidate c: nwin * (11 n + 32 * 2^(c-1)) field multiplications (one
-// mixed addition per non-zero digit, two full additions per bucket in the reduction).  Signed digits put bit `nbits`
-// (the last carry) into the top window; a top window of only a few bits would funnel n / 2^bits entries into each of
-// its few buckets, so widths that leave it fewer than 6 bits are skipped (for nbits = 255: c = 16, 13, 10, 8 qualify).
-static inline void msm_shape(size_t n, int nbits, int &c, int &nwin) {
-    int lg = 0;
-    while ((n >> (lg + 1)) != 0) lg++;
-    static const int c_env = getenv("BLSGPU_MSM_C") ? atoi(getenv("BLSGPU_MSM_C")) : 0;
-    int best_c = 0;
-    double best = 0.0;
-    const int hi = lg - 2 > 16 ? 16 : lg - 2, lo = lg - 8 < 2 ? 2 : lg - 8;
-    for (int cc = hi; cc >= lo; cc--) {
-        const int nw = (nbits + 1 + cc - 1) / cc, top = nbits + 1 - (nw - 1) * cc;
-        if (nw > 1 && top < (cc < 6 ? cc : 6)) continue;
-        const double cost = (double)nw * (11.0 * (double)n + 32.0 * (double)((size_t)1 << (cc - 1)));
-        if (!best_c || cost < best) { best_c = cc; best = cost; }
-    }
-    if (!best_c) best_c = lg - 4 < 2 ? 2 : (lg - 4 > 16 ? 16 : lg - 4);
-    c = c_env > 0 ? c_env : best_c;
-    nwin = (nbits + 1 + c - 1) / c;
-}
-
 // Stream-ordered: d_points (stride pstride bytes, aff_t<F> each) and d_scalars (stride sstride bytes, little-endian,
 // nbits bits used) are device pointers; the sum lands in d_out_jac and/or d_out_aff (device, either may be null).
+// p is the shape route::plan_msm chose for (n, nbits).  horner_prog, when set, launches the window-Horner dataflow
+// program of that shape on (stream, homogeneous window sums, homogeneous result); otherwise k_msm_horner runs.
 // No host synchronisation unless the scratch buffer has to grow.
 template <class F>
-static inline int msm_run(msm_state &st, const uint8_t *d_points, size_t pstride, const uint8_t *d_scalars, size_t sstride,
-                          size_t n, int nbits, cudaStream_t s, jac_t<F> *d_out_jac, aff_t<F> *d_out_aff, int *launches,
-                          std::string &err) {
+static inline int msm_run(msm_state &st, const route::msm_plan &p,
+                          const std::function<void(cudaStream_t, const fp *, fp *)> &horner_prog, const uint8_t *d_points,
+                          size_t pstride, const uint8_t *d_scalars, size_t sstride, size_t n, int nbits, cudaStream_t s,
+                          jac_t<F> *d_out_jac, aff_t<F> *d_out_aff, int *launches, std::string &err) {
     typedef jac_t<F> J;
     if (n >= ((size_t)1 << 31)) { err = "msm: too many points"; return -2; }
     const int sb = (nbits + 7) / 8;
-    int c, nwin;
-    msm_shape(n, nbits, c, nwin);
-    const size_t B = (size_t)1 << (c - 1);
-    const size_t nb = (size_t)nwin * B;
-    const size_t emax = n * (size_t)nwin;
-    const size_t wave = (size_t)st.sms * BLS_LB_BLOCKS * 128;
-    size_t L = B / 512;                            // segment length: short serial chains, <= 512 segments per window
-    if (L < 4) L = 4;
-    if (L > 32) L = 32;
-    static const int l_env = getenv("BLSGPU_MSM_L") ? atoi(getenv("BLSGPU_MSM_L")) : 0;
-    if (l_env > 0) L = (size_t)l_env;
-    if (L > B) L = B;
-    const size_t nseg = B / L;
-    // Window groups, top windows first.  The tail of a group is latency-bound (a few thousand threads, then one), so
-    // it runs on the tail stream while the main stream accumulates the buckets of the next group.
-    static const int g_env = getenv("BLSGPU_MSM_GROUPS") ? atoi(getenv("BLSGPU_MSM_GROUPS")) : 0;
-    int G = g_env > 0 ? g_env : 1;
-    if (G > 8) G = 8;
-    if (G > nwin) G = nwin;
-    int gw0[9];                                    // group g = windows [gw0[g+1], gw0[g]) counted from the top
-    gw0[0] = nwin;
-    for (int g = 0; g < G; g++) gw0[g + 1] = nwin - (int)(((size_t)nwin * (g + 1)) / G);
-    // entries per chunk, per group: the chunk grid of a group fills whole waves of the resident-thread capacity
-    // (SMs x 4 blocks x 128) with about 32 additions per thread; short MSMs get one wave of shorter chunks
-    uint32_t Kg[8];
-    size_t preg[9];                                // partial-slot regions: chunks of the group + its buckets + 1
-    preg[0] = 0;
-    for (int g = 0; g < G; g++) {
-        const size_t wg = (size_t)(gw0[g] - gw0[g + 1]), eg = n * wg;
-        size_t waves = eg / (wave * 32);
-        if (waves < 1) waves = 1;
-        size_t Kz = (eg + waves * wave - 1) / (waves * wave);
-        if (Kz < 8) Kz = 8;
-        static const int k_env = getenv("BLSGPU_MSM_K") ? atoi(getenv("BLSGPU_MSM_K")) : 0;
-        if (k_env > 0) Kz = (size_t)k_env;
-        Kg[g] = (uint32_t)Kz;
-        preg[g + 1] = preg[g] + (eg + Kz - 1) / Kz + 1 + wg * B + 1;
-    }
-    const size_t pmax = preg[G];
-    const size_t nsb = (nb + 1023) / 1024;         // scan blocks
-    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
-    size_t o_counts = 0;
-    size_t o_offsets = o_counts + al(nb * 4);
-    size_t o_cursor = o_offsets + al((nb + 1) * 4);
-    size_t o_rank = o_cursor + al(nb * 4);
-    size_t o_bsums = o_rank + al((nb + 1) * 4);
-    size_t o_big = o_bsums + al(nsb * 8);
-    size_t o_bigcount = o_big + al(nb * 4);
-    size_t o_carry = o_bigcount + 256;
-    size_t o_hom = o_carry + al(sizeof(J));
-    size_t o_entries = o_hom + al((size_t)(6 * nwin + 6) * 48);
-    size_t o_partials = o_entries + al(emax * 4);
-    size_t o_buckets = o_partials + al(pmax * sizeof(J));
-    size_t o_segs = o_buckets + al(nb * sizeof(J));
-    size_t total = o_segs + al((size_t)nwin * nseg * sizeof(J));
+    const int c = p.c, nwin = p.nwin, G = p.G;
+    const size_t B = p.B, nseg = p.nseg;
+    const size_t nb = (size_t)nwin * B, nsb = (nb + 1023) / 1024;
+    const route::msm_layout o = route::msm_scratch(p, sizeof(J));
     cudaError_t e;
 #define MCK(call) if ((e = (call)) != cudaSuccess) { err = std::string(#call ": ") + cudaGetErrorString(e); return -1; }
-    if (st.bytes < total) {
+    if (st.bytes < o.total) {
         if (st.buf) { MCK(cudaStreamSynchronize(s)); if (st.tail) MCK(cudaStreamSynchronize(st.tail)); cudaFree(st.buf); }
         st.buf = nullptr;
         st.bytes = 0;
-        MCK(cudaMalloc((void **)&st.buf, total));
-        st.bytes = total;
+        MCK(cudaMalloc((void **)&st.buf, o.total));
+        st.bytes = o.total;
     }
     if (G > 1 && !st.tail) {
         int lo_pri = 0, hi_pri = 0;
@@ -537,13 +462,13 @@ static inline int msm_run(msm_state &st, const uint8_t *d_points, size_t pstride
         MCK(cudaEventCreateWithFlags(&st.ev_done, cudaEventDisableTiming));
         st.ev_ok = true;
     }
-    uint32_t *counts = (uint32_t *)(st.buf + o_counts), *offsets = (uint32_t *)(st.buf + o_offsets);
-    uint32_t *cursor = (uint32_t *)(st.buf + o_cursor), *rank = (uint32_t *)(st.buf + o_rank);
-    uint32_t *bsums = (uint32_t *)(st.buf + o_bsums);
-    uint32_t *biglist = (uint32_t *)(st.buf + o_big), *bigcount = (uint32_t *)(st.buf + o_bigcount);
-    uint32_t *entries = (uint32_t *)(st.buf + o_entries);
-    J *partials = (J *)(st.buf + o_partials), *buckets = (J *)(st.buf + o_buckets), *segs = (J *)(st.buf + o_segs);
-    J *carry = (J *)(st.buf + o_carry);
+    uint32_t *counts = (uint32_t *)(st.buf + o.counts), *offsets = (uint32_t *)(st.buf + o.offsets);
+    uint32_t *cursor = (uint32_t *)(st.buf + o.cursor), *rank = (uint32_t *)(st.buf + o.rank);
+    uint32_t *bsums = (uint32_t *)(st.buf + o.bsums);
+    uint32_t *biglist = (uint32_t *)(st.buf + o.big), *bigcount = (uint32_t *)(st.buf + o.bigcount);
+    uint32_t *entries = (uint32_t *)(st.buf + o.entries);
+    J *partials = (J *)(st.buf + o.partials), *buckets = (J *)(st.buf + o.buckets), *segs = (J *)(st.buf + o.segs);
+    J *carry = (J *)(st.buf + o.carry);
     MCK(cudaMemsetAsync(counts, 0, nb * 4, s));
     MCK(cudaMemsetAsync(bigcount, 0, 4 * 8, s));
     int nl = 0;
@@ -554,11 +479,11 @@ static inline int msm_run(msm_state &st, const uint8_t *d_points, size_t pstride
     k_msm_scatter<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(d_scalars, sstride, n, sb, nbits, c, nwin, cursor, entries);
     nl += 5;
     for (int g = 0; g < G; g++) {
-        const int w0 = gw0[g + 1], wg = gw0[g] - gw0[g + 1];
+        const int w0 = p.gw0[g + 1], wg = p.gw0[g] - p.gw0[g + 1];
         const size_t b0 = (size_t)w0 * B, b1 = b0 + (size_t)wg * B;
-        const uint32_t K = Kg[g];
+        const uint32_t K = p.K[g];
         const size_t gchunks = (n * (size_t)wg + K - 1) / K + 1;
-        J *pg = partials + preg[g];
+        J *pg = partials + p.preg[g];
         k_msm_chunks<F><<<(unsigned)((gchunks + 127) / 128), 128, 0, s>>>(d_points, pstride, offsets, rank, entries, b0, b1, K, pg);
         cudaStream_t ts = s;
         if (G > 1) {
@@ -570,7 +495,7 @@ static inline int msm_run(msm_state &st, const uint8_t *d_points, size_t pstride
         k_msm_combine_big<F><<<128, 128, 0, ts>>>(pg, offsets, rank, b0, K, biglist, bigcount + g, buckets);
         size_t nt = (size_t)wg * nseg;
         J *sg = segs + (size_t)w0 * nseg;
-        k_msm_segment<F><<<(unsigned)((nt + 127) / 128), 128, 0, ts>>>(buckets + b0, c, wg, (uint32_t)L, sg);
+        k_msm_segment<F><<<(unsigned)((nt + 127) / 128), 128, 0, ts>>>(buckets + b0, c, wg, (uint32_t)p.L, sg);
         nl += 4;
         for (size_t m = nseg; m > 1;) {
             size_t half = (m + 1) / 2;
@@ -578,43 +503,17 @@ static inline int msm_run(msm_state &st, const uint8_t *d_points, size_t pstride
             nl++;
             m = half;
         }
-        bool programmed = false;
-        {
-            static const bool prog_env = !(getenv("BLSGPU_MSM_HORNER_PROG") && atoi(getenv("BLSGPU_MSM_HORNER_PROG")) == 0);
+        if (p.horner_prog && horner_prog) {                  // p.horner_prog: G == 1
             constexpr bool is_g1 = std::is_same<F, fp>::value;
             constexpr int per = is_g1 ? 3 : 6;               // field elements per homogeneous point
-            if (G == 1 && nwin <= 128 && prog_env) {
-                msm_state::horner_prog hp;
-                const int key = (nwin * 64 + c) * 2 + (is_g1 ? 0 : 1);
-                auto it = st.horner.find(key);
-                if (it != st.horner.end()) hp = it->second;
-                else {
-                    fpprog::Program P = is_g1 ? fpprog::build_msm_horner_g1(nwin, c) : fpprog::build_msm_horner_g2(nwin, c);
-                    if (P.ok && (size_t)P.nslots * sizeof(fp) <= 48 * 1024) {
-                        MCK(cudaMalloc((void **)&hp.d, P.words.size() * 4));
-                        MCK(cudaMemcpyAsync(hp.d, P.words.data(), P.words.size() * 4, cudaMemcpyHostToDevice, s));
-                        MCK(cudaStreamSynchronize(s));       // first use of this shape only: the host vector goes away
-                        hp.nslots = P.nslots;
-                        hp.version = P.version;
-                    }
-                    st.horner[key] = hp;
-                }
-                if (hp.d) {
-                    fp *hom = (fp *)(st.buf + o_hom);
-                    if constexpr (is_g1) k_msm_horner_prep<<<1, 128, 0, ts>>>(sg, nseg, nwin, hom);
-                    else k_msm_horner_prep_g2<<<1, 128, 0, ts>>>(sg, nseg, nwin, hom);
-                    if (hp.version == 2)
-                        k_fp_program2<<<1, 32, (size_t)hp.nslots * sizeof(fp), ts>>>(hp.d, hom, nullptr, nullptr, hom + per * nwin, 0, 0, 0);
-                    else
-                        k_fp_program<<<1, 32, (size_t)hp.nslots * sizeof(fp), ts>>>(hp.d, hom, nullptr, nullptr, hom + per * nwin, 0, 0, 0);
-                    if constexpr (is_g1) k_msm_horner_finish<<<1, 32, 0, ts>>>(hom + per * nwin, d_out_jac, d_out_aff);
-                    else k_msm_horner_finish_g2<<<1, 32, 0, ts>>>(hom + per * nwin, d_out_jac, d_out_aff);
-                    nl += 3;
-                    programmed = true;
-                }
-            }
-        }
-        if (!programmed) {
+            fp *hom = (fp *)(st.buf + o.hom);
+            if constexpr (is_g1) k_msm_horner_prep<<<1, 128, 0, ts>>>(sg, nseg, nwin, hom);
+            else k_msm_horner_prep_g2<<<1, 128, 0, ts>>>(sg, nseg, nwin, hom);
+            horner_prog(ts, hom, hom + per * nwin);
+            if constexpr (is_g1) k_msm_horner_finish<<<1, 32, 0, ts>>>(hom + per * nwin, d_out_jac, d_out_aff);
+            else k_msm_horner_finish_g2<<<1, 32, 0, ts>>>(hom + per * nwin, d_out_jac, d_out_aff);
+            nl += 2;                                         // horner_prog counts its own launch
+        } else {
             k_msm_horner<F><<<1, 32, 0, ts>>>(sg, nseg, wg, c, g == 0, g == G - 1, carry, d_out_jac, d_out_aff);
             nl++;
         }

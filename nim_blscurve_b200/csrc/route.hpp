@@ -1,9 +1,11 @@
 // route.hpp — the batch pipeline's route policy: which kernels a batch of n sets runs, and the measured size thresholds
-// that decide it.  Plain C++ without CUDA, so that tests/hostsim compiles it and checks the plans on the host.
+// that decide it; and the shape of the Pippenger MSM (window width, segments, window groups, chunks, scratch layout).
+// Plain C++ without CUDA, so that tests/hostsim compiles it and checks the plans on the host.
 //
 // Every threshold is read from the environment by read_thresholds() (INTEGRATION.md section 8); libblsgpu caches the
 // result once per process.  The per-context switches (BLSGPU_SIDE_STREAM, BLSGPU_ACC_TEAM, BLSGPU_SERIAL_TAIL,
-// BLSGPU_GRAPH) are read by blsgpu_create and come in through `switches`.
+// BLSGPU_GRAPH) are read by blsgpu_create and come in through `switches`.  BLSGPU_PROG_FORMAT is the one variable read
+// elsewhere, by fpprog.hpp, whose tests override it per thread.
 #pragma once
 #include <stddef.h>
 #include <stdint.h>
@@ -18,6 +20,7 @@ namespace route {
 static const size_t SMALL_ROUTE_CAP = 4096;
 static const size_t SMALL_LINES_CAP = 16385;
 static const unsigned ACC_BLOCK = 128;               // threads per block of k_miller_acc (BLS_ACC_BS)
+static const unsigned LB_BLOCKS = 4;                 // resident 128-thread blocks per SM of the BLS_LB kernels (BLS_LB_BLOCKS)
 
 enum { SMALL_HASH = 1, SMALL_SIG = 2, SMALL_LINES = 4, SMALL_GTPROD = 8 };   // bits of BLSGPU_SMALL_ROUTE
 
@@ -34,6 +37,8 @@ struct thresholds {
     int map_lanes2, acc_old_rule;
     bool miller_g_set, miller_nseg_set;              // BLSGPU_MILLER_G / _NSEG override the shape rule of miller_shape
     int miller_g, miller_nseg;
+    int msm_c, msm_l, msm_groups, msm_k;             // BLSGPU_MSM_C / _L / _GROUPS / _K override the MSM shape when > 0
+    bool msm_horner_prog;                            // BLSGPU_MSM_HORNER_PROG=0 keeps the window Horner off the program
 };
 
 inline size_t env_size(const char *name, size_t def) { const char *e = getenv(name); return e ? (size_t)atoll(e) : def; }
@@ -85,6 +90,11 @@ inline thresholds read_thresholds() {
     t.miller_g = g ? atoi(g) : 0;
     t.miller_nseg_set = ns != nullptr;
     t.miller_nseg = ns ? atoi(ns) : 0;
+    t.msm_c = env_int("BLSGPU_MSM_C", 0);
+    t.msm_l = env_int("BLSGPU_MSM_L", 0);
+    t.msm_groups = env_int("BLSGPU_MSM_GROUPS", 0);
+    t.msm_k = env_int("BLSGPU_MSM_K", 0);
+    t.msm_horner_prog = env_int("BLSGPU_MSM_HORNER_PROG", 1) != 0;
     return t;
 }
 
@@ -256,6 +266,102 @@ inline miller_plan plan_miller(const thresholds &t, size_t np, size_t lines_cap,
         p.lines_last = last <= t.pair_lines_max ? LINES_LANES2 : LINES_THREAD;
     }
     return p;
+}
+
+// Window width c and count.  Cost model per candidate c: nwin * (11 n + 32 * 2^(c-1)) field multiplications (one
+// mixed addition per non-zero digit, two full additions per bucket in the reduction).  Signed digits put bit `nbits`
+// (the last carry) into the top window; a top window of only a few bits would funnel n / 2^bits entries into each of
+// its few buckets, so widths that leave it fewer than 6 bits are skipped (for nbits = 255: c = 16, 13, 10, 8 qualify).
+inline void msm_shape(const thresholds &t, size_t n, int nbits, int &c, int &nwin) {
+    int lg = 0;
+    while ((n >> (lg + 1)) != 0) lg++;
+    int best_c = 0;
+    double best = 0.0;
+    const int hi = lg - 2 > 16 ? 16 : lg - 2, lo = lg - 8 < 2 ? 2 : lg - 8;
+    for (int cc = hi; cc >= lo; cc--) {
+        const int nw = (nbits + 1 + cc - 1) / cc, top = nbits + 1 - (nw - 1) * cc;
+        if (nw > 1 && top < (cc < 6 ? cc : 6)) continue;
+        const double cost = (double)nw * (11.0 * (double)n + 32.0 * (double)((size_t)1 << (cc - 1)));
+        if (!best_c || cost < best) { best_c = cc; best = cost; }
+    }
+    if (!best_c) best_c = lg - 4 < 2 ? 2 : (lg - 4 > 16 ? 16 : lg - 4);
+    c = t.msm_c > 0 ? t.msm_c : best_c;
+    nwin = (nbits + 1 + c - 1) / c;
+}
+
+struct msm_plan {
+    int c, nwin;           // window width, windows
+    size_t B;              // buckets per window: digit magnitudes 1 .. 2^(c-1)
+    size_t L, nseg;        // buckets per segment, segments per window
+    int G;                 // window groups, top windows first
+    int gw0[9];            // group g = windows [gw0[g+1], gw0[g]) counted from the top
+    uint32_t K[8];         // entries per chunk of group g
+    size_t preg[9];        // partial-slot region of group g: [preg[g], preg[g+1])
+    size_t emax;           // entries of the bucket-sorted list: n * nwin
+    bool horner_prog;      // the window Horner may run as a dataflow program (if its program builds)
+};
+
+// n points with nbits-bit scalars on a device of `sms` SMs
+inline msm_plan plan_msm(const thresholds &t, size_t n, int nbits, int sms) {
+    msm_plan p;
+    msm_shape(t, n, nbits, p.c, p.nwin);
+    p.B = (size_t)1 << (p.c - 1);
+    p.emax = n * (size_t)p.nwin;
+    const size_t wave = (size_t)sms * LB_BLOCKS * 128;
+    size_t L = p.B / 512;                          // segment length: short serial chains, <= 512 segments per window
+    if (L < 4) L = 4;
+    if (L > 32) L = 32;
+    if (t.msm_l > 0) L = (size_t)t.msm_l;
+    if (L > p.B) L = p.B;
+    p.L = L;
+    p.nseg = p.B / L;
+    // Window groups, top windows first.  The tail of a group is latency-bound (a few thousand threads, then one), so
+    // it runs on the tail stream while the main stream accumulates the buckets of the next group.
+    int G = t.msm_groups > 0 ? t.msm_groups : 1;
+    if (G > 8) G = 8;
+    if (G > p.nwin) G = p.nwin;
+    p.G = G;
+    p.gw0[0] = p.nwin;
+    for (int g = 0; g < G; g++) p.gw0[g + 1] = p.nwin - (int)(((size_t)p.nwin * (g + 1)) / G);
+    // entries per chunk, per group: the chunk grid of a group fills whole waves of the resident-thread capacity
+    // (SMs x 4 blocks x 128) with about 32 additions per thread; short MSMs get one wave of shorter chunks
+    p.preg[0] = 0;                                 // partial slots of a group: its chunks + its buckets + 1
+    for (int g = 0; g < G; g++) {
+        const size_t wg = (size_t)(p.gw0[g] - p.gw0[g + 1]), eg = n * wg;
+        size_t waves = eg / (wave * 32);
+        if (waves < 1) waves = 1;
+        size_t Kz = (eg + waves * wave - 1) / (waves * wave);
+        if (Kz < 8) Kz = 8;
+        if (t.msm_k > 0) Kz = (size_t)t.msm_k;
+        p.K[g] = (uint32_t)Kz;
+        p.preg[g + 1] = p.preg[g] + (eg + Kz - 1) / Kz + 1 + wg * p.B + 1;
+    }
+    p.horner_prog = G == 1 && p.nwin <= 128 && t.msm_horner_prog;
+    return p;
+}
+
+// byte offsets into the MSM's scratch buffer, for Jacobian points of jac_bytes bytes
+struct msm_layout { size_t counts, offsets, cursor, rank, bsums, big, bigcount, carry, hom, entries, partials, buckets, segs, total; };
+
+inline msm_layout msm_scratch(const msm_plan &p, size_t jac_bytes) {
+    const size_t nb = (size_t)p.nwin * p.B, nsb = (nb + 1023) / 1024;   // buckets, scan blocks
+    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
+    msm_layout o;
+    o.counts = 0;
+    o.offsets = o.counts + al(nb * 4);
+    o.cursor = o.offsets + al((nb + 1) * 4);
+    o.rank = o.cursor + al(nb * 4);
+    o.bsums = o.rank + al((nb + 1) * 4);
+    o.big = o.bsums + al(nsb * 8);
+    o.bigcount = o.big + al(nb * 4);
+    o.carry = o.bigcount + 256;
+    o.hom = o.carry + al(jac_bytes);
+    o.entries = o.hom + al((size_t)(6 * p.nwin + 6) * 48);
+    o.partials = o.entries + al(p.emax * 4);
+    o.buckets = o.partials + al(p.preg[p.G] * jac_bytes);
+    o.segs = o.buckets + al(nb * jac_bytes);
+    o.total = o.segs + al((size_t)p.nwin * p.nseg * jac_bytes);
+    return o;
 }
 
 }  // namespace route

@@ -289,7 +289,7 @@ int hs_signature_from_bytes(const uint8_t *in, int len, int group_check, g2_aff 
 void hs_g1_compress(const g1_aff *p, uint8_t *out) { g1_compress(out, *p); }
 void hs_miller_combine(const fp12 *seg, int nseg, fp12 *out) { miller_combine(*out, seg, nseg); }
 
-// ---- route.hpp: the plans of the batch pipeline, thresholds read from the environment at every call ----
+// ---- route.hpp: the plans of the batch pipeline and of the MSM, thresholds read from the environment at every call ----
 // out: the fields of route::batch_plan in declaration order
 void hs_plan_batch(size_t n, size_t total_n, uint32_t chunks, int host_src, int scalars, int use_side, int acc_team,
                    int serial_tail, int use_graph, int *out) {
@@ -304,5 +304,18 @@ void hs_plan_miller(size_t np, size_t lines_cap, int team, int serial_tail, long
     const route::miller_plan p = route::plan_miller(route::read_thresholds(), np, lines_cap, team != 0, serial_tail != 0);
     const long long v[6] = {p.G, p.nseg, p.lines, p.lines_last, (long long)p.ncols, p.gt_prog};
     memcpy(out, v, sizeof v);
+}
+// out: c, nwin, B, L, nseg, G, emax, horner_prog, scratch bytes of the G1 and of the G2 MSM, gw0[0..G], K[0..G-1],
+// preg[0..G]
+void hs_plan_msm(size_t n, int nbits, int sms, long long *out) {
+    const route::msm_plan p = route::plan_msm(route::read_thresholds(), n, nbits, sms);
+    const long long v[10] = {p.c, p.nwin, (long long)p.B, (long long)p.L, (long long)p.nseg, p.G, (long long)p.emax,
+                             p.horner_prog, (long long)route::msm_scratch(p, sizeof(g1_jac)).total,
+                             (long long)route::msm_scratch(p, sizeof(g2_jac)).total};
+    memcpy(out, v, sizeof v);
+    long long *o = out + 10;
+    for (int g = 0; g <= p.G; g++) *o++ = p.gw0[g];
+    for (int g = 0; g < p.G; g++) *o++ = p.K[g];
+    for (int g = 0; g <= p.G; g++) *o++ = (long long)p.preg[g];
 }
 }

@@ -453,8 +453,10 @@ def test_route_plans(hs, monkeypatch):
     """route.hpp: the batch plan (hash route, host copy, small-route buffers, signature sum, streams, affine mode, scalar
     chain, graph replay) and the Miller plan (G, segments, lines route of each tile, GT product) at the size boundaries of
     the pipeline, with and without a host source, explicit scalars and the serial tail, under the default thresholds and
-    under non-default ones (clamps included).  tests/golden/route_plans.json holds the routes the batch pipeline took for
-    these inputs before its decisions moved into route.hpp."""
+    under non-default ones (clamps included).  The MSM plan (window width, segments, window groups, chunk lengths,
+    partial-slot regions, Horner program, scratch bytes of the G1 and the G2 MSM) for 1 to 2^22 points, 1 to 256 scalar
+    bits and two SM counts, under the default shape and every BLSGPU_MSM_* override.  tests/golden/route_plans.json
+    holds the routes and shapes the library chose for these inputs before its decisions moved into route.hpp."""
     d = json.load(open(os.path.join(GOLD, "route_plans.json")))
     names = {"hash": ["program", "lanes2", "pair", "thread"], "sig": ["program", "mul", "msm"],
              "affine": ["default", "warp", "block"], "lines": ["program", "lanes2", "thread"]}
@@ -476,5 +478,17 @@ def test_route_plans(hs, monkeypatch):
             hs.hs_plan_miller(C.c_size_t(np_), C.c_size_t(cap), team, serial, o)
             got = [names[f][v] if f in names else v for f, v in zip(d["miller_plan"], o)]
             assert got == want, (cfg["env"], inp)
+        for k in cfg["env"]:
+            monkeypatch.delenv(k)
+    for cfg in d["msm"]:
+        for k, v in cfg["env"].items():
+            monkeypatch.setenv(k, v)
+        for inp, want in cfg["plans"]:
+            n, nbits, sms = inp
+            o = (C.c_longlong * 37)()
+            hs.hs_plan_msm(C.c_size_t(n), nbits, sms, o)
+            c, nwin, B, L, nseg, G, emax, prog, bytes_g1, bytes_g2 = o[:10]
+            gw0, K, preg = o[10:11 + G], o[11 + G:11 + 2 * G], o[11 + 2 * G:12 + 3 * G]
+            assert [c, nwin, B, L, nseg, G, gw0, K, preg, emax, prog, bytes_g1, bytes_g2] == want, (cfg["env"], inp)
         for k in cfg["env"]:
             monkeypatch.delenv(k)
