@@ -201,6 +201,35 @@ int blsgpu_last_launches(const blsgpu_ctx *ctx);
 /* Fp unit ops on the device: op 0=mul 1=add 2=sub 3=sqr 4=inverse (Fermat) 6=inverse (binary Euclid); a,b,out: n x 48
  * bytes (Montgomery). */
 int blsgpu_test_fp(blsgpu_ctx *ctx, int op, const void *a, const void *b, size_t n, void *out);
+/* One device field primitive on n records, through the functions the pipelines call.  A record is field elements
+ * (48 B each, Montgomery, little-endian) followed by an op-specific tail of u32 words padded to 16 B; in_rec_bytes and
+ * out_rec_bytes must be the op's sizes, else (or for an unknown op) BLSGPU_ERR_ARG.  Per op, inputs -> outputs:
+ *   Fp, one thread per record:    FP_MUL, FP_MUL_NI (a, b -> a b/R);  FP_SQR, FP_SQR_NI (a -> a^2/R);  FP_ADD, FP_SUB
+ *                                 (a, b -> a +- b);  FP_NEG, FP_INV, FP_INV_VARTIME, FP_POW_P34, FP_FROM_MONT (a -> r);
+ *                                 FP_PARITY, FP_IS_LEXICALLY_LARGEST_CANON (a -> word)
+ *   Fp2, one thread per record:   FP2_MUL (a, b -> r);  FP2_SQR, FP2_MUL_XI, FP2_INV, FP2_INV_VARTIME (a -> r);
+ *                                 FP2_MUL_FP (a, Fp k -> r);  FP2_RSQRT_OR_Z (a -> r, word is_square);
+ *                                 FP2_SGN0, FP2_IS_LEXICALLY_LARGEST (a -> word)
+ *   Fp2 on a lane pair (fp2h):    H_MUL (a, b -> r);  H_SQR, H_MUL_XI, H_CONJ, H_INV (a -> r);  H_MUL_FP (a, Fp k -> r)
+ *   one lane of a six-lane team:  TEAM_DOT3 (a0..a2, b0..b2 -> sum a_t b_t / R);  TEAM_DOT4 (a0..a3, b0..b3, words
+ *                                 dbl_mask, zero_mask -> the same with a_t doubled / zeroed per mask bit)
+ *   one six-lane team:            TEAM_MUL_LINE (Fp12 f in tower order, line l0 l1 l2 -> f * line);
+ *                                 TEAM_SQUARE (f -> f^2)
+ *   Fp, one thread per record:    LIN_FINISH (x0..x6 positive, x7..x13 negative, words m0..m13 in 0..15 ->
+ *                                 sum m_j x_j over the positive terms minus the negative ones, mod p) */
+enum {
+    BLSGPU_TF_FP_MUL, BLSGPU_TF_FP_MUL_NI, BLSGPU_TF_FP_SQR, BLSGPU_TF_FP_SQR_NI, BLSGPU_TF_FP_ADD, BLSGPU_TF_FP_SUB,
+    BLSGPU_TF_FP_NEG, BLSGPU_TF_FP_INV, BLSGPU_TF_FP_INV_VARTIME, BLSGPU_TF_FP_POW_P34, BLSGPU_TF_FP_FROM_MONT,
+    BLSGPU_TF_FP_PARITY, BLSGPU_TF_FP_IS_LEXICALLY_LARGEST_CANON,
+    BLSGPU_TF_FP2_MUL, BLSGPU_TF_FP2_SQR, BLSGPU_TF_FP2_MUL_XI, BLSGPU_TF_FP2_MUL_FP, BLSGPU_TF_FP2_INV,
+    BLSGPU_TF_FP2_INV_VARTIME, BLSGPU_TF_FP2_RSQRT_OR_Z, BLSGPU_TF_FP2_SGN0, BLSGPU_TF_FP2_IS_LEXICALLY_LARGEST,
+    BLSGPU_TF_H_MUL, BLSGPU_TF_H_SQR, BLSGPU_TF_H_MUL_XI, BLSGPU_TF_H_MUL_FP, BLSGPU_TF_H_CONJ, BLSGPU_TF_H_INV,
+    BLSGPU_TF_TEAM_DOT3, BLSGPU_TF_TEAM_DOT4, BLSGPU_TF_TEAM_MUL_LINE, BLSGPU_TF_TEAM_SQUARE,
+    BLSGPU_TF_LIN_FINISH,
+    BLSGPU_TF_COUNT
+};
+int blsgpu_test_field(blsgpu_ctx *ctx, int op, const void *in, size_t in_rec_bytes, size_t n, void *out,
+                      size_t out_rec_bytes);
 /* The message hash of the small-batch route (two-lane map kernel, then the cofactor-clearing dataflow program):
  * n <= 4096 sets in (host, 320 B each); out_in / out_out (nullable): n x 6 field elements (48 B each, Montgomery) =
  * the homogeneous E2 point (X : Y : Z) before / after the program.  H(m_i) = (X/Z, Y/Z) of out_out. */

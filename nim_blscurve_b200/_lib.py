@@ -17,7 +17,7 @@ SYMBOLS = [
     "blsgpu_msm_g1", "blsgpu_msm_g1_dev", "blsgpu_msm_g2", "blsgpu_msm_g2_dev", "blsgpu_combine", "blsgpu_last_stage_ms", "blsgpu_stage_name", "blsgpu_last_launches",
     "blsgpu_subtract_g1", "blsgpu_subtract_g2", "blsgpu_aggregate_g1_segments", "blsgpu_aggregate_verify", "blsgpu_fast_aggregate_verify",
     "blsgpu_pubkeys_from_bytes", "blsgpu_signatures_from_bytes", "blsgpu_pubkeys_to_bytes", "blsgpu_signatures_to_bytes",
-    "blsgpu_test_fp", "blsgpu_test_small_hash", "blsgpu_imad_peak", "blsgpu_fpmul_peak", "blsgpu_make_sets", "blsgpu_msm_make_inputs",
+    "blsgpu_test_fp", "blsgpu_test_field", "blsgpu_test_small_hash", "blsgpu_imad_peak", "blsgpu_fpmul_peak", "blsgpu_make_sets", "blsgpu_msm_make_inputs",
 ]
 
 _lib = None
@@ -78,6 +78,7 @@ def lib():
     L.blsgpu_stage_name.argtypes = [C.c_int]
     L.blsgpu_last_launches.argtypes = [vp]
     L.blsgpu_test_fp.argtypes = [vp, C.c_int, vp, vp, sz, vp]
+    L.blsgpu_test_field.argtypes = [vp, C.c_int, vp, sz, sz, vp, sz]
     L.blsgpu_imad_peak.restype = C.c_double
     L.blsgpu_imad_peak.argtypes = [vp, C.c_int]
     L.blsgpu_fpmul_peak.restype = C.c_double

@@ -1624,19 +1624,55 @@ extern "C" int blsgpu_last_stage_ms(const blsgpu_ctx *ctx, float *ms, int max) {
 extern "C" const char *blsgpu_stage_name(int stage) { return stage >= 0 && stage < ST_COUNT ? STAGE_NAMES[stage] : ""; }
 extern "C" int blsgpu_last_launches(const blsgpu_ctx *ctx) { return ctx ? ctx->launches : 0; }
 
+// n records of field test op `op` from d_in to d_out (device scratch), on the context's stream
+static int launch_test_field(blsgpu_ctx *ctx, int op, const uint8_t *d_in, size_t n, uint8_t *d_out) {
+    const test_field_shape &sh = TEST_FIELD_OPS[op];
+    const size_t per_block = sh.geom == TF_THREAD ? ACC_BS : sh.geom == TF_PAIR ? ACC_BS / 2
+                           : sh.geom == TF_TEAM_LANE ? 6 * ACC_TPB : ACC_TPB;
+    k_test_field<<<nblk(n, (unsigned)per_block), ACC_BS, 0, ctx->stream>>>(op, d_in, test_field_rec(sh.nin, sh.nin_w), n, d_out,
+                                                                         test_field_rec(sh.nout, sh.nout_w));
+    CK(cudaGetLastError());
+    return 0;
+}
+
+extern "C" int blsgpu_test_field(blsgpu_ctx *ctx, int op, const void *in, size_t in_rec_bytes, size_t n, void *out,
+                                 size_t out_rec_bytes) {
+    if (!ctx) return BLSGPU_ERR_ARG;
+    if (op < 0 || op >= BLSGPU_TF_COUNT) return fail(ctx, BLSGPU_ERR_ARG, "unknown field test op");
+    const test_field_shape &sh = TEST_FIELD_OPS[op];
+    if (in_rec_bytes != test_field_rec(sh.nin, sh.nin_w) || out_rec_bytes != test_field_rec(sh.nout, sh.nout_w))
+        return fail(ctx, BLSGPU_ERR_ARG, "record size does not match the field test op");
+    if (n == 0) return 0;
+    if (!in || !out) return BLSGPU_ERR_ARG;
+    CK(cudaSetDevice(ctx->device));
+    int rc = ensure_misc(ctx, n * (in_rec_bytes + out_rec_bytes));
+    if (rc) return rc;
+    uint8_t *d_in = (uint8_t *)ctx->d_misc, *d_out = d_in + n * in_rec_bytes;
+    cudaStream_t s = ctx->stream;
+    CK(cudaMemcpyAsync(d_in, in, n * in_rec_bytes, cudaMemcpyHostToDevice, s));
+    rc = launch_test_field(ctx, op, d_in, n, d_out);
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(out, d_out, n * out_rec_bytes, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    return 0;
+}
+
 extern "C" int blsgpu_test_fp(blsgpu_ctx *ctx, int op, const void *a, const void *b, size_t n, void *out) {
     if (!ctx || !a || !out) return BLSGPU_ERR_ARG;
     if (n == 0) return 0;
     CK(cudaSetDevice(ctx->device));
-    int rc = ensure_misc(ctx, 3 * n * 48);
+    const int fop = op == 0 ? BLSGPU_TF_FP_MUL : op == 1 ? BLSGPU_TF_FP_ADD : op == 2 ? BLSGPU_TF_FP_SUB
+                  : op == 3 ? BLSGPU_TF_FP_SQR : op == 6 ? BLSGPU_TF_FP_INV_VARTIME : BLSGPU_TF_FP_INV;
+    const size_t rec = 48 * (size_t)TEST_FIELD_OPS[fop].nin;   // a, or a and b (b = a when NULL) side by side
+    int rc = ensure_misc(ctx, n * (rec + 48));
     if (rc) return rc;
-    fp *da = (fp *)ctx->d_misc, *db = da + n, *dout = db + n;
+    uint8_t *d_in = (uint8_t *)ctx->d_misc, *d_out = d_in + n * rec;
     cudaStream_t s = ctx->stream;
-    CK(cudaMemcpyAsync(da, a, n * 48, cudaMemcpyHostToDevice, s));
-    if (b) CK(cudaMemcpyAsync(db, b, n * 48, cudaMemcpyHostToDevice, s));
-    k_test_fp<<<nblk(n), 128, 0, s>>>(op, da, b ? db : nullptr, n, dout);
-    CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(out, dout, n * 48, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpy2DAsync(d_in, rec, a, 48, 48, n, cudaMemcpyHostToDevice, s));
+    if (rec == 96) CK(cudaMemcpy2DAsync(d_in + 48, rec, b ? b : a, 48, 48, n, cudaMemcpyHostToDevice, s));
+    rc = launch_test_field(ctx, fop, d_in, n, d_out);
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(out, d_out, n * 48, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     return 0;
 }

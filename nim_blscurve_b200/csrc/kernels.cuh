@@ -13,6 +13,7 @@
 //   k_final         A9/A10 pairing.c:371-404, fp12_tower.c:773-786        product, final exp, ==1, GT bytes
 #pragma once
 #include <cuda_runtime.h>
+#include "../../include/blsgpu.h"
 #include "h2c.cuh"
 #include "pairing.cuh"
 #include "acc_team.cuh"
@@ -1101,21 +1102,144 @@ template <class F> __global__ void k_pt_neg(jac_t<F> *p) {
     *p = r;
 }
 
-// ---- diagnostics ----
-__global__ void k_test_fp(int op, const fp *a, const fp *b, size_t n, fp *out) {
-    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    fp x = a[i], y, r;
-    if (b) y = b[i]; else y = x;
-    switch (op) {
-        case 0: fp_mul(r, x, y); break;
-        case 1: fp_add(r, x, y); break;
-        case 2: fp_sub(r, x, y); break;
-        case 3: fp_sqr(r, x); break;
-        case 6: fp_inv_vartime(r, x); break;
-        default: fp_inv(r, x); break;
+// ---- diagnostics: the field primitives one at a time (blsgpu_test_field, blsgpu_test_fp) ----
+// Records: nin field elements and nin_w u32 words in, nout elements and nout_w words out (words padded to 16 bytes).
+// Geometry: a thread per record; a lane pair per record (fp2h.cuh, pair-uniform bounds check); one lane of a six-lane
+// team per record or one team per record (launch shape of k_miller_acc_team: ACC_BS threads, ACC_TPW teams per warp).
+enum { TF_THREAD, TF_PAIR, TF_TEAM_LANE, TF_TEAM };
+struct test_field_shape { int nin, nin_w, nout, nout_w, geom; };
+static const test_field_shape TEST_FIELD_OPS[BLSGPU_TF_COUNT] = {
+    {2, 0, 1, 0, TF_THREAD}, {2, 0, 1, 0, TF_THREAD}, {1, 0, 1, 0, TF_THREAD}, {1, 0, 1, 0, TF_THREAD},   // mul .. sqr_ni
+    {2, 0, 1, 0, TF_THREAD}, {2, 0, 1, 0, TF_THREAD}, {1, 0, 1, 0, TF_THREAD}, {1, 0, 1, 0, TF_THREAD},   // add .. inv
+    {1, 0, 1, 0, TF_THREAD}, {1, 0, 1, 0, TF_THREAD}, {1, 0, 1, 0, TF_THREAD},                            // .. from_mont
+    {1, 0, 0, 1, TF_THREAD}, {1, 0, 0, 1, TF_THREAD},                                                     // parity, lex
+    {4, 0, 2, 0, TF_THREAD}, {2, 0, 2, 0, TF_THREAD}, {2, 0, 2, 0, TF_THREAD}, {3, 0, 2, 0, TF_THREAD},   // fp2 mul .. mul_fp
+    {2, 0, 2, 0, TF_THREAD}, {2, 0, 2, 0, TF_THREAD}, {2, 0, 2, 1, TF_THREAD},                            // inv, inv_vt, rsqrt
+    {2, 0, 0, 1, TF_THREAD}, {2, 0, 0, 1, TF_THREAD},                                                     // sgn0, lex
+    {4, 0, 2, 0, TF_PAIR}, {2, 0, 2, 0, TF_PAIR}, {2, 0, 2, 0, TF_PAIR}, {3, 0, 2, 0, TF_PAIR},           // h_mul .. h_mul_fp
+    {2, 0, 2, 0, TF_PAIR}, {2, 0, 2, 0, TF_PAIR},                                                         // h_conj, h_inv
+    {6, 0, 1, 0, TF_TEAM_LANE}, {8, 2, 1, 0, TF_TEAM_LANE}, {18, 0, 12, 0, TF_TEAM}, {12, 0, 12, 0, TF_TEAM},
+    {14, 14, 1, 0, TF_THREAD},                                                                            // lin_finish
+};
+static inline size_t test_field_rec(int nfe, int nw) { return 48 * (size_t)nfe + 16 * (((size_t)nw + 3) / 4); }
+
+__global__ void __launch_bounds__(ACC_BS) k_test_field(int op, const uint8_t *in, size_t in_rec, size_t n, uint8_t *out,
+                                                      size_t out_rec) {
+    __shared__ acc_team_sm sm[ACC_TPB];
+    const int tid = threadIdx.x;
+    if (op >= BLSGPU_TF_TEAM_DOT3 && op <= BLSGPU_TF_TEAM_SQUARE) {
+        const int lane = tid & 31, warp = tid >> 5;
+        if (lane >= 6 * ACC_TPW) return;                   // lanes 30, 31 idle, as in k_miller_acc_team
+        const uint32_t mask = (1u << (6 * ACC_TPW)) - 1;
+        const int team = lane / 6, k = lane % 6;
+        acc_team_sm &T = sm[warp * ACC_TPW + team];
+        const size_t g = ((size_t)blockIdx.x * (ACC_BS / 32) + warp) * ACC_TPW + team;
+        if (op == BLSGPU_TF_TEAM_DOT3 || op == BLSGPU_TF_TEAM_DOT4) {
+            const size_t i = 6 * g + k;                    // a record per lane; no barriers on this path
+            if (i >= n) return;
+            const fp *x = (const fp *)(in + i * in_rec);
+            fp *S = (fp *)&T + 4 * k;                      // streamed side from shared memory, register side from the record
+            fp r;
+            if (op == BLSGPU_TF_TEAM_DOT3) {
+                for (int t = 0; t < 3; t++) S[t] = x[3 + t];
+                team_dot3(r, &x[0], &x[1], &x[2], &S[0], &S[1], &S[2]);
+            } else {
+                const uint32_t *w = (const uint32_t *)(x + 8);
+                for (int t = 0; t < 4; t++) S[t] = x[4 + t];
+                const fp *const ap[4] = {&x[0], &x[1], &x[2], &x[3]}, *const bp[4] = {&S[0], &S[1], &S[2], &S[3]};
+                team_dot4(r, ap, bp, w[0], w[1]);
+            }
+            *(fp *)(out + i * out_rec) = r;
+            return;
+        }
+        // a record per team: Fp12 f in the tower layout (coefficient of w^k at Fp2 index 3 (k & 1) + (k >> 1)), then
+        // the line; teams past n run on zeros so that every lane of the mask reaches every barrier
+        const bool valid = g < n;
+        const fp *x = (const fp *)(in + (valid ? g : 0) * in_rec);
+        const int s = 3 * (k & 1) + (k >> 1);
+        fp c0, c1;
+        if (valid) { c0 = x[2 * s]; c1 = x[2 * s + 1]; } else { fp_set_zero(c0); fp_set_zero(c1); }
+        team_store_coeff(T, k, c0, c1);
+        if (op == BLSGPU_TF_TEAM_MUL_LINE) {
+            fp v;
+            if (valid) v = x[12 + k]; else fp_set_zero(v);
+            T.l[k] = v;
+            __syncwarp(mask);
+            if (k < 3) { fp sum; fp_add(sum, T.l[2 * k], T.l[2 * k + 1]); T.l[6 + k] = sum; }
+            __syncwarp(mask);
+            team_mul_line(T, k, mask);
+        } else {
+            __syncwarp(mask);
+            team_square(T, k, mask);
+        }
+        if (valid) {
+            fp *y = (fp *)(out + g * out_rec);
+            y[2 * s] = T.f[k][FV_C0];
+            y[2 * s + 1] = T.f[k][FV_C1];
+        }
+        return;
     }
-    out[i] = r;
+    if (op >= BLSGPU_TF_H_MUL && op <= BLSGPU_TF_H_INV) {
+        const size_t e = ((size_t)blockIdx.x * blockDim.x + tid) >> 1;
+        if (e >= n) return;                                // the same for both lanes of a pair
+        const fp *x = (const fp *)(in + e * in_rec);
+        const int h = tid & 1;
+        fp2h a, b, r;
+        a.v = x[h];
+        switch (op) {
+            case BLSGPU_TF_H_MUL: b.v = x[2 + h]; h_mul(r, a, b); break;
+            case BLSGPU_TF_H_SQR: h_sqr(r, a); break;
+            case BLSGPU_TF_H_MUL_XI: h_mul_xi(r, a); break;
+            case BLSGPU_TF_H_MUL_FP: { fp kk = x[2]; h_mul_fp(r, a, kk); break; }
+            case BLSGPU_TF_H_CONJ: h_conj(r, a); break;
+            default: h_inv(r, a); break;
+        }
+        ((fp *)(out + e * out_rec))[h] = r.v;
+        return;
+    }
+    const size_t i = (size_t)blockIdx.x * blockDim.x + tid;
+    if (i >= n) return;
+    const fp *x = (const fp *)(in + i * in_rec);
+    fp *y = (fp *)(out + i * out_rec);
+    const fp a = x[0];
+    fp r;
+    fp2 a2, r2;
+    if (op >= BLSGPU_TF_FP2_MUL && op <= BLSGPU_TF_FP2_IS_LEXICALLY_LARGEST) { a2.c0 = x[0]; a2.c1 = x[1]; }
+    switch (op) {
+        case BLSGPU_TF_FP_MUL: { fp b = x[1]; fp_mul(r, a, b); break; }
+        case BLSGPU_TF_FP_MUL_NI: fp_mul_ni(r, a, x[1]); break;
+        case BLSGPU_TF_FP_SQR: fp_sqr(r, a); break;
+        case BLSGPU_TF_FP_SQR_NI: fp_sqr_ni(r, a); break;
+        case BLSGPU_TF_FP_ADD: { fp b = x[1]; fp_add(r, a, b); break; }
+        case BLSGPU_TF_FP_SUB: { fp b = x[1]; fp_sub(r, a, b); break; }
+        case BLSGPU_TF_FP_NEG: fp_neg(r, a); break;
+        case BLSGPU_TF_FP_INV: fp_inv(r, a); break;
+        case BLSGPU_TF_FP_INV_VARTIME: fp_inv_vartime(r, a); break;
+        case BLSGPU_TF_FP_POW_P34: fp_pow_p34(r, a); break;
+        case BLSGPU_TF_FP_FROM_MONT: fp_from_mont(r, a); break;
+        case BLSGPU_TF_FP_PARITY: *(uint32_t *)y = fp_parity(a); return;
+        case BLSGPU_TF_FP_IS_LEXICALLY_LARGEST_CANON: *(uint32_t *)y = fp_is_lexically_largest_canon(a); return;
+        case BLSGPU_TF_FP2_MUL: { fp2 b2; b2.c0 = x[2]; b2.c1 = x[3]; fp2_mul(r2, a2, b2); break; }
+        case BLSGPU_TF_FP2_SQR: fp2_sqr(r2, a2); break;
+        case BLSGPU_TF_FP2_MUL_XI: fp2_mul_xi(r2, a2); break;
+        case BLSGPU_TF_FP2_MUL_FP: { fp kk = x[2]; fp2_mul_fp(r2, a2, kk); break; }
+        case BLSGPU_TF_FP2_INV: fp2_inv(r2, a2); break;
+        case BLSGPU_TF_FP2_INV_VARTIME: fp2_inv_vartime(r2, a2); break;
+        case BLSGPU_TF_FP2_RSQRT_OR_Z: ((uint32_t *)(y + 2))[0] = fp2_rsqrt_or_z(r2, a2); break;
+        case BLSGPU_TF_FP2_SGN0: *(uint32_t *)y = fp2_sgn0(a2); return;
+        case BLSGPU_TF_FP2_IS_LEXICALLY_LARGEST: *(uint32_t *)y = fp2_is_lexically_largest(a2); return;
+        default: {                                         // BLSGPU_TF_LIN_FINISH, built as fp_program2_body builds it
+            const uint32_t *w = (const uint32_t *)(x + 14);
+            lin_acc A;
+            lin_clear(A);
+            for (int j = 0; j < 7; j++) { fp t = x[j]; lin_add_term(A.P, t, w[j]); }
+            for (int j = 0; j < 7; j++) { fp t = x[7 + j]; lin_add_term(A.N, t, w[7 + j]); }
+            lin_finish(r, A);
+            break;
+        }
+    }
+    if (op >= BLSGPU_TF_FP2_MUL && op <= BLSGPU_TF_FP2_IS_LEXICALLY_LARGEST) { y[0] = r2.c0; y[1] = r2.c1; }
+    else y[0] = r;
 }
 
 // Integer-multiply pipe peak: 8 independent mad.wide (or mad.lo) chains per thread, no memory traffic.

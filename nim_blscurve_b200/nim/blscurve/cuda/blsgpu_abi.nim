@@ -63,6 +63,8 @@ proc blsgpu_stage_name*(stage: cint): cstring
 proc blsgpu_last_launches*(ctx: BlsGpuCtx): cint
 # diagnostics / synthetic workloads (benchmarks and tests only)
 proc blsgpu_test_fp*(ctx: BlsGpuCtx, op: cint, a, b: pointer, n: csize_t, dst: pointer): cint
+proc blsgpu_test_field*(ctx: BlsGpuCtx, op: cint, src: pointer, inRecBytes, n: csize_t, dst: pointer,
+                        outRecBytes: csize_t): cint
 proc blsgpu_test_small_hash*(ctx: BlsGpuCtx, sets: pointer, n: csize_t, outIn, outOut: ptr byte): cint
 proc blsgpu_imad_peak*(ctx: BlsGpuCtx, wide: cint): cdouble
 proc blsgpu_fpmul_peak*(ctx: BlsGpuCtx, threadsPerBlock, blocksPerSm: cint): cdouble

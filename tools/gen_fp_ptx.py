@@ -278,6 +278,8 @@ def check():
         assert unl(run_ptx(W, ops)[:24]) == x2 * y2, ("mulw-wide", hex(x2), hex(y2))
     tvals = [0, 1, P * R - 1, P * R - P, (P - 1) * (P - 1), 4 * (P - 1) * (P - 1) % (P * R), R - 1, R, R + 1, (R - 1) * (P - 1) % (P * R)]
     tvals += [rng.randrange(P * R) for _ in range(400)]
+    # T = p (mod 2^384): every reduction multiplier is 0xffffffff and the sum before the final subtraction reaches p
+    tvals += [P + k * R for k in [0, 1, P - 2, P - 1, (P - 1) // 2] + [rng.randrange(P) for _ in range(100)]]
     for T in tvals:
         ops = [0] * 12 + limbs(T, 24)
         got = unl(run_ptx(Rd, ops)[:12])
@@ -303,7 +305,8 @@ def emit_fn(name, A, nout, nin_groups, doc):
     return txt
 
 
-def write():
+def render():
+    """the text of fp_gen.cuh"""
     hdr = """// fp_gen.cuh — GENERATED by tools/gen_fp_ptx.py (do not edit; rerun the generator).  Straight-line PTX bodies:
 // every 32x32->64 partial product is a mad.lo.cc/madc.hi.cc pair on an aligned register pair (one IMAD.WIDE.U32.X),
 // registers are block-local so the even/odd accumulator swap of each Montgomery row is a renaming, not a move.
@@ -325,8 +328,12 @@ namespace bls {
     out += emit_fn("fp_redc_ptx", gen_redc(), 12, [("t", 24)],
                    "r (12 limbs, < 2p) = t / 2^384 mod p up to one subtraction, t (24 limbs) < p * 2^384; 156 IMADs")
     out += "\n}  // namespace bls\n#endif  // __CUDA_ARCH__\n"
+    return out
+
+
+def write():
     path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "nim_blscurve_b200", "csrc", "fp_gen.cuh")
-    open(path, "w").write(out)
+    open(path, "w").write(render())
     print("wrote", os.path.normpath(path))
 
 
