@@ -230,7 +230,7 @@ enum {
 };
 int blsgpu_test_field(blsgpu_ctx *ctx, int op, const void *in, size_t in_rec_bytes, size_t n, void *out,
                       size_t out_rec_bytes);
-/* The message hash of the small-batch route (two-lane map kernel, then the cofactor-clearing dataflow program):
+/* The message hash of the small-batch route (the pipeline's map kernel, then the cofactor-clearing dataflow program):
  * n <= 4096 sets in (host, 320 B each); out_in / out_out (nullable): n x 6 field elements (48 B each, Montgomery) =
  * the homogeneous E2 point (X : Y : Z) before / after the program.  H(m_i) = (X/Z, Y/Z) of out_out. */
 int blsgpu_test_small_hash(blsgpu_ctx *ctx, const void *sets320, size_t n, uint8_t *out_in, uint8_t *out_out);

@@ -21,8 +21,6 @@ using namespace bls;
 enum { ST_SCALARS = 0, ST_G2MUL, ST_G2SUM, ST_HASH, ST_G1MUL, ST_AFFINE, ST_LINES, ST_ACC, ST_GTPROD, ST_PARTIAL, ST_FINAL, ST_COUNT };
 static const char *STAGE_NAMES[ST_COUNT] = {"rlc_scalars", "g2_mul64", "g2_sum", "hash_to_g2", "g1_mul64", "pairs_affine",
                                             "miller_lines", "miller_acc", "gt_product", "partial", "final_exp"};
-// Miller-loop tiling: at most LINES_TILE pairs have their 68 x 288-byte line triples resident at once
-static const size_t LINES_TILE = (size_t)1 << 18;
 static_assert(route::ACC_BLOCK == BLS_ACC_BS && ST_ACC == ST_LINES + 1 && ST_GTPROD == ST_LINES + 2 && ST_PARTIAL == ST_LINES + 3,
               "route.hpp / miller_ws layout");
 static_assert(route::LB_BLOCKS == BLS_LB_BLOCKS, "route.hpp plan_msm sizes the chunk grid for the BLS_LB occupancy");
@@ -32,17 +30,32 @@ enum prog_kind { PROG_COMBINE, PROG_FINAL, PROG_NORM, PROG_SET, PROG_PRODUCT, PR
 
 // Buffers, stream and stage events of one multi-Miller loop (run_miller)
 struct miller_ws {
-    uint32_t *lines = nullptr;    // 68 x 72 words x lines_cap
-    size_t lines_cap = 0;         // pairs per tile
+    route::miller_caps caps = {}; // sizes of the buffers below
+    uint32_t *lines = nullptr;    // 68 x 72 words x caps.lines_cap
     fp12 *F = nullptr;            // per-segment block products, nseg rows
-    size_t f_cap = 0;
     fp12 *F2 = nullptr;           // second-level block products
-    size_t f2_cap = 0;
     fp12 *seg = nullptr;          // 64 segment products
     fp *small_lines = nullptr;    // 68 x 6 field elements per pair (small-batch route), allocated on first use
     cudaStream_t stream = nullptr;
     cudaEvent_t *ev = nullptr;    // begin/end pairs of miller_lines, miller_acc, gt_product, partial
 };
+
+static void miller_ws_free(miller_ws &ws) {
+    cudaFree(ws.lines); cudaFree(ws.F); cudaFree(ws.F2); cudaFree(ws.seg); cudaFree(ws.small_lines);
+    ws.lines = nullptr; ws.F = ws.F2 = ws.seg = nullptr; ws.small_lines = nullptr;
+}
+
+// lines, F, F2 and seg of ws, sized from ws.caps; all or none: on failure ws is left without buffers
+static cudaError_t miller_ws_alloc(miller_ws &ws) {
+    cudaError_t e = cudaMalloc((void **)&ws.lines, (size_t)ML_NLINES * ML_LINE_WORDS * 4 * ws.caps.lines_cap);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&ws.F, ws.caps.f_cap * sizeof(fp12));
+    if (e == cudaSuccess) e = cudaMalloc((void **)&ws.F2, ws.caps.f2_cap * sizeof(fp12));
+    if (e == cudaSuccess) e = cudaMalloc((void **)&ws.seg, 64 * sizeof(fp12));
+    if (e != cudaSuccess) miller_ws_free(ws);
+    return e;
+}
+
+enum { H2D_SLICES = 4 };
 
 struct blsgpu_ctx {
     int device = 0;
@@ -90,11 +103,11 @@ struct blsgpu_ctx {
     bool serial_tail = false;
     bool prog_smem_raised = false;                           // k_fp_program allowed > 48 KiB of shared memory on this device
     // host-buffer calls on large batches: the H2D copy is cut into H2D_SLICES pieces on a copy stream and the hash kernel
-    // into as many launches on their own streams, each waiting for its piece only (run_partial_impl)
+    // into as many launches on their own streams, each waiting for its piece only (run_partial_impl); created on first
+    // use by create_slices
     const uint8_t *h_src = nullptr;                          // caller's host buffer for the current call (borrowed)
-    cudaStream_t copy_stream = nullptr, slice_stream[4] = {nullptr, nullptr, nullptr, nullptr};
-    cudaEvent_t ev_copy[4], ev_slice[4];
-    bool slices_ready = false;
+    cudaStream_t copy_stream = nullptr, slice_stream[H2D_SLICES] = {};
+    cudaEvent_t ev_copy[H2D_SLICES] = {}, ev_slice[H2D_SLICES] = {};
     bool chain_smem_raised = false;                          // k_rlc_scalars allowed to reserve a whole SM's shared memory
     // multi-device context (blsgpu_create_multi): this context is the leader (share 0 + the one final exponentiation),
     // peers[k-1] owns share k on its own device; the 576-byte partials and the flags are gathered into the leader
@@ -133,6 +146,12 @@ static int fail(blsgpu_ctx *c, int code, const char *what, cudaError_t e = cudaS
 
 static inline unsigned nblk(size_t n, unsigned bs = 128) { return (unsigned)((n + bs - 1) / bs); }
 
+// the route thresholds, read from the environment once per process (route.hpp)
+static const route::thresholds &thr() {
+    static const route::thresholds t = route::read_thresholds();
+    return t;
+}
+
 extern "C" int blsgpu_device_count(void) {
     int n = 0;
     if (cudaGetDeviceCount(&n) != cudaSuccess) { cudaGetLastError(); return 0; }
@@ -142,19 +161,41 @@ extern "C" int blsgpu_device_count(void) {
 extern "C" const char *blsgpu_last_error(const blsgpu_ctx *ctx) { return ctx ? ctx->err.c_str() : g_err.c_str(); }
 extern "C" size_t blsgpu_capacity(const blsgpu_ctx *ctx) { return ctx ? (ctx->multi_cap ? ctx->multi_cap : ctx->cap) : 0; }
 
+static void destroy_slices(blsgpu_ctx *ctx) {
+    if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
+    ctx->copy_stream = nullptr;
+    for (int k = 0; k < H2D_SLICES; k++) {
+        if (ctx->slice_stream[k]) cudaStreamDestroy(ctx->slice_stream[k]);
+        if (ctx->ev_copy[k]) cudaEventDestroy(ctx->ev_copy[k]);
+        if (ctx->ev_slice[k]) cudaEventDestroy(ctx->ev_slice[k]);
+        ctx->slice_stream[k] = nullptr;
+        ctx->ev_copy[k] = ctx->ev_slice[k] = nullptr;
+    }
+}
+
+// the copy stream and the streams and events of the slices; all or none: on failure the context is left without them
+static cudaError_t create_slices(blsgpu_ctx *ctx) {
+    cudaError_t e = cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking);
+    for (int k = 0; k < H2D_SLICES && e == cudaSuccess; k++) {
+        e = cudaStreamCreateWithFlags(&ctx->slice_stream[k], cudaStreamNonBlocking);
+        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_copy[k], cudaEventDisableTiming);
+        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_slice[k], cudaEventDisableTiming);
+    }
+    if (e != cudaSuccess) destroy_slices(ctx);
+    return e;
+}
+
 extern "C" void blsgpu_destroy(blsgpu_ctx *ctx) {
     if (!ctx) return;
     for (blsgpu_ctx *p : ctx->peers) blsgpu_destroy(p);
     ctx->peers.clear();
     cudaSetDevice(ctx->device);
     cudaFree(ctx->d_gather); cudaFree(ctx->d_gather_flags); cudaFree(ctx->d_srb);
-    for (miller_ws *w : {&ctx->ml, &ctx->ml_sig}) { cudaFree(w->lines); cudaFree(w->F); cudaFree(w->F2); cudaFree(w->seg); cudaFree(w->small_lines); }
+    miller_ws_free(ctx->ml);
+    miller_ws_free(ctx->ml_sig);
     for (auto &g : ctx->graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
     if (ctx->ev_share) cudaEventDestroy(ctx->ev_share);
-    if (ctx->slices_ready) {
-        cudaStreamDestroy(ctx->copy_stream);
-        for (int k = 0; k < 4; k++) { cudaStreamDestroy(ctx->slice_stream[k]); cudaEventDestroy(ctx->ev_copy[k]); cudaEventDestroy(ctx->ev_slice[k]); }
-    }
+    destroy_slices(ctx);
     if (ctx->ev_scratch_valid) for (int i = 0; i < 8; i++) cudaEventDestroy(ctx->ev_scratch[i]);
     cudaFree(ctx->d_sets); cudaFree(ctx->d_r); cudaFree(ctx->d_H); cudaFree(ctx->d_Pj); cudaFree(ctx->d_Q);
     cudaFree(ctx->d_P); cudaFree(ctx->d_S); cudaFree(ctx->d_partials); cudaFree(ctx->d_gtb);
@@ -200,16 +241,9 @@ extern "C" blsgpu_ctx *blsgpu_create(int device, size_t max_sets) {
     ALLOC(ctx->d_Q, (n + 1) * sizeof(g2_aff));            // + the signature-side pair
     ALLOC(ctx->d_P, (n + 1) * sizeof(g1_aff));
     ALLOC(ctx->d_S, n * sizeof(g2_jac));
-    miller_ws &ml = ctx->ml;
-    ml.lines_cap = ((n + 1 < LINES_TILE ? n + 1 : LINES_TILE) + 31) & ~(size_t)31;
-    ALLOC(ml.lines, (size_t)ML_NLINES * ML_LINE_WORDS * 4 * ml.lines_cap);
-    // block products: <= 64 segments x (blocks per tile + 1) x tiles
-    ml.f_cap = (n + 1) / 2 + 40000 + 64 * ((n + 1) / LINES_TILE + 2);   // >= nseg * groups for every miller_shape
-    ALLOC(ml.F, ml.f_cap * sizeof(fp12));
-    ml.f2_cap = ml.f_cap / 8 + 4096;                          // level-1 output of the 8-way product trees (+ padding)
-    ALLOC(ml.F2, ml.f2_cap * sizeof(fp12));
-    ALLOC(ml.seg, 64 * sizeof(fp12));
-    ml.ev = ctx->ev + 2 * ST_LINES;
+    ctx->ml.caps = route::miller_caps_batch(thr(), n);
+    if ((e = miller_ws_alloc(ctx->ml)) != cudaSuccess) return bad("cudaMalloc Miller workspace", e);
+    ctx->ml.ev = ctx->ev + 2 * ST_LINES;
     ALLOC(ctx->d_partials, 64 * sizeof(fp12));
     ALLOC(ctx->d_gtb, 576);
     ALLOC(ctx->d_gt, sizeof(fp12));
@@ -245,9 +279,7 @@ extern "C" blsgpu_ctx *blsgpu_create(int device, size_t max_sets) {
     if ((e = cudaEventCreateWithFlags(&ctx->ev_share, cudaEventDisableTiming)) != cudaSuccess) return bad("cudaEventCreate", e);
     for (int i = 0; i < 8; i++) if ((e = cudaEventCreate(&ctx->ev_scratch[i])) != cudaSuccess) return bad("cudaEventCreate", e);
     ctx->ev_scratch_valid = true;
-    ctx->ml_sig.lines_cap = 32;
-    ctx->ml_sig.f_cap = 2048;
-    ctx->ml_sig.f2_cap = 512;
+    ctx->ml_sig.caps = route::miller_caps_sig();
     ctx->ml_sig.stream = ctx->side;
     ctx->ml_sig.ev = ctx->ev_scratch;
     return ctx;
@@ -327,11 +359,6 @@ static_assert(fpprog::CONST_COUNT == fpprog_const_count && fpprog::CONST_FROB1 =
 #define EV_SC (2 * ST_COUNT + 3)
 #define EV_HASHED (2 * ST_COUNT + 4)
 
-// the route thresholds, read from the environment once per process (route.hpp)
-static const route::thresholds &thr() {
-    static const route::thresholds t = route::read_thresholds();
-    return t;
-}
 static route::batch_plan batch_plan_of(const blsgpu_ctx *ctx, size_t n, size_t total_n, uint32_t chunks, bool host_src, bool scalars) {
     return route::plan_batch(thr(), {ctx->use_side, ctx->acc_team, ctx->serial_tail, ctx->use_graph}, n, total_n, chunks, host_src,
                              scalars);
@@ -467,7 +494,36 @@ static int run_msm(blsgpu_ctx *ctx, const uint8_t *d_points, size_t pstride, con
     return rc ? fail(ctx, rc == -1 ? BLSGPU_ERR_CUDA : BLSGPU_ERR_ARG, err.c_str()) : 0;
 }
 
-#define SMALL_FP_PER_SET (6 + 6 + 6 + 6 + 64)
+// Per-set inputs and outputs of the small-batch route's programs, SMALL_ROUTE_CAP sets each: homogeneous points of 6
+// field elements, and the 64 bits of a scalar as field elements 0 / 1
+struct small_bufs { fp *hash_in, *hash_out, *sig_in, *sig_out, *bits; };
+
+// the small-route buffers, allocated on first use
+static int small_buffers(blsgpu_ctx *ctx, small_bufs &b) {
+    const size_t cap = route::SMALL_ROUTE_CAP;
+    if (!ctx->d_small) CK(cudaMalloc((void **)&ctx->d_small, cap * (6 + 6 + 6 + 6 + 64) * sizeof(fp)));
+    b.hash_in = ctx->d_small;
+    b.hash_out = b.hash_in + 6 * cap;
+    b.sig_in = b.hash_out + 6 * cap;
+    b.sig_out = b.sig_in + 6 * cap;
+    b.bits = b.sig_out + 6 * cap;
+    return 0;
+}
+
+// H(m_i) of the small-batch route on stream s, up to the homogeneous point in b.hash_out: the map to E2 (two lanes per
+// message, or the pair kernel with BLSGPU_MAP_LANES2=0) into b.hash_in, then the cofactor clearing as a per-set program.
+// The messages are those of `sets`, or with sets == nullptr msgs + offs[i] .. offs[i + 1] under the tag dst.
+static int launch_small_hash(blsgpu_ctx *ctx, const small_bufs &b, cudaStream_t s, size_t n, const sigset *sets,
+                             const uint8_t *msgs, const uint32_t *offs, const uint8_t *dst, size_t dst_len) {
+    blsgpu_ctx::dev_prog p_cof;
+    int rc = get_prog(ctx, PROG_SET, SETPROG_COFACTOR, p_cof, s);
+    if (rc) return rc;
+    if (thr().map_lanes2) k_hash_map_lanes2<<<nblk(2 * n, 64), 64, 0, s>>>(sets, msgs, offs, dst, (uint32_t)dst_len, n, b.hash_in);
+    else if (sets) k_hash_map_pair<<<nblk(2 * n), 128, 0, s>>>(sets, n, b.hash_in);
+    else k_hash_map_pair_msgs<<<nblk(2 * n), 128, 0, s>>>(msgs, offs, dst, (uint32_t)dst_len, n, b.hash_in);
+    launch_prog_many(ctx, p_cof, s, n, b.hash_in, 6, nullptr, 0, b.hash_out, 6);
+    return 0;
+}
 
 // Multi-Miller loop over the np pairs (d_Q[pair0 + i], d_P[pair0 + i]) + reductions, on the buffers, stream and stage
 // events of workspace ws; leaves conj(prod ML) in d_partials[slot]
@@ -478,21 +534,18 @@ static int run_miller(blsgpu_ctx *ctx, miller_ws &ws, size_t np, int slot, size_
     int rc;
     // tile by tile: lines, then per-(group, segment) accumulation
     const bool team = ctx->acc_team;
-    const route::miller_plan mp = route::plan_miller(thr(), np, ws.lines_cap, team, ctx->serial_tail);
+    const size_t lines_cap = ws.caps.lines_cap;
+    const route::miller_plan mp = route::plan_miller(thr(), np, lines_cap, team, ctx->serial_tail);
     const int G = mp.G, nseg = mp.nseg;
-    const size_t ncols = mp.ncols;                          // entries per segment row of F
-    // small batches: the GT product of each segment row runs as product-tree programs over groups of 8 columns, so
-    // the rows of F are padded to a multiple of 8 with ones
-    const size_t row_stride = mp.gt_prog && ncols > 8 ? ((ncols + 7) & ~(size_t)7) : ncols;
-    const size_t ncols2 = mp.gt_prog ? ((((ncols + 7) / 8) + 7) & ~(size_t)7) : (ncols + BLS_ACC_BS - 1) / BLS_ACC_BS;
-    if ((size_t)nseg * row_stride > ws.f_cap || (size_t)nseg * ncols2 > ws.f2_cap)
-        return fail(ctx, BLSGPU_ERR_CAPACITY, "segment product buffer too small");
+    const size_t ncols = mp.ncols, row_stride = mp.row_stride, ncols2 = mp.ncols2;
+    // every default plan fits (tests/test_hostsim.py); threshold overrides may not
+    if (!route::fits(mp, ws.caps)) return fail(ctx, BLSGPU_ERR_CAPACITY, "segment product buffer too small");
     size_t col = 0;
     WBEGIN(ST_LINES);
-    bool single = np <= ws.lines_cap;
-    for (size_t off = 0; off < np; off += ws.lines_cap) {
-        size_t t = np - off < ws.lines_cap ? np - off : ws.lines_cap;
-        size_t stride = ws.lines_cap;
+    bool single = np <= lines_cap;
+    for (size_t off = 0; off < np; off += lines_cap) {
+        size_t t = np - off < lines_cap ? np - off : lines_cap;
+        size_t stride = lines_cap;
         const int lines = off + t < np ? mp.lines : mp.lines_last;
         if (lines == route::LINES_PROGRAM) {
             // one warp per pair runs the 68 line evaluations as a dataflow program, then a scatter into the
@@ -501,7 +554,7 @@ static int run_miller(blsgpu_ctx *ctx, miller_ws &ws, size_t np, int slot, size_
             rc = get_prog(ctx, PROG_SET, SETPROG_LINES, lp, s);
             if (rc) return rc;
             const size_t per = (size_t)ML_NLINES * 6;
-            if (!ws.small_lines) CK(cudaMalloc((void **)&ws.small_lines, thr().small_lines_max * per * sizeof(fp)));
+            if (!ws.small_lines) CK(cudaMalloc((void **)&ws.small_lines, ws.caps.small_lines * per * sizeof(fp)));
             launch_prog_many(ctx, lp, s, t, (const fp *)(ctx->d_Q + pair0), 4, (const fp *)(ctx->d_P + pair0), 2, ws.small_lines, per, true);
             k_lines_from_prog<<<nblk(t * ML_NLINES * ML_LINE_WORDS, 256), 256, 0, s>>>((const uint32_t *)ws.small_lines, ctx->d_Q + pair0, ctx->d_P + pair0, t,
                                                                                       ws.lines, stride);
@@ -589,9 +642,9 @@ static int run_partial(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, size_t f
         cudaStreamSynchronize(ctx->chain);
         cudaStreamSynchronize(ctx->side);
         cudaStreamSynchronize(ctx->side2);
-        if (ctx->slices_ready) {
+        if (ctx->copy_stream) {
             cudaStreamSynchronize(ctx->copy_stream);
-            for (int k = 0; k < 4; k++) cudaStreamSynchronize(ctx->slice_stream[k]);
+            for (int k = 0; k < H2D_SLICES; k++) cudaStreamSynchronize(ctx->slice_stream[k]);
         }
         cudaStreamSynchronize(ctx->stream);
         cudaGetLastError();
@@ -616,18 +669,9 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
     // copy ahead of everything.  Large ones: H2D_SLICES pieces on a copy stream, each followed at once by the launch of
     // the hash kernel over that piece on its own stream, so the copy (and, for pageable memory, the host-side staging
     // that blocks the calling thread piece by piece) hides behind H(m_i) of the earlier pieces.
-    enum { H2D_SLICES = 4 };
     const bool sliced = plan.sliced;
     if (ctx->h_src && !sliced) CK(cudaMemcpyAsync(ctx->d_sets, ctx->h_src, n * sizeof(sigset), cudaMemcpyHostToDevice, s));
-    if (sliced && !ctx->slices_ready) {
-        CK(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
-        for (int k = 0; k < H2D_SLICES; k++) {
-            CK(cudaStreamCreateWithFlags(&ctx->slice_stream[k], cudaStreamNonBlocking));
-            CK(cudaEventCreateWithFlags(&ctx->ev_copy[k], cudaEventDisableTiming));
-            CK(cudaEventCreateWithFlags(&ctx->ev_slice[k], cudaEventDisableTiming));
-        }
-        ctx->slices_ready = true;
-    }
+    if (sliced && !ctx->copy_stream) CK(create_slices(ctx));
     CK(cudaMemsetAsync(ctx->d_flags, 0, 4 * sizeof(int), s));
     // fork: the scalar chain (strictly sequential SHA-256 per reference chunk: tens of milliseconds for a large batch
     // when the caller passes tp.numThreads = 16..32 chunks) and the signature-side sum that consumes the scalars run on
@@ -654,18 +698,12 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
     }
     // Small-batch route: the serial stretches of a set (cofactor clearing, [r_i] sig_i) run as per-set dataflow
     // programs, one warp per set (fpprog.hpp build_g2_clear_cofactor / build_g2_mul64)
-    blsgpu_ctx::dev_prog p_cof, p_mul;
-    fp *sm_hash_in = nullptr, *sm_hash_out = nullptr, *sm_sig_in = nullptr, *sm_sig_out = nullptr, *sm_bits = nullptr;
+    blsgpu_ctx::dev_prog p_mul;
+    small_bufs sb = {};
     if (plan.small) {
-        if (!ctx->d_small) CK(cudaMalloc((void **)&ctx->d_small, route::SMALL_ROUTE_CAP * SMALL_FP_PER_SET * sizeof(fp)));
-        rc = get_prog(ctx, PROG_SET, SETPROG_COFACTOR, p_cof, s);
+        rc = small_buffers(ctx, sb);
         if (!rc) rc = get_prog(ctx, PROG_SET, SETPROG_G2MUL64, p_mul, s);
         if (rc) return rc;
-        sm_hash_in = ctx->d_small;
-        sm_hash_out = sm_hash_in + 6 * route::SMALL_ROUTE_CAP;
-        sm_sig_in = sm_hash_out + 6 * route::SMALL_ROUTE_CAP;
-        sm_sig_out = sm_sig_in + 6 * route::SMALL_ROUTE_CAP;
-        sm_bits = sm_sig_out + 6 * route::SMALL_ROUTE_CAP;
     }
     if (sliced) {
         if (!ctx->use_side) CK(cudaEventRecord(ctx->ev[EV_FORK], s));
@@ -704,11 +742,10 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
         if (sliced) return 0;
         BEGIN(ST_HASH, s);
         if (plan.hash == route::HASH_PROGRAM) {
-            if (thr().map_lanes2) k_hash_map_lanes2<<<nblk(2 * n, 64), 64, 0, s>>>(d_sets, nullptr, nullptr, nullptr, 0, n, sm_hash_in);
-            else k_hash_map_pair<<<nblk(2 * n), 128, 0, s>>>(d_sets, n, sm_hash_in);
-            launch_prog_many(ctx, p_cof, s, n, sm_hash_in, 6, nullptr, 0, sm_hash_out, 6);
-            k_g2_hom_to_jac<<<nblk(n), 128, 0, s>>>(sm_hash_out, n, ctx->d_H);
-            ctx->launches += 2;
+            int rch = launch_small_hash(ctx, sb, s, n, d_sets, nullptr, nullptr, nullptr, 0);
+            if (rch) return rch;
+            k_g2_hom_to_jac<<<nblk(n), 128, 0, s>>>(sb.hash_out, n, ctx->d_H);
+            ctx->launches += 2;                             // the map and the conversion
         } else if (plan.hash == route::HASH_LANES2) k_hash_sets_lanes2<<<nblk(2 * n), 128, 0, s>>>(d_sets, n, ctx->d_H);
         else if (plan.hash == route::HASH_PAIR) k_hash_sets_pair<<<nblk(2 * n), 128, 0, s>>>(d_sets, n, ctx->d_H);
         else k_hash_sets<<<nblk(n), 128, 0, s>>>(d_sets, n, ctx->d_H);
@@ -731,9 +768,9 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
         BEGIN(ST_G2SUM, g);
     } else {
         if (plan.sig == route::SIG_PROGRAM) {
-            k_g2_mul_prep<<<nblk(64 * n), 128, 0, g>>>(d_sets, ctx->d_r, n, sm_sig_in, sm_bits);
-            launch_prog_many(ctx, p_mul, g, n, sm_sig_in, 6, sm_bits, 64, sm_sig_out, 6);
-            k_g2_hom_to_jac<<<nblk(n), 128, 0, g>>>(sm_sig_out, n, ctx->d_S);
+            k_g2_mul_prep<<<nblk(64 * n), 128, 0, g>>>(d_sets, ctx->d_r, n, sb.sig_in, sb.bits);
+            launch_prog_many(ctx, p_mul, g, n, sb.sig_in, 6, sb.bits, 64, sb.sig_out, 6);
+            k_g2_hom_to_jac<<<nblk(n), 128, 0, g>>>(sb.sig_out, n, ctx->d_S);
             ctx->launches += 2;
         } else {
             k_g2_mul<<<nblk(n), 128, 0, g>>>(d_sets, ctx->d_r, n, ctx->d_S);
@@ -755,15 +792,8 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
     // on its own workspace, beside the big loop of the main stream; after the join the two values are multiplied (one
     // Fp12 product program).  Same product of the same n + 1 Miller values, hence same GT.
     if (plan.defer_sig) {
-        miller_ws &ws = ctx->ml_sig;
-        if (!ws.lines) {
-            CK(cudaMalloc((void **)&ws.lines, (size_t)ML_NLINES * ML_LINE_WORDS * 4 * ws.lines_cap));
-            CK(cudaMalloc((void **)&ws.F, ws.f_cap * sizeof(fp12)));
-            CK(cudaMalloc((void **)&ws.F2, ws.f2_cap * sizeof(fp12)));
-            CK(cudaMalloc((void **)&ws.seg, 64 * sizeof(fp12)));
-            CK(cudaMalloc((void **)&ws.small_lines, 2 * (size_t)ML_NLINES * 6 * sizeof(fp)));
-        }
-        rc = run_miller(ctx, ws, 1, slot + 1, n);
+        if (!ctx->ml_sig.lines) CK(miller_ws_alloc(ctx->ml_sig));
+        rc = run_miller(ctx, ctx->ml_sig, 1, slot + 1, n);
         if (rc) return rc;
     }
     if (ctx->use_side) CK(cudaEventRecord(ctx->ev[EV_JOIN], g));
@@ -1157,17 +1187,15 @@ extern "C" int blsgpu_test_small_hash(blsgpu_ctx *ctx, const void *sets320, size
     if (!ctx || !sets320 || n == 0 || n > route::SMALL_ROUTE_CAP || n > ctx->cap) return BLSGPU_ERR_ARG;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->stream;
-    if (!ctx->d_small) CK(cudaMalloc((void **)&ctx->d_small, route::SMALL_ROUTE_CAP * SMALL_FP_PER_SET * sizeof(fp)));
-    blsgpu_ctx::dev_prog p_cof;
-    int rc = get_prog(ctx, PROG_SET, SETPROG_COFACTOR, p_cof, s);
+    small_bufs sb;
+    int rc = small_buffers(ctx, sb);
     if (rc) return rc;
-    fp *hin = ctx->d_small, *hout = hin + 6 * route::SMALL_ROUTE_CAP;
     CK(cudaMemcpyAsync(ctx->d_sets, sets320, n * 320, cudaMemcpyHostToDevice, s));
-    k_hash_map_lanes2<<<nblk(2 * n, 64), 64, 0, s>>>(ctx->d_sets, nullptr, nullptr, nullptr, 0, n, hin);
-    launch_prog_many(ctx, p_cof, s, n, hin, 6, nullptr, 0, hout, 6);
+    rc = launch_small_hash(ctx, sb, s, n, ctx->d_sets, nullptr, nullptr, nullptr, 0);
+    if (rc) return rc;
     CK(cudaGetLastError());
-    if (out_in) CK(cudaMemcpyAsync(out_in, hin, n * 6 * sizeof(fp), cudaMemcpyDeviceToHost, s));
-    if (out_out) CK(cudaMemcpyAsync(out_out, hout, n * 6 * sizeof(fp), cudaMemcpyDeviceToHost, s));
+    if (out_in) CK(cudaMemcpyAsync(out_in, sb.hash_in, n * 6 * sizeof(fp), cudaMemcpyDeviceToHost, s));
+    if (out_out) CK(cudaMemcpyAsync(out_out, sb.hash_out, n * 6 * sizeof(fp), cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     return 0;
 }
@@ -1268,17 +1296,12 @@ static int verify_pairs_dev(blsgpu_ctx *ctx, const g1_aff *d_pks, size_t n, cons
     CK(cudaMemsetAsync(ctx->d_flags, 0, 4 * sizeof(int), s));
     BEGIN(ST_HASH, s);
     if (route::program_hash(thr(), n, ctx->serial_tail)) {
-        // small-batch route (see run_partial): two lanes per message, cofactor clearing as a per-message program
-        blsgpu_ctx::dev_prog p_cof;
-        int rcp = get_prog(ctx, PROG_SET, SETPROG_COFACTOR, p_cof, s);
+        small_bufs sb;
+        int rcp = small_buffers(ctx, sb);
+        if (!rcp) rcp = launch_small_hash(ctx, sb, s, n, nullptr, d_msgs, d_offs, d_dst, dst_len);
         if (rcp) return rcp;
-        if (!ctx->d_small) CK(cudaMalloc((void **)&ctx->d_small, route::SMALL_ROUTE_CAP * SMALL_FP_PER_SET * sizeof(fp)));
-        fp *hin = ctx->d_small, *hout = hin + 6 * route::SMALL_ROUTE_CAP;
-        if (thr().map_lanes2) k_hash_map_lanes2<<<nblk(2 * n, 64), 64, 0, s>>>(nullptr, d_msgs, d_offs, d_dst, (uint32_t)dst_len, n, hin);
-        else k_hash_map_pair_msgs<<<nblk(2 * n), 128, 0, s>>>(d_msgs, d_offs, d_dst, (uint32_t)dst_len, n, hin);
-        launch_prog_many(ctx, p_cof, s, n, hin, 6, nullptr, 0, hout, 6);
-        k_g2_hom_to_affine<<<(unsigned)n, 32, 0, s>>>(hout, n, ctx->d_Q);
-        ctx->launches += 2;
+        k_g2_hom_to_affine<<<(unsigned)n, 32, 0, s>>>(sb.hash_out, n, ctx->d_Q);
+        ctx->launches += 2;                                 // the map and the conversion
     } else {
         k_hash_to_g2<<<nblk(n), 128, 0, s>>>(d_msgs, n, 0, d_offs, d_dst, (uint32_t)dst_len, ctx->d_Q, nullptr);
     }

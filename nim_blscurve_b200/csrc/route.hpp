@@ -1,5 +1,6 @@
 // route.hpp — the batch pipeline's route policy: which kernels a batch of n sets runs, and the measured size thresholds
-// that decide it; and the shape of the Pippenger MSM (window width, segments, window groups, chunks, scratch layout).
+// that decide it; the capacities of the Miller-loop workspaces, which every Miller plan must fit; and the shape of the
+// Pippenger MSM (window width, segments, window groups, chunks, scratch layout).
 // Plain C++ without CUDA, so that tests/hostsim compiles it and checks the plans on the host.
 //
 // Every threshold is read from the environment by read_thresholds() (INTEGRATION.md section 8); libblsgpu caches the
@@ -236,12 +237,41 @@ inline void miller_shape(const thresholds &t, size_t np, bool team, int &G, int 
 
 enum { LINES_PROGRAM, LINES_LANES2, LINES_THREAD };   // per-pair program + scatter / k_miller_lines_lanes2 / k_miller_lines
 
+// Miller-loop tiling: at most LINES_TILE pairs have their 68 x 288-byte line triples resident at once
+static const size_t LINES_TILE = (size_t)1 << 18;
+
+// Capacities of a Miller-loop workspace (blsgpu.cu miller_ws)
+struct miller_caps {
+    size_t lines_cap;      // pairs per tile of the lines buffer
+    size_t f_cap;          // entries of the block products F
+    size_t f2_cap;         // entries of the second-level block products F2
+    size_t small_lines;    // pairs of the lines-program buffer (allocated on first use)
+};
+
+// the workspace of the batch's Miller loop in a context of max_sets sets: the set pairs + the signature-side pair
+// (tests/test_hostsim.py checks that the plans of 1 to max_sets + 1 pairs fit it)
+inline miller_caps miller_caps_batch(const thresholds &t, size_t max_sets) {
+    const size_t n = max_sets;
+    miller_caps c;
+    c.lines_cap = ((n + 1 < LINES_TILE ? n + 1 : LINES_TILE) + 31) & ~(size_t)31;
+    // block products: <= 64 segments x (blocks per tile + 1) x tiles
+    c.f_cap = (n + 1) / 2 + 40000 + 64 * ((n + 1) / LINES_TILE + 2);   // >= nseg * groups for every miller_shape
+    c.f2_cap = c.f_cap / 8 + 4096;                          // level-1 output of the 8-way product trees (+ padding)
+    c.small_lines = t.small_lines_max;
+    return c;
+}
+
+// the workspace of the deferred signature pair's one-pair Miller loop
+inline miller_caps miller_caps_sig() { return {32, 2048, 512, 2}; }
+
 struct miller_plan {
     int G, nseg;
     int lines;             // LINES_* of every tile of lines_cap pairs but the last
     int lines_last;        // LINES_* of the last tile (the only one when np <= lines_cap)
     size_t ncols;          // entries per segment row of the block products
     bool gt_prog;          // the GT product of each segment row runs as product-tree programs over groups of 8 columns
+    size_t row_stride;     // entries between segment rows of F
+    size_t ncols2;         // entries per segment row of F2
 };
 
 // np pairs, tiled by lines_cap (the pairs whose line triples fit the workspace at once)
@@ -256,6 +286,10 @@ inline miller_plan plan_miller(const thresholds &t, size_t np, size_t lines_cap,
     }
     const bool single = np <= lines_cap;
     p.gt_prog = (t.small_route & SMALL_GTPROD) && team && single && p.ncols <= t.gt_prog_max && !serial_tail;
+    // small batches: the GT product of each segment row runs as product-tree programs over groups of 8 columns, so
+    // the rows of F are padded to a multiple of 8 with ones
+    p.row_stride = p.gt_prog && p.ncols > 8 ? ((p.ncols + 7) & ~(size_t)7) : p.ncols;
+    p.ncols2 = p.gt_prog ? ((((p.ncols + 7) / 8) + 7) & ~(size_t)7) : (p.ncols + ACC_BLOCK - 1) / ACC_BLOCK;
     // one warp per pair runs the 68 line evaluations as a dataflow program (two multiplication levels per tangent
     // instead of ~20 dependent products)
     if ((t.small_route & SMALL_LINES) && single && np <= t.small_lines_max && !serial_tail) {
@@ -266,6 +300,11 @@ inline miller_plan plan_miller(const thresholds &t, size_t np, size_t lines_cap,
         p.lines_last = last <= t.pair_lines_max ? LINES_LANES2 : LINES_THREAD;
     }
     return p;
+}
+
+// the plan's block products fit the workspace
+inline bool fits(const miller_plan &p, const miller_caps &c) {
+    return (size_t)p.nseg * p.row_stride <= c.f_cap && (size_t)p.nseg * p.ncols2 <= c.f2_cap;
 }
 
 // Window width c and count.  Cost model per candidate c: nwin * (11 n + 32 * 2^(c-1)) field multiplications (one

@@ -289,7 +289,8 @@ int hs_signature_from_bytes(const uint8_t *in, int len, int group_check, g2_aff 
 void hs_g1_compress(const g1_aff *p, uint8_t *out) { g1_compress(out, *p); }
 void hs_miller_combine(const fp12 *seg, int nseg, fp12 *out) { miller_combine(*out, seg, nseg); }
 
-// ---- route.hpp: the plans of the batch pipeline and of the MSM, thresholds read from the environment at every call ----
+// ---- route.hpp: the plans of the batch pipeline and of the MSM and the Miller-loop workspaces, thresholds read from the
+// environment at every call ----
 // out: the fields of route::batch_plan in declaration order
 void hs_plan_batch(size_t n, size_t total_n, uint32_t chunks, int host_src, int scalars, int use_side, int acc_team,
                    int serial_tail, int use_graph, int *out) {
@@ -304,6 +305,21 @@ void hs_plan_miller(size_t np, size_t lines_cap, int team, int serial_tail, long
     const route::miller_plan p = route::plan_miller(route::read_thresholds(), np, lines_cap, team != 0, serial_tail != 0);
     const long long v[6] = {p.G, p.nseg, p.lines, p.lines_last, (long long)p.ncols, p.gt_prog};
     memcpy(out, v, sizeof v);
+}
+// The Miller-loop workspace of a context of max_sets sets (sig == 0) or of the deferred signature pair (sig != 0).
+// out: lines_cap, f_cap, f2_cap, small_lines
+void hs_miller_caps(size_t max_sets, int sig, long long *out) {
+    const route::miller_caps c = sig ? route::miller_caps_sig() : route::miller_caps_batch(route::read_thresholds(), max_sets);
+    const long long v[4] = {(long long)c.lines_cap, (long long)c.f_cap, (long long)c.f2_cap, (long long)c.small_lines};
+    memcpy(out, v, sizeof v);
+}
+// the first np in 1 .. np_max whose Miller plan does not fit that workspace, 0 if every plan fits
+size_t hs_miller_misfit(size_t max_sets, int sig, size_t np_max, int team, int serial_tail) {
+    const route::thresholds t = route::read_thresholds();
+    const route::miller_caps c = sig ? route::miller_caps_sig() : route::miller_caps_batch(t, max_sets);
+    for (size_t np = 1; np <= np_max; np++)
+        if (!route::fits(route::plan_miller(t, np, c.lines_cap, team != 0, serial_tail != 0), c)) return np;
+    return 0;
 }
 // out: c, nwin, B, L, nseg, G, emax, horner_prog, scratch bytes of the G1 and of the G2 MSM, gw0[0..G], K[0..G-1],
 // preg[0..G]

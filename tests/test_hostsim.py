@@ -492,3 +492,49 @@ def test_route_plans(hs, monkeypatch):
             assert [c, nwin, B, L, nseg, G, gw0, K, preg, emax, prog, bytes_g1, bytes_g2] == want, (cfg["env"], inp)
         for k in cfg["env"]:
             monkeypatch.delenv(k)
+
+
+# context capacities at the edges of the Miller plan's regimes: tiles of 2^18 pairs, the latency and throughput rules
+# of miller_shape, the G steps of the throughput rule
+FIT_CAPS = [1, 2, 32, 33, 64, 129, 1024, 1025, 4096, 4097, 8192, 8193, 16384, 24575, 24576, 65535, 65536, 98303, 131072,
+            262143, 262144, 262145, 1 << 20]
+
+
+def test_miller_workspace_fit(hs, monkeypatch):
+    """route.hpp: the Miller-loop workspaces (miller_caps_batch, miller_caps_sig) hold every plan that runs on them.
+    A context of cap sets runs plans of 1 to cap + 1 pairs (the sets and the signature-side pair) on its batch workspace;
+    each one must fit, with team accumulation and the serial tail on and off, under the default thresholds and the
+    old accumulation-shape rule and with the small route off.  The deferred signature pair's one-pair plan must fit its
+    own workspace under every configuration of route_plans.json.  The capacities are those blsgpu_create allocated
+    before they moved into route.hpp."""
+    hs.hs_miller_misfit.restype = C.c_size_t
+    for k in [k for k in os.environ if k.startswith("BLSGPU_")]:
+        monkeypatch.delenv(k)
+    tile = 1 << 18
+    o = (C.c_longlong * 4)()
+    for cap in FIT_CAPS:
+        hs.hs_miller_caps(C.c_size_t(cap), 0, o)
+        f_cap = (cap + 1) // 2 + 40000 + 64 * ((cap + 1) // tile + 2)
+        assert list(o) == [(min(cap + 1, tile) + 31) & ~31, f_cap, f_cap // 8 + 4096, 1025], cap
+    hs.hs_miller_caps(C.c_size_t(0), 1, o)
+    assert list(o) == [32, 2048, 512, 2]
+    for env in ({}, {"BLSGPU_ACC_OLD_RULE": "1"}, {"BLSGPU_SMALL_ROUTE": "0"}):
+        for k, v in env.items():
+            monkeypatch.setenv(k, v)
+        for cap in FIT_CAPS:
+            for team in (1, 0):
+                for serial in (0, 1):
+                    assert hs.hs_miller_misfit(C.c_size_t(cap), 0, C.c_size_t(cap + 1), team, serial) == 0, (env, cap, team, serial)
+        for k in env:
+            monkeypatch.delenv(k)
+    for cfg in json.load(open(os.path.join(GOLD, "route_plans.json")))["configs"]:
+        for k, v in cfg["env"].items():
+            monkeypatch.setenv(k, v)
+        for team in (1, 0):
+            for serial in (0, 1):
+                assert hs.hs_miller_misfit(C.c_size_t(0), 1, C.c_size_t(1), team, serial) == 0, (cfg["env"], team, serial)
+        for k in cfg["env"]:
+            monkeypatch.delenv(k)
+    # the check can fail: one pair per group (BLSGPU_MILLER_G=0 clamps to 1) outgrows the block products at 3 001 pairs
+    monkeypatch.setenv("BLSGPU_MILLER_G", "0")
+    assert hs.hs_miller_misfit(C.c_size_t(4096), 0, C.c_size_t(4097), 1, 0) == 3001
