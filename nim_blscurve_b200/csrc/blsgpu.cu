@@ -2,6 +2,7 @@
 // Everything that computes runs in the kernels of kernels.cuh / msm.cuh; this file only moves bytes and
 // launches.  There is no CPU implementation of any operation behind these entry points.
 #include <cuda_runtime.h>
+#include <limits.h>
 #include <stddef.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -100,6 +101,8 @@ struct blsgpu_ctx {
     fp *d_norm = nullptr;                                    // [0] Fp norm taken out of the final exponentiation, [1] its inverse
     fp *d_consts = nullptr;                                  // Frobenius coefficients (fpprog::CONST_*)
     fp12 *d_gt = nullptr;                                    // final exponentiation result, Montgomery form
+    fp12 *d_fold = nullptr;                                  // levels of the product of many partials (fold_partials)
+    size_t fold_cap = 0;
     bool serial_tail = false;
     bool prog_smem_raised = false;                           // k_fp_program allowed > 48 KiB of shared memory on this device
     // host-buffer calls on large batches: the H2D copy is cut into H2D_SLICES pieces on a copy stream and the hash kernel
@@ -201,7 +204,7 @@ extern "C" void blsgpu_destroy(blsgpu_ctx *ctx) {
     cudaFree(ctx->d_P); cudaFree(ctx->d_S); cudaFree(ctx->d_partials); cudaFree(ctx->d_gtb);
     cudaFree(ctx->d_flags); cudaFree(ctx->d_dbg); cudaFree(ctx->d_misc); cudaFree(ctx->d_misc2); cudaFree(ctx->d_consts); cudaFree(ctx->d_gt);
     for (auto &kv : ctx->progs) cudaFree(kv.second.d);
-    cudaFree(ctx->d_norm); cudaFree(ctx->d_small);
+    cudaFree(ctx->d_norm); cudaFree(ctx->d_small); cudaFree(ctx->d_fold);
     msm_free(ctx->msm);
     if (ctx->h_pinned) cudaFreeHost(ctx->h_pinned);
     for (int i = 0; i < 2 * ST_COUNT + 5; i++) if (ctx->ev_valid[i]) cudaEventDestroy(ctx->ev[i]);
@@ -838,6 +841,42 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
     return 0;
 }
 
+// The final-exponentiation programs take at most FINAL_DIRECT_MAX partials: every partial holds 12 slots of the slot
+// file from the first round on, and from 25 partials on the pair of programs no longer fits it.
+static const int FINAL_DIRECT_MAX = 8;
+
+// Multiply `count` > FINAL_DIRECT_MAX partials eight at a time (product programs, one warp per group), level after level,
+// until at most FINAL_DIRECT_MAX remain; parts / count then name the last level.  The levels alternate between the two
+// halves of ctx->d_fold.
+static int fold_partials(blsgpu_ctx *ctx, cudaStream_t s, const fp12 *&parts, int &count) {
+    const size_t half = ((size_t)count + 7) / 8;
+    if (ctx->fold_cap < 2 * half) {
+        cudaFree(ctx->d_fold);
+        ctx->d_fold = nullptr;
+        ctx->fold_cap = 0;
+        CK(cudaMalloc((void **)&ctx->d_fold, 2 * half * sizeof(fp12)));
+        ctx->fold_cap = 2 * half;
+    }
+    for (int level = 0; count > FINAL_DIRECT_MAX; level++) {
+        fp12 *out = ctx->d_fold + (level & 1) * half;
+        const int full = count / 8, rest = count % 8;
+        blsgpu_ctx::dev_prog p8, pr;
+        int rc = get_prog(ctx, PROG_PRODUCT, 8, p8, s);
+        if (rc) return rc;
+        launch_prog_many(ctx, p8, s, (size_t)full, (const fp *)parts, 8 * 12, nullptr, 0, (fp *)out, 12);
+        if (rest > 1) {
+            rc = get_prog(ctx, PROG_PRODUCT, rest, pr, s);
+            if (rc) return rc;
+            launch_prog_many(ctx, pr, s, 1, (const fp *)(parts + 8 * full), 0, nullptr, 0, (fp *)(out + full), 0);
+        } else if (rest == 1) {
+            CK(cudaMemcpyAsync(out + full, parts + 8 * full, sizeof(fp12), cudaMemcpyDeviceToDevice, s));
+        }
+        parts = out;
+        count = full + (rest ? 1 : 0);
+    }
+    return 0;
+}
+
 // enqueue: product of the partials, final exponentiation, verdict + GT bytes, and their copies into h_pinned
 static int run_final_enqueue(blsgpu_ctx *ctx, int count, const fp12 *d_partials = nullptr, const int *d_rank_flags = nullptr) {
     cudaStream_t s = ctx->stream;
@@ -847,10 +886,15 @@ static int run_final_enqueue(blsgpu_ctx *ctx, int count, const fp12 *d_partials 
         k_final<<<1, 32, 0, s>>>(parts, count, d_rank_flags, ctx->d_gtb, ctx->d_flags + 1);
         ctx->launches++;
     } else {
-        // norm program -> one-thread binary-Euclid inversion -> main program (fpprog.hpp build_final)
+        // [fold ->] norm program -> one-thread binary-Euclid inversion -> main program (fpprog.hpp build_final)
+        int nparts = count;
+        if (nparts > FINAL_DIRECT_MAX) {
+            int rc = fold_partials(ctx, s, parts, nparts);
+            if (rc) return rc;
+        }
         blsgpu_ctx::dev_prog fpn, fpg;
-        int rc = get_prog(ctx, PROG_NORM, count, fpn, s);
-        if (!rc) rc = get_prog(ctx, PROG_FINAL, count, fpg, s);
+        int rc = get_prog(ctx, PROG_NORM, nparts, fpn, s);
+        if (!rc) rc = get_prog(ctx, PROG_FINAL, nparts, fpg, s);
         if (rc) return rc;
         rc = launch_prog(ctx, fpn, s, (const fp *)parts, ctx->d_norm);
         if (rc) return rc;
@@ -1136,6 +1180,7 @@ extern "C" int blsgpu_finalize_dev(blsgpu_ctx *ctx, const void *d_partials, size
     if (!ctx || !d_partials) return BLSGPU_ERR_ARG;
     if (gt_out) memset(gt_out, 0, 576);
     if (count == 0) return 0;
+    if (count > (size_t)INT_MAX) return fail(ctx, BLSGPU_ERR_ARG, "too many partials");
     CK(cudaSetDevice(ctx->device));
     int bad = 0;
     int rc = run_final(ctx, (int)count, gt_out, d_flags ? &bad : nullptr, (const fp12 *)d_partials, d_flags);

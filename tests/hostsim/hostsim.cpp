@@ -300,6 +300,27 @@ void hs_plan_batch(size_t n, size_t total_n, uint32_t chunks, int host_src, int 
                        p.chain_wait, p.graph, p.copy_ahead};
     memcpy(out, v, sizeof v);
 }
+// The routes of every batch of 1 .. n_max sets in a context of as many sets, under the default switches of blsgpu_create
+// (side streams, team accumulation, graph replay; no serial tail).  out: n_max rows of 14 ints = the fields of
+// route::batch_plan in declaration order, then the lines route of every tile but the last and of the last tile of the
+// Miller plan of the pairs the batch runs (n + 1, or n when the signature pair is deferred; blsgpu.cu run_partial_impl).
+void hs_plan_routes(size_t n_max, uint32_t chunks, int host_src, int scalars, int *out) {
+    const route::thresholds t = route::read_thresholds();
+    const route::switches sw = {true, true, false, true};
+    for (size_t n = 1; n <= n_max; n++, out += 14) {
+        const route::batch_plan p = route::plan_batch(t, sw, n, n, chunks, host_src != 0, scalars != 0);
+        const size_t np = p.defer_sig ? n : n + 1;
+        const route::miller_plan m = route::plan_miller(t, np, route::miller_caps_batch(t, n).lines_cap, true, false);
+        const int v[14] = {p.hash, p.sliced, p.small, p.sig, p.g1_aside, p.msm_after_hash, p.defer_sig, p.affine, p.chain_hog,
+                           p.chain_wait, p.graph, p.copy_ahead, m.lines, m.lines_last};
+        memcpy(out, v, sizeof v);
+    }
+}
+// 1 if the pair of final-exponentiation programs over `count` partials (norm, then the exponentiation around the
+// external inversion) builds within the slot file, as blsgpu.cu run_final_enqueue needs them
+int hs_prog_final_builds(int count) {
+    return fpprog::build_final(count, fpprog::INV_EMIT_ARG).ok && fpprog::build_final(count, fpprog::INV_EXTERNAL).ok;
+}
 // out: G, nseg, lines, lines_last, ncols, gt_prog
 void hs_plan_miller(size_t np, size_t lines_cap, int team, int serial_tail, long long *out) {
     const route::miller_plan p = route::plan_miller(route::read_thresholds(), np, lines_cap, team != 0, serial_tail != 0);
