@@ -667,6 +667,21 @@ def rlc_scalars(srb, n, chunks=0):
     return out
 
 
+def combine_scalars(srb, n):
+    """The n 64-bit scalars of MultiSignatureSet.combine (blst_min_pubkey_sig_core.nim:570-647): seed <- SHA256(seed)
+    whenever the four little-endian 64-bit words of the current seed are used up, taken from the last word down; zero
+    words are skipped."""
+    seed, avail, sc = srb, 0, []
+    while len(sc) < n:
+        if avail == 0:
+            seed, avail = hashlib.sha256(seed).digest(), 4
+        avail -= 1
+        v = int.from_bytes(seed[8 * avail:8 * avail + 8], "little")
+        if v:
+            sc.append(v)
+    return sc
+
+
 def batch_verify(sets, srb, chunks=0, scalars=None):
     """sets: list of (pk affine|None, msg bytes, sig affine|None).  Returns (ok, gt_bytes|None).
 

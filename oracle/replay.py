@@ -340,15 +340,7 @@ def _ref_combine(srb, pks, sigs):
     n = len(pks) // 96
     if n == 1:
         return pks, sigs
-    seed, avail, sc = srb, 0, []
-    while len(sc) < n:
-        if avail == 0:
-            seed, avail = hashlib.sha256(seed).digest(), 4
-        avail -= 1
-        v = int.from_bytes(seed[8 * avail:8 * avail + 8], "little")
-        if v:
-            sc.append(v)
-    scb = b"".join(v.to_bytes(8, "little") for v in sc)
+    scb = b"".join(v.to_bytes(8, "little") for v in pr.combine_scalars(srb, n))
     return _ref_msm(pks, scb, 64, False), _ref_msm(sigs, scb, 64, True)
 
 

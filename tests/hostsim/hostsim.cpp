@@ -355,4 +355,28 @@ void hs_plan_msm(size_t n, int nbits, int sms, long long *out) {
     for (int g = 0; g < p.G; g++) *o++ = p.K[g];
     for (int g = 0; g <= p.G; g++) *o++ = (long long)p.preg[g];
 }
+// The runs of equal MSM shape over n = 1 .. n_max points with nbits-bit scalars on `sms` SMs.  The shape is (c, nwin, L,
+// nseg, G, horner_prog, and for every group whether its chunk length K sits at its floor of 8); K above the floor grows
+// with n and is not part of it.  out: (first n, last n) of each run, at most cap runs; returns the number of runs, or
+// -1 if there are more than cap.
+int hs_msm_runs(int nbits, int sms, size_t n_max, long long *out, int cap) {
+    const route::thresholds t = route::read_thresholds();
+    long long prev[15] = {}, cur[15];
+    int runs = 0;
+    for (size_t n = 1; n <= n_max; n++) {
+        const route::msm_plan p = route::plan_msm(t, n, nbits, sms);
+        const long long v[7] = {p.c, p.nwin, (long long)p.L, (long long)p.nseg, p.G, p.horner_prog, 0};
+        memcpy(cur, v, sizeof v);
+        for (int g = 0; g < 8; g++) cur[7 + g] = g < p.G && p.K[g] == 8;
+        if (n == 1 || memcmp(cur, prev, sizeof cur) != 0) {
+            if (runs == cap) return -1;
+            if (runs) out[2 * runs - 1] = (long long)n - 1;
+            out[2 * runs] = (long long)n;
+            runs++;
+            memcpy(prev, cur, sizeof cur);
+        }
+    }
+    if (runs) out[2 * runs - 1] = (long long)n_max;
+    return runs;
+}
 }
