@@ -149,6 +149,17 @@ static int fail(blsgpu_ctx *c, int code, const char *what, cudaError_t e = cudaS
 
 static inline unsigned nblk(size_t n, unsigned bs = 128) { return (unsigned)((n + bs - 1) / bs); }
 
+// pairwise tree sum of the n Jacobian points at J into J[0], one launch per level; returns the number of launches
+template <class F> static int tree_sum(jac_t<F> *J, size_t n, cudaStream_t s) {
+    int levels = 0;
+    for (size_t m = n; m > 1; levels++) {
+        size_t half = (m + 1) / 2;
+        k_pt_tree<F><<<nblk(half), 128, 0, s>>>(J, m, half);
+        m = half;
+    }
+    return levels;
+}
+
 // the route thresholds, read from the environment once per process (route.hpp)
 static const route::thresholds &thr() {
     static const route::thresholds t = route::read_thresholds();
@@ -781,12 +792,7 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
         }
         END(ST_G2MUL, g);
         BEGIN(ST_G2SUM, g);
-        for (size_t m = n; m > 1;) {
-            size_t half = (m + 1) / 2;
-            k_g2_tree<<<nblk(half), 128, 0, g>>>(ctx->d_S, m, half);
-            ctx->launches++;
-            m = half;
-        }
+        ctx->launches += tree_sum(ctx->d_S, n, g);
     }
     k_sig_pair<<<1, 32, 0, g>>>(ctx->d_S, n, ctx->d_Q, ctx->d_P);
     ctx->launches++;
@@ -1245,54 +1251,39 @@ extern "C" int blsgpu_test_small_hash(blsgpu_ctx *ctx, const void *sets320, size
     return 0;
 }
 
-extern "C" int blsgpu_aggregate_g1(blsgpu_ctx *ctx, const void *points96, size_t n, uint8_t out96[96]) {
-    if (!ctx || !out96) return BLSGPU_ERR_ARG;
-    if (n == 0) return 0;                                   // blst_min_pubkey_sig_core.nim:183-184
-    if (!points96) return BLSGPU_ERR_ARG;
+// aggregateAll (blst_min_pubkey_sig_core.nim:179-195): tree sum of n affine points, one inversion
+template <class F> static int aggregate_all(blsgpu_ctx *ctx, const void *points, size_t n, uint8_t *out) {
+    if (!ctx || !out) return BLSGPU_ERR_ARG;
+    if (n == 0) return 0;                                   // :183-184
+    if (!points) return BLSGPU_ERR_ARG;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->stream;
-    int rc = ensure_misc(ctx, n * (sizeof(g1_aff) + sizeof(g1_jac)) + 256);
+    int rc = ensure_misc(ctx, n * (sizeof(aff_t<F>) + sizeof(jac_t<F>)) + 256);
     if (rc) return rc;
-    g1_jac *J = (g1_jac *)ctx->d_misc;
-    g1_aff *A = (g1_aff *)((uint8_t *)ctx->d_misc + n * sizeof(g1_jac));
-    CK(cudaMemcpyAsync(A, points96, n * sizeof(g1_aff), cudaMemcpyHostToDevice, s));
-    k_g1_load<<<nblk(n), 128, 0, s>>>(A, n, J);
-    for (size_t m = n; m > 1;) { size_t half = (m + 1) / 2; k_g1_tree<<<nblk(half), 128, 0, s>>>(J, m, half); m = half; }
-    k_g1_to_affine<<<1, 32, 0, s>>>(J, A);
+    jac_t<F> *J = (jac_t<F> *)ctx->d_misc;
+    aff_t<F> *A = (aff_t<F> *)((uint8_t *)ctx->d_misc + n * sizeof(jac_t<F>));
+    CK(cudaMemcpyAsync(A, points, n * sizeof(aff_t<F>), cudaMemcpyHostToDevice, s));
+    k_pt_load<F><<<nblk(n), 128, 0, s>>>(A, n, J);
+    tree_sum(J, n, s);
+    k_pt_to_affine<F><<<1, 32, 0, s>>>(J, A);
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(out96, A, 96, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(out, A, sizeof(aff_t<F>), cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     return 1;
 }
 
+extern "C" int blsgpu_aggregate_g1(blsgpu_ctx *ctx, const void *points96, size_t n, uint8_t out96[96]) {
+    return aggregate_all<fp>(ctx, points96, n, out96);
+}
 extern "C" int blsgpu_aggregate_g2(blsgpu_ctx *ctx, const void *points192, size_t n, uint8_t out192[192]) {
-    if (!ctx || !out192) return BLSGPU_ERR_ARG;
-    if (n == 0) return 0;
-    if (!points192) return BLSGPU_ERR_ARG;
-    CK(cudaSetDevice(ctx->device));
-    cudaStream_t s = ctx->stream;
-    int rc = ensure_misc(ctx, n * (sizeof(g2_aff) + sizeof(g2_jac)) + 256);
-    if (rc) return rc;
-    g2_jac *J = (g2_jac *)ctx->d_misc;
-    g2_aff *A = (g2_aff *)((uint8_t *)ctx->d_misc + n * sizeof(g2_jac));
-    CK(cudaMemcpyAsync(A, points192, n * sizeof(g2_aff), cudaMemcpyHostToDevice, s));
-    k_g2_load<<<nblk(n), 128, 0, s>>>(A, n, J);
-    for (size_t m = n; m > 1;) { size_t half = (m + 1) / 2; k_g2_tree<<<nblk(half), 128, 0, s>>>(J, m, half); m = half; }
-    k_g2_to_affine<<<1, 32, 0, s>>>(J, A);
-    CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(out192, A, 192, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    return 1;
+    return aggregate_all<fp2>(ctx, points192, n, out192);
 }
 
 // ---- SURVEY §8f N1: subtractAll (blst_min_pubkey_sig_core.nim:197-209) ----
 // dst - sum(elems) computed as -((sum(elems)) + (-dst)): one tree over n + 1 points with the negated dst in the last
 // slot, one negation of the root, one inversion.  Affine output, hence bit-identical to the reference's
 // aggregate / cneg / aggregate(dst) / finish sequence whatever the order of the additions.
-template <class F> static int subtract_all(blsgpu_ctx *ctx, void *dst, const void *elems, size_t n,
-                                           void (*load)(const aff_t<F> *, size_t, jac_t<F> *, cudaStream_t),
-                                           void (*tree)(jac_t<F> *, size_t, size_t, cudaStream_t),
-                                           void (*to_affine)(const jac_t<F> *, aff_t<F> *, cudaStream_t)) {
+template <class F> static int subtract_all(blsgpu_ctx *ctx, void *dst, const void *elems, size_t n) {
     if (!ctx || !dst) return BLSGPU_ERR_ARG;
     if (n == 0) return 1;                                   // :199-200: dst untouched
     if (!elems) return BLSGPU_ERR_ARG;
@@ -1305,11 +1296,11 @@ template <class F> static int subtract_all(blsgpu_ctx *ctx, void *dst, const voi
     aff_t<F> *A = (aff_t<F> *)((uint8_t *)ctx->d_misc + m * sizeof(jac_t<F>));
     CK(cudaMemcpyAsync(A, elems, n * sizeof(aff_t<F>), cudaMemcpyHostToDevice, s));
     CK(cudaMemcpyAsync(A + n, dst, sizeof(aff_t<F>), cudaMemcpyHostToDevice, s));
-    load(A, m, J, s);
+    k_pt_load<F><<<nblk(m), 128, 0, s>>>(A, m, J);
     k_pt_neg<F><<<1, 32, 0, s>>>(J + n);
-    for (size_t k = m; k > 1;) { size_t half = (k + 1) / 2; tree(J, k, half, s); k = half; }
+    tree_sum(J, m, s);
     k_pt_neg<F><<<1, 32, 0, s>>>(J);
-    to_affine(J, A, s);
+    k_pt_to_affine<F><<<1, 32, 0, s>>>(J, A);
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(dst, A, sizeof(aff_t<F>), cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
@@ -1317,19 +1308,10 @@ template <class F> static int subtract_all(blsgpu_ctx *ctx, void *dst, const voi
 }
 
 extern "C" int blsgpu_subtract_g1(blsgpu_ctx *ctx, uint8_t dst96[96], const void *elems96, size_t n) {
-    return subtract_all<fp>(
-        ctx, dst96, elems96, n,
-        [](const g1_aff *a, size_t m, g1_jac *j, cudaStream_t s) { k_g1_load<<<nblk(m), 128, 0, s>>>(a, m, j); },
-        [](g1_jac *j, size_t k, size_t half, cudaStream_t s) { k_g1_tree<<<nblk(half), 128, 0, s>>>(j, k, half); },
-        [](const g1_jac *j, g1_aff *a, cudaStream_t s) { k_g1_to_affine<<<1, 32, 0, s>>>(j, a); });
+    return subtract_all<fp>(ctx, dst96, elems96, n);
 }
-
 extern "C" int blsgpu_subtract_g2(blsgpu_ctx *ctx, uint8_t dst192[192], const void *elems192, size_t n) {
-    return subtract_all<fp2>(
-        ctx, dst192, elems192, n,
-        [](const g2_aff *a, size_t m, g2_jac *j, cudaStream_t s) { k_g2_load<<<nblk(m), 128, 0, s>>>(a, m, j); },
-        [](g2_jac *j, size_t k, size_t half, cudaStream_t s) { k_g2_tree<<<nblk(half), 128, 0, s>>>(j, k, half); },
-        [](const g2_jac *j, g2_aff *a, cudaStream_t s) { k_g2_to_affine<<<1, 32, 0, s>>>(j, a); });
+    return subtract_all<fp2>(ctx, dst192, elems192, n);
 }
 
 // ---- SURVEY §8f N3: aggregateVerify / fastAggregateVerify on the device ----
@@ -1462,10 +1444,10 @@ extern "C" int blsgpu_aggregate_g1_segments(blsgpu_ctx *ctx, const void *points9
 }
 
 // ---- SURVEY §8f N2: batched fromBytes with checks ----
-template <int G2>
+template <class F>
 static int from_bytes_api(blsgpu_ctx *ctx, const uint8_t *in, size_t n, size_t in_len, int group_check, uint8_t *out,
                           uint8_t *status) {
-    const size_t pb = G2 ? 192 : 96, clen = G2 ? 96 : 48;
+    const size_t pb = sizeof(aff_t<F>), clen = sizeof(F);
     if (!ctx || !out) return BLSGPU_ERR_ARG;
     if (n == 0) return 1;
     if (!in) return BLSGPU_ERR_ARG;
@@ -1479,10 +1461,8 @@ static int from_bytes_api(blsgpu_ctx *ctx, const uint8_t *in, size_t n, size_t i
     uint8_t *base = (uint8_t *)ctx->d_misc;
     CK(cudaMemcpyAsync(base + o_in, in, n * in_len, cudaMemcpyHostToDevice, s));
     CK(cudaMemsetAsync(base + o_cnt, 0, 4, s));
-    if (G2) k_signatures_from_bytes<<<nblk(n), 128, 0, s>>>(base + o_in, n, (int)in_len, group_check, (g2_aff *)(base + o_out),
-                                                            base + o_st, (int *)(base + o_cnt));
-    else k_pubkeys_from_bytes<<<nblk(n), 128, 0, s>>>(base + o_in, n, (int)in_len, group_check, (g1_aff *)(base + o_out),
-                                                      base + o_st, (int *)(base + o_cnt));
+    k_pt_from_bytes<F><<<nblk(n), 128, 0, s>>>(base + o_in, n, (int)in_len, group_check, (aff_t<F> *)(base + o_out), base + o_st,
+                                               (int *)(base + o_cnt));
     ctx->launches = 1;
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(out, base + o_out, n * pb, cudaMemcpyDeviceToHost, s));
@@ -1496,16 +1476,16 @@ static int from_bytes_api(blsgpu_ctx *ctx, const uint8_t *in, size_t n, size_t i
 
 extern "C" int blsgpu_pubkeys_from_bytes(blsgpu_ctx *ctx, const uint8_t *in, size_t n, size_t in_len, int group_check,
                                          uint8_t *out96, uint8_t *status) {
-    return from_bytes_api<0>(ctx, in, n, in_len, group_check, out96, status);
+    return from_bytes_api<fp>(ctx, in, n, in_len, group_check, out96, status);
 }
 extern "C" int blsgpu_signatures_from_bytes(blsgpu_ctx *ctx, const uint8_t *in, size_t n, size_t in_len, int group_check,
                                             uint8_t *out192, uint8_t *status) {
-    return from_bytes_api<1>(ctx, in, n, in_len, group_check, out192, status);
+    return from_bytes_api<fp2>(ctx, in, n, in_len, group_check, out192, status);
 }
 
-template <int G2>
+template <class F>
 static int compress_api(blsgpu_ctx *ctx, const void *points, size_t n, uint8_t *out) {
-    const size_t pb = G2 ? 192 : 96, clen = G2 ? 96 : 48;
+    const size_t pb = sizeof(aff_t<F>), clen = sizeof(F);
     if (!ctx || !out) return BLSGPU_ERR_ARG;
     if (n == 0) return 1;
     if (!points) return BLSGPU_ERR_ARG;
@@ -1516,8 +1496,7 @@ static int compress_api(blsgpu_ctx *ctx, const void *points, size_t n, uint8_t *
     if (rc) return rc;
     uint8_t *base = (uint8_t *)ctx->d_misc;
     CK(cudaMemcpyAsync(base, points, n * pb, cudaMemcpyHostToDevice, s));
-    if (G2) k_g2_compress<<<nblk(n), 128, 0, s>>>((const g2_aff *)base, n, base + o_out);
-    else k_g1_compress<<<nblk(n), 128, 0, s>>>((const g1_aff *)base, n, base + o_out);
+    k_pt_compress<F><<<nblk(n), 128, 0, s>>>((const aff_t<F> *)base, n, base + o_out);
     ctx->launches = 1;
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(out, base + o_out, n * clen, cudaMemcpyDeviceToHost, s));
@@ -1525,10 +1504,10 @@ static int compress_api(blsgpu_ctx *ctx, const void *points, size_t n, uint8_t *
     return 1;
 }
 extern "C" int blsgpu_pubkeys_to_bytes(blsgpu_ctx *ctx, const void *points96, size_t n, uint8_t *out48) {
-    return compress_api<0>(ctx, points96, n, out48);
+    return compress_api<fp>(ctx, points96, n, out48);
 }
 extern "C" int blsgpu_signatures_to_bytes(blsgpu_ctx *ctx, const void *points192, size_t n, uint8_t *out96) {
-    return compress_api<1>(ctx, points192, n, out96);
+    return compress_api<fp2>(ctx, points192, n, out96);
 }
 
 template <class F>
@@ -1620,7 +1599,7 @@ static int msm_api_multi(blsgpu_ctx *lead, const uint8_t *points, const uint8_t 
     }
     cudaSetDevice(lead->device);
     if (rc) return rc;
-    rc = sizeof(F) == sizeof(fp) ? blsgpu_aggregate_g1(lead, parts.data(), ndev, out) : blsgpu_aggregate_g2(lead, parts.data(), ndev, out);
+    rc = aggregate_all<F>(lead, parts.data(), ndev, out);
     lead->launches = launches;
     return rc;
 }

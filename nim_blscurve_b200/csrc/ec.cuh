@@ -231,6 +231,38 @@ template <class F> BLS_NOINLINE void pt_to_affine_zinv(aff_t<F> &r, const jac_t<
     f_mul(r.y, p.y, zi2);
 }
 
+// Homogeneous (X : Y : Z), x = X / Z and y = Y / Z: the point form of the dataflow programs (fpprog.hpp), 3 F per point.
+// from Jacobian: (X Z : Y : Z^3); infinity -> (0 : 1 : 0)
+template <class F> BLS_NOINLINE void pt_jac_to_hom(F *h, const jac_t<F> &p) {
+    F x, y, z;
+    if (pt_is_inf(p)) {
+        f_set_zero(x); f_set_one(y); f_set_zero(z);
+    } else {
+        F z2;
+        f_mul(x, p.x, p.z);
+        y = p.y;
+        f_sqr(z2, p.z);
+        f_mul(z, z2, p.z);
+    }
+    h[0] = x; h[1] = y; h[2] = z;
+}
+
+// to Jacobian (X Z, Y Z^2, Z); Z = 0 -> infinity
+template <class F> BLS_FN void pt_hom_to_jac(jac_t<F> &r, const F *h) {
+    const F X = h[0], Y = h[1], Z = h[2];
+    if (f_is_zero(Z)) pt_set_inf(r);
+    else { F z2; f_mul(r.x, X, Z); f_sqr(z2, Z); f_mul(r.y, Y, z2); r.z = Z; }
+}
+
+// to affine (X / Z, Y / Z) through the variable-time inversion; Z = 0 -> 0 -> the all-zero affine encoding of infinity
+template <class F> BLS_FN void pt_hom_to_affine(aff_t<F> &r, const F *h) {
+    const F X = h[0], Y = h[1], Z = h[2];
+    F zi;
+    f_inv_vt(zi, Z);
+    f_mul(r.x, X, zi);
+    f_mul(r.y, Y, zi);
+}
+
 // r = [k]P for a 64-bit k, P affine: MSB-first double-and-add with mixed additions.
 // (BLST uses a 5-bit Booth window, ec_mult.h:178-223; the affine result is the same point.)
 template <class F> BLS_NOINLINE void pt_mul_u64(jac_t<F> &r, const aff_t<F> &p, uint64_t k) {

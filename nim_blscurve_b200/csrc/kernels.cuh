@@ -5,7 +5,7 @@
 //   k_hash_sets     A3  map_to_g2.c:388-396                               H(m_i), Jacobian
 //   k_g1_mul        A5  ec_mult.h:178-223 (G1)                            [r_i] pk_i, Jacobian
 //   k_pairs_affine  A4  e2.c:97-112, e1.c:60-75                           one shared inversion per set
-//   k_g2_mul        A5  ec_mult.h:178-223 (G2)                            [r_i] sig_i ; k_g2_tree sums them
+//   k_g2_mul        A5  ec_mult.h:178-223 (G2)                            [r_i] sig_i ; k_pt_tree sums them
 //   k_sig_pair      A9  aggregate.c:479-495                               (S, -G1) becomes pair number n
 //   k_miller_lines  A7  pairing.c:220-261 (line_dbl/line_add/line_by_Px2) 68 line triples per pair, word-major
 //   k_miller_acc    A6/A7/A8 pairing.c:253-260, aggregate.c:410-458       per (group, segment) Fp12 + block product
@@ -13,6 +13,7 @@
 //   k_final         A9/A10 pairing.c:371-404, fp12_tower.c:773-786        product, final exp, ==1, GT bytes
 #pragma once
 #include <cuda_runtime.h>
+#include <type_traits>
 #include "../../include/blsgpu.h"
 #include "h2c.cuh"
 #include "pairing.cuh"
@@ -247,20 +248,6 @@ __global__ void __launch_bounds__(128, BLS_LB_BLOCKS) k_miller_lines_lanes2(cons
 }
 
 // ---- small-batch route (<= 1024 sets): the long serial stretches run as per-set dataflow programs ----
-// homogeneous (X : Y : Z) over Fp2 <- Jacobian; infinity -> (0 : 1 : 0)
-BLS_NOINLINE void g2_jac_to_hom(fp *hom, const g2_jac &p) {
-    fp2 x, y, z;
-    if (pt_is_inf(p)) {
-        fp2_set_zero(x); fp2_set_zero(y); y.c0 = FP_ONE; fp2_set_zero(z);
-    } else {
-        fp2 z2;
-        fp2_mul(x, p.x, p.z);
-        y = p.y;
-        fp2_sqr(z2, p.z);
-        fp2_mul(z, z2, p.z);
-    }
-    hom[0] = x.c0; hom[1] = x.c1; hom[2] = y.c0; hom[3] = y.c1; hom[4] = z.c0; hom[5] = z.c1;
-}
 // first half of k_hash_sets_pair: XMD, one SSWU map per lane, sum on E2', 3-isogeny; the cofactor clearing follows
 // as a program (fpprog.hpp build_g2_clear_cofactor)
 __global__ void BLS_LB k_hash_map_pair(const sigset *sets, size_t n, fp *hom) {
@@ -283,7 +270,7 @@ __global__ void BLS_LB k_hash_map_pair(const sigset *sets, size_t n, fp *hom) {
     if (odd || !live) return;
     pt_add(q, q, other, &SSWU_A);
     iso3_g2(q, q);
-    g2_jac_to_hom(hom + 6 * i, q);
+    pt_jac_to_hom((fp2 *)hom + 3 * i, q);
 }
 // The same on lane pairs with every Fp2 operation split over the two lanes (pair_route.cuh): the two square-root chains
 // still run one map per lane, and the Fp2 stretches around them (SSWU, sum on E2', isogeny) take half as long.
@@ -328,30 +315,20 @@ __global__ void BLS_LB k_hash_map_pair_msgs(const uint8_t *msgs, const uint32_t 
     if (odd || !live) return;
     pt_add(q, q, other, &SSWU_A);
     iso3_g2(q, q);
-    g2_jac_to_hom(hom + 6 * i, q);
+    pt_jac_to_hom((fp2 *)hom + 3 * i, q);
 }
-// homogeneous (X : Y : Z) -> affine (X / Z, Y / Z), one working lane per warp-sized block (binary-Euclid inversion)
+// homogeneous -> affine, one working lane per warp-sized block (binary-Euclid inversion)
 __global__ void k_g2_hom_to_affine(const fp *hom, size_t n, g2_aff *out) {
     if (threadIdx.x != 0 || blockIdx.x >= n) return;
-    const fp *h = hom + 6 * (size_t)blockIdx.x;
-    fp2 X, Y, Z, zi;
-    X.c0 = h[0]; X.c1 = h[1]; Y.c0 = h[2]; Y.c1 = h[3]; Z.c0 = h[4]; Z.c1 = h[5];
     g2_aff a;
-    fp2_inv_vartime(zi, Z);                 // Z = 0 -> 0 -> the all-zero affine encoding of infinity
-    fp2_mul(a.x, X, zi);
-    fp2_mul(a.y, Y, zi);
+    pt_hom_to_affine(a, (const fp2 *)hom + 3 * (size_t)blockIdx.x);
     out[blockIdx.x] = a;
 }
-// homogeneous (X : Y : Z) -> Jacobian (X Z, Y Z^2, Z); Z = 0 -> infinity
 __global__ void k_g2_hom_to_jac(const fp *hom, size_t n, g2_jac *out) {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const fp *h = hom + 6 * i;
-    fp2 X, Y, Z;
-    X.c0 = h[0]; X.c1 = h[1]; Y.c0 = h[2]; Y.c1 = h[3]; Z.c0 = h[4]; Z.c1 = h[5];
     g2_jac j;
-    if (fp2_is_zero(Z)) pt_set_inf(j);
-    else { fp2 z2; fp2_mul(j.x, X, Z); fp2_sqr(z2, Z); fp2_mul(j.y, Y, z2); j.z = Z; }
+    pt_hom_to_jac(j, (const fp2 *)hom + 3 * i);
     out[i] = j;
 }
 // inputs of the [r_i] sig_i program (build_g2_mul64): the signature as (x : y : 1) (infinity (0 : 1 : 0)) and the 64
@@ -368,7 +345,7 @@ __global__ void k_g2_mul_prep(const sigset *sets, const uint64_t *r, size_t n, f
         g2_aff a = sets[i].sig;
         g2_jac j;
         pt_from_affine(j, a);
-        g2_jac_to_hom(hom + 6 * i, j);
+        pt_jac_to_hom((fp2 *)hom + 3 * i, j);
     }
 }
 
@@ -492,29 +469,14 @@ __global__ void BLS_LB k_g2_mul(const sigset *sets, const uint64_t *r, size_t n,
     S[i] = j;
 }
 
-// pairwise tree step: x[i] (op)= x[i + half] for i + half < n
-__global__ void BLS_LB k_g2_tree(g2_jac *S, size_t n, size_t half) {
+// pairwise tree step: S[i] += S[i + half] for i + half < n
+template <class F>
+__global__ void BLS_LB k_pt_tree(jac_t<F> *S, size_t n, size_t half) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= half || i + half >= n) return;
-    g2_jac a = S[i], b = S[i + half];
+    jac_t<F> a = S[i], b = S[i + half];
     pt_add(a, a, b);
     S[i] = a;
-}
-
-__global__ void BLS_LB k_g1_tree(g1_jac *S, size_t n, size_t half) {
-    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= half || i + half >= n) return;
-    g1_jac a = S[i], b = S[i + half];
-    pt_add(a, a, b);
-    S[i] = a;
-}
-
-__global__ void BLS_LB k_fp12_tree(fp12 *F, size_t n, size_t half) {
-    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= half || i + half >= n) return;
-    fp12 a = F[i], b = F[i + half];
-    fp12_mul(a, a, b);
-    F[i] = a;
 }
 
 // ---- split Miller loop (pairing.cuh): lines per pair, then accumulation per (group, segment) ----
@@ -1024,72 +986,48 @@ __global__ void BLS_LB k_g1_to_affine_many(const g1_jac *in, size_t n, g1_aff *o
     out[i] = a;
 }
 
-// ---- batched fromBytes with checks (SURVEY §8f N2; io.cuh) ----
-__global__ void BLS_LB k_pubkeys_from_bytes(const uint8_t *in, size_t n, int len, int group_check, g1_aff *out,
-                                            uint8_t *status, int *nfail) {
+// ---- batched fromBytes with checks (SURVEY §8f N2; io.cuh): public keys in G1, signatures in G2 ----
+// `len` is the compressed (sizeof(F)) or the serialized (sizeof(aff_t<F>)) size
+template <class F>
+__global__ void BLS_LB k_pt_from_bytes(const uint8_t *in, size_t n, int len, int group_check, aff_t<F> *out, uint8_t *status,
+                                       int *nfail) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    uint8_t raw[96];
+    uint8_t raw[sizeof(aff_t<F>)];
     for (int k = 0; k < len; k++) raw[k] = in[i * len + k];
-    g1_aff p;
-    int err = pubkey_from_bytes(p, raw, len, group_check != 0);
+    aff_t<F> p;
+    int err;
+    if constexpr (std::is_same<F, fp>::value) err = pubkey_from_bytes(p, raw, len, group_check != 0);
+    else err = signature_from_bytes(p, raw, len, group_check != 0);
     out[i] = p;
     status[i] = (uint8_t)err;
     if (err) atomicAdd(nfail, 1);
 }
-__global__ void BLS_LB k_signatures_from_bytes(const uint8_t *in, size_t n, int len, int group_check, g2_aff *out,
-                                               uint8_t *status, int *nfail) {
+// Zcash compressed encoding: sizeof(F) bytes per point
+template <class F>
+__global__ void k_pt_compress(const aff_t<F> *in, size_t n, uint8_t *out) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    uint8_t raw[192];
-    for (int k = 0; k < len; k++) raw[k] = in[i * len + k];
-    g2_aff p;
-    int err = signature_from_bytes(p, raw, len, group_check != 0);
-    out[i] = p;
-    status[i] = (uint8_t)err;
-    if (err) atomicAdd(nfail, 1);
-}
-__global__ void k_g1_compress(const g1_aff *in, size_t n, uint8_t *out) {
-    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    g1_aff a = in[i];
-    g1_compress(out + 48 * i, a);
-}
-__global__ void k_g2_compress(const g2_aff *in, size_t n, uint8_t *out) {
-    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    g2_aff a = in[i];
-    g2_compress(out + 96 * i, a);
+    aff_t<F> a = in[i];
+    if constexpr (std::is_same<F, fp>::value) g1_compress(out + sizeof(F) * i, a);
+    else g2_compress(out + sizeof(F) * i, a);
 }
 
 // ---- aggregateAll helpers ----
-__global__ void __launch_bounds__(128) k_g1_load(const g1_aff *in, size_t n, g1_jac *out) {
+template <class F>
+__global__ void __launch_bounds__(128) k_pt_load(const aff_t<F> *in, size_t n, jac_t<F> *out) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    g1_aff a = in[i];
-    g1_jac j;
+    aff_t<F> a = in[i];
+    jac_t<F> j;
     pt_from_affine(j, a);
     out[i] = j;
 }
-__global__ void __launch_bounds__(128) k_g2_load(const g2_aff *in, size_t n, g2_jac *out) {
-    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    g2_aff a = in[i];
-    g2_jac j;
-    pt_from_affine(j, a);
-    out[i] = j;
-}
-__global__ void k_g1_to_affine(const g1_jac *in, g1_aff *out) {
+template <class F>
+__global__ void k_pt_to_affine(const jac_t<F> *in, aff_t<F> *out) {
     if (blockIdx.x != 0 || threadIdx.x != 0) return;
-    g1_jac j = *in;
-    g1_aff a;
-    pt_to_affine_vt(a, j);
-    *out = a;
-}
-__global__ void k_g2_to_affine(const g2_jac *in, g2_aff *out) {
-    if (blockIdx.x != 0 || threadIdx.x != 0) return;
-    g2_jac j = *in;
-    g2_aff a;
+    jac_t<F> j = *in;
+    aff_t<F> a;
     pt_to_affine_vt(a, j);
     *out = a;
 }

@@ -22,7 +22,6 @@
 #pragma once
 #include <functional>
 #include <string>
-#include <type_traits>
 #include "kernels.cuh"
 #include "route.hpp"
 
@@ -336,68 +335,28 @@ __global__ void k_msm_horner(const jac_t<F> *W, size_t stride, int nwin, int c, 
     }
 }
 
-// G1 window Horner as a warp-cooperative dataflow program (fpprog.hpp build_msm_horner_g1, run by k_fp_program):
+// Window Horner as a warp-cooperative dataflow program (fpprog.hpp build_msm_horner_g1 / _g2, run by k_fp_program):
 // the 255 sequential doublings cost two multiplication levels each instead of seven dependent multiplications.
-// prep: window sums, Jacobian (X, Y, Z) -> homogeneous (X Z : Y : Z^3), infinity -> (0 : 1 : 0)
-__global__ void k_msm_horner_prep(const g1_jac *W, size_t stride, int nwin, fp *hom) {
+// prep: window sums -> homogeneous (ec.cuh pt_jac_to_hom), 3 F per window
+template <class F>
+__global__ void k_msm_horner_prep(const jac_t<F> *W, size_t stride, int nwin, fp *hom) {
     const int w = blockIdx.x * blockDim.x + threadIdx.x;
     if (w >= nwin) return;
-    g1_jac p = W[(size_t)w * stride];
-    fp x, y, z;
-    if (pt_is_inf(p)) {
-        fp_set_zero(x); y = FP_ONE; fp_set_zero(z);
-    } else {
-        fp z2;
-        fp_mul_ni(x, p.x, p.z);
-        y = p.y;
-        fp_sqr_ni(z2, p.z);
-        fp_mul_ni(z, z2, p.z);
-    }
-    hom[3 * w] = x; hom[3 * w + 1] = y; hom[3 * w + 2] = z;
+    jac_t<F> p = W[(size_t)w * stride];
+    pt_jac_to_hom((F *)hom + 3 * w, p);
 }
-// finish: homogeneous (X : Y : Z) -> affine (X/Z, Y/Z) and/or Jacobian (X Z, Y Z^2, Z); infinity -> all zero
-__global__ void k_msm_horner_finish(const fp *hom, g1_jac *out_jac, g1_aff *out_aff) {
+// finish: homogeneous result -> Jacobian and/or affine; infinity -> Z = 0 / all zero
+template <class F>
+__global__ void k_msm_horner_finish(const fp *hom, jac_t<F> *out_jac, aff_t<F> *out_aff) {
     if (blockIdx.x != 0 || threadIdx.x != 0) return;
-    fp X = hom[0], Y = hom[1], Z = hom[2];
     if (out_jac) {
-        g1_jac j;
-        if (fp_is_zero(Z)) pt_set_inf(j);
-        else { fp z2; fp_mul_ni(j.x, X, Z); fp_sqr_ni(z2, Z); fp_mul_ni(j.y, Y, z2); j.z = Z; }
+        jac_t<F> j;
+        pt_hom_to_jac(j, (const F *)hom);
         *out_jac = j;
     }
     if (out_aff) {
-        g1_aff a;
-        fp zi;
-        fp_inv_vartime(zi, Z);
-        fp_mul_ni(a.x, X, zi);
-        fp_mul_ni(a.y, Y, zi);
-        *out_aff = a;
-    }
-}
-
-// the G2 forms (window sums of the signature-side MSM; Jacobian result only)
-__global__ void k_msm_horner_prep_g2(const g2_jac *W, size_t stride, int nwin, fp *hom) {
-    const int w = blockIdx.x * blockDim.x + threadIdx.x;
-    if (w >= nwin) return;
-    g2_jac p = W[(size_t)w * stride];
-    g2_jac_to_hom(hom + 6 * w, p);
-}
-__global__ void k_msm_horner_finish_g2(const fp *hom, g2_jac *out_jac, g2_aff *out_aff) {
-    if (blockIdx.x != 0 || threadIdx.x != 0) return;
-    fp2 X, Y, Z;
-    X.c0 = hom[0]; X.c1 = hom[1]; Y.c0 = hom[2]; Y.c1 = hom[3]; Z.c0 = hom[4]; Z.c1 = hom[5];
-    if (out_jac) {
-        g2_jac j;
-        if (fp2_is_zero(Z)) pt_set_inf(j);
-        else { fp2 z2; fp2_mul(j.x, X, Z); fp2_sqr(z2, Z); fp2_mul(j.y, Y, z2); j.z = Z; }
-        *out_jac = j;
-    }
-    if (out_aff) {
-        g2_aff a;
-        fp2 zi;
-        fp2_inv_vartime(zi, Z);
-        fp2_mul(a.x, X, zi);
-        fp2_mul(a.y, Y, zi);
+        aff_t<F> a;
+        pt_hom_to_affine(a, (const F *)hom);
         *out_aff = a;
     }
 }
@@ -504,14 +463,10 @@ static inline int msm_run(msm_state &st, const route::msm_plan &p,
             m = half;
         }
         if (p.horner_prog && horner_prog) {                  // p.horner_prog: G == 1
-            constexpr bool is_g1 = std::is_same<F, fp>::value;
-            constexpr int per = is_g1 ? 3 : 6;               // field elements per homogeneous point
-            fp *hom = (fp *)(st.buf + o.hom);
-            if constexpr (is_g1) k_msm_horner_prep<<<1, 128, 0, ts>>>(sg, nseg, nwin, hom);
-            else k_msm_horner_prep_g2<<<1, 128, 0, ts>>>(sg, nseg, nwin, hom);
-            horner_prog(ts, hom, hom + per * nwin);
-            if constexpr (is_g1) k_msm_horner_finish<<<1, 32, 0, ts>>>(hom + per * nwin, d_out_jac, d_out_aff);
-            else k_msm_horner_finish_g2<<<1, 32, 0, ts>>>(hom + per * nwin, d_out_jac, d_out_aff);
+            fp *hom = (fp *)(st.buf + o.hom), *res = (fp *)((F *)hom + 3 * nwin);
+            k_msm_horner_prep<F><<<1, 128, 0, ts>>>(sg, nseg, nwin, hom);
+            horner_prog(ts, hom, res);
+            k_msm_horner_finish<F><<<1, 32, 0, ts>>>(res, d_out_jac, d_out_aff);
             nl += 2;                                         // horner_prog counts its own launch
         } else {
             k_msm_horner<F><<<1, 32, 0, ts>>>(sg, nseg, wg, c, g == 0, g == G - 1, carry, d_out_jac, d_out_aff);
