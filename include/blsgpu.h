@@ -11,6 +11,8 @@
  *     = blst_p1_affine (2 x 48 B) | 32 B message | blst_p2_affine (4 x 48 B) = 320 bytes, no padding;
  *     every Fp is 6 x u64 little-endian limbs in Montgomery form    vendor/blst/bindings/blst.h:63,:170,:197
  *   affine infinity = all-zero bytes.
+ *   Compressed set (blsgpu_batch_verify_compressed) = the same with the signature as its 96-byte Zcash encoding
+ *     (bls_sig_io.nim:20-36): 224 bytes, no padding.
  *   GT output = 576 bytes as blst_bendian_from_fp12 writes them     vendor/blst/src/fp12_tower.c:773-786
  *
  * Return convention for verification calls: 1 = valid, 0 = invalid (same booleans as the reference,
@@ -80,6 +82,19 @@ int blsgpu_rlc_scalars(blsgpu_ctx *ctx, const uint8_t srb[32], size_t n, uint32_
  */
 int blsgpu_batch_verify(blsgpu_ctx *ctx, const void *sets, size_t n, const uint8_t srb[32], uint32_t chunks,
                         const uint64_t *scalars, uint8_t gt_out[576]);
+
+#define BLSGPU_COMPRESSED_SET_BYTES 224
+/* Replaces Signature.fromBytes (bls_sig_io.nim:42-60) + batchVerify for sets whose signature is still the 96-byte Zcash
+ * compressed encoding that arrives from the network: a record is blst_p1_affine (96 B) | 32 B message | compressed
+ * signature (96 B), no padding.  Each signature is decoded and subgroup-checked on the device, inside the batch pipeline
+ * (the decode ahead of the signature sum, the subgroup check beside it).  status (nullable) receives n BLST_ERROR codes
+ * (0 success, 1 bad encoding, 2 not on curve, 3 not in group), as blsgpu_signatures_from_bytes with group_check = 1; the
+ * infinite signature (0xc0 0 ... 0) decodes with status 0 and contributes nothing, as in blsgpu_batch_verify.
+ * Returns 1 / 0 / < 0 as blsgpu_batch_verify.  Any status != 0 makes the result 0 with an all-zero GT.  Otherwise the
+ * verdict and the GT equal blsgpu_batch_verify on the decoded 320-byte sets with the same srb / chunks / scalars.
+ * On a multi-device context every share decodes its own slice; status is indexed over the whole batch. */
+int blsgpu_batch_verify_compressed(blsgpu_ctx *ctx, const void *sets224, size_t n, const uint8_t srb[32],
+                                   uint32_t chunks, const uint64_t *scalars, uint8_t gt_out[576], uint8_t *status);
 
 /* Same with the sets already resident in device memory (d_sets: device pointer, n x 320 bytes). */
 int blsgpu_batch_verify_dev(blsgpu_ctx *ctx, const void *d_sets, size_t n, const uint8_t srb[32],

@@ -9,7 +9,7 @@ plus the companion G1 MSM.  All arithmetic runs in hand-written sm_100a CUDA ker
 """
 from ._lib import BlsGpuError, LIB_PATH, lib  # noqa: F401
 from .batch_verifier import (  # noqa: F401
-    BatchedBLSVerifierCache, MultiSignatureSet, SignatureSet, Taskpool, aggregateAll, combine, batchVerify, batchVerifyParallel,
+    BatchedBLSVerifierCache, MultiSignatureSet, SignatureSet, SignatureSetCompressed, Taskpool, batchVerifyCompressed, aggregateAll, combine, batchVerify, batchVerifyParallel,
     batchVerifySerial, hashToG2, msmG1, msmG2, rlcScalars, aggregateVerify, verify, fastAggregateVerify, aggregateAllSegments, subtractAll,
     publicKeysFromBytes, signaturesFromBytes, publicKeysToBytes, signaturesToBytes,
 )

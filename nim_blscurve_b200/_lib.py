@@ -12,7 +12,7 @@ LIB_PATH = os.environ.get("BLSGPU_LIB") or os.path.join(_HERE, "libblsgpu.so")  
 # every symbol include/blsgpu.h declares (tests check the export list against the header)
 SYMBOLS = [
     "blsgpu_device_count", "blsgpu_create", "blsgpu_create_multi", "blsgpu_device_span", "blsgpu_destroy", "blsgpu_last_error", "blsgpu_capacity",
-    "blsgpu_set_stream", "blsgpu_rlc_scalars", "blsgpu_batch_verify", "blsgpu_batch_verify_dev",
+    "blsgpu_set_stream", "blsgpu_rlc_scalars", "blsgpu_batch_verify", "blsgpu_batch_verify_compressed", "blsgpu_batch_verify_dev",
     "blsgpu_partial", "blsgpu_partial_dev", "blsgpu_finalize", "blsgpu_finalize_dev", "blsgpu_hash_to_g2", "blsgpu_aggregate_g1", "blsgpu_aggregate_g2",
     "blsgpu_msm_g1", "blsgpu_msm_g1_dev", "blsgpu_msm_g2", "blsgpu_msm_g2_dev", "blsgpu_combine", "blsgpu_last_stage_ms", "blsgpu_stage_name", "blsgpu_last_launches",
     "blsgpu_subtract_g1", "blsgpu_subtract_g2", "blsgpu_aggregate_g1_segments", "blsgpu_aggregate_verify", "blsgpu_fast_aggregate_verify",
@@ -50,6 +50,7 @@ def lib():
     L.blsgpu_set_stream.argtypes = [vp, vp]
     L.blsgpu_rlc_scalars.argtypes = [vp, u8p, sz, C.c_uint32, vp]
     L.blsgpu_batch_verify.argtypes = [vp, vp, sz, u8p, C.c_uint32, vp, vp]
+    L.blsgpu_batch_verify_compressed.argtypes = [vp, vp, sz, u8p, C.c_uint32, vp, vp, vp]
     L.blsgpu_batch_verify_dev.argtypes = [vp, vp, sz, u8p, C.c_uint32, vp, vp]
     L.blsgpu_partial.argtypes = [vp, vp, C.c_int, sz, sz, sz, u8p, C.c_uint32, vp, vp, vp]
     L.blsgpu_finalize.argtypes = [vp, vp, sz, vp]

@@ -8,6 +8,8 @@ Names, argument meaning and error behaviour follow the reference:
   * batchVerifyParallel(tp, cache, input, secureRandomBytes)           :296-397
   * batchVerify(tp, cache, input, secureRandomBytes)                   :420-495  (parallel iff
     tp.numThreads > 1 and len >= 3, :440, :468)
+  * batchVerifyCompressed(tp, cache, input, secureRandomBytes)         Signature.fromBytes (bls_sig_io.nim:42-60) of
+    every SignatureSetCompressed + batchVerify, decoded and subgroup-checked on the device -> (bool, status)
   * aggregateAll(elems) -> (ok, point)                                 blst_min_pubkey_sig_core.nim:179-195
   * subtractAll(dst, elems) -> point                                   blst_min_pubkey_sig_core.nim:197-209
 The Taskpool argument stays in the signatures; it no longer fans work out to threads — its
@@ -26,6 +28,17 @@ class SignatureSet(NamedTuple):
 
     def to_bytes(self) -> bytes:
         assert len(self.pubkey) == 96 and len(self.message) == 32 and len(self.signature) == 192
+        return self.pubkey + self.message + self.signature
+
+
+class SignatureSetCompressed(NamedTuple):
+    """A set as it comes off the network: the signature still in its 96-byte Zcash compressed encoding."""
+    pubkey: bytes     # 96 B blst_p1_affine
+    message: bytes    # 32 B
+    signature: bytes  # 96 B compressed (bls_sig_io.nim:20-36)
+
+    def to_bytes(self) -> bytes:
+        assert len(self.pubkey) == 96 and len(self.message) == 32 and len(self.signature) == 96
         return self.pubkey + self.message + self.signature
 
 
@@ -49,6 +62,15 @@ def _pack(sets) -> bytes:
         assert len(b) % 320 == 0
         return b
     return b"".join(s.to_bytes() if isinstance(s, SignatureSet) else SignatureSet(*s).to_bytes() for s in sets)
+
+
+def _pack_compressed(sets) -> bytes:
+    if isinstance(sets, (bytes, bytearray, memoryview)):
+        b = bytes(sets)
+        assert len(b) % 224 == 0
+        return b
+    return b"".join(s.to_bytes() if isinstance(s, SignatureSetCompressed) else SignatureSetCompressed(*s).to_bytes()
+                    for s in sets)
 
 
 class BatchedBLSVerifierCache:
@@ -115,6 +137,30 @@ class BatchedBLSVerifierCache:
         if rc < 0:
             raise BlsGpuError(f"blsgpu_batch_verify failed ({rc}): {self.last_error()}")
         return (bool(rc), bytes(gt)) if want_gt else bool(rc)
+
+    def verify_compressed_raw(self, sets: bytes, srb: bytes, chunks: int, scalars: Optional[Sequence[int]] = None,
+                              want_gt: bool = False):
+        """224-byte compressed sets -> (ok, [BLST_ERROR per set]) or (ok, status, gt)."""
+        n = len(sets) // 224
+        self._ensure(n)
+        gt = (C.c_uint8 * 576)() if want_gt else None
+        sc = (C.c_uint64 * n)(*scalars) if scalars is not None else None
+        st = (C.c_uint8 * n)()
+        rc = lib().blsgpu_batch_verify_compressed(self._h, sets, n, srb, chunks, sc, gt, st)
+        if rc < 0:
+            raise BlsGpuError(f"blsgpu_batch_verify_compressed failed ({rc}): {self.last_error()}")
+        return (bool(rc), list(st), bytes(gt)) if want_gt else (bool(rc), list(st))
+
+
+def batchVerifyCompressed(tp: Taskpool, cache: BatchedBLSVerifierCache, input, secureRandomBytes: bytes):
+    """Signature.fromBytes of every signature (decode + subgroup check, on the device) + batchVerify in one call:
+    (verdict, [BLST_ERROR per set]).  A set whose signature fails to decode or is outside G2 fails the batch.  Scalar
+    chunking as batchVerify (parallel derivation iff tp.numThreads > 1 and len >= 3); empty input is (False, [])."""
+    sets = _pack_compressed(input)
+    n = len(sets) // 224
+    if n == 0:
+        return False, []
+    return cache.verify_compressed_raw(sets, secureRandomBytes, max(1, tp.numThreads) if tp.numThreads > 1 and n >= 3 else 0)
 
 
 def batchVerifySerial(cache: BatchedBLSVerifierCache, input, secureRandomBytes: bytes) -> bool:

@@ -58,6 +58,17 @@ static cudaError_t miller_ws_alloc(miller_ws &ws) {
 
 enum { H2D_SLICES = 4 };
 
+// Staging of blsgpu_batch_verify_compressed, allocated for the context's capacity by its first call (comp_alloc)
+struct comp_ws {
+    uint8_t *recs = nullptr;      // the 224-byte records as they came from the host
+    g2_aff *sig = nullptr;        // decoded signatures (all-zero where decoding failed)
+    uint8_t *status = nullptr;    // BLST_ERROR per set
+    fp *check = nullptr;          // small route: subgroup-check program inputs, outputs (6 Fp per set) and the bits of |z|
+    uint8_t *h_status = nullptr;  // pinned: the statuses on their way to the caller
+    cudaStream_t stream = nullptr;                         // the subgroup check, beside the signature sum
+    cudaEvent_t decoded = nullptr, checked = nullptr;
+};
+
 struct blsgpu_ctx {
     int device = 0;
     size_t cap = 0;
@@ -111,6 +122,11 @@ struct blsgpu_ctx {
     const uint8_t *h_src = nullptr;                          // caller's host buffer for the current call (borrowed)
     cudaStream_t copy_stream = nullptr, slice_stream[H2D_SLICES] = {};
     cudaEvent_t ev_copy[H2D_SLICES] = {}, ev_slice[H2D_SLICES] = {};
+    cudaEvent_t ev_spread[H2D_SLICES] = {};                  // compressed sets: keys and messages of slice k in d_sets
+    // the current call's sets are compressed records (blsgpu_batch_verify_compressed): h_src and comp.recs hold 224-byte
+    // records, run_partial_impl spreads their keys and messages into d_sets and decodes and checks the signatures
+    bool comp_call = false;
+    comp_ws comp;
     bool chain_smem_raised = false;                          // k_rlc_scalars allowed to reserve a whole SM's shared memory
     // multi-device context (blsgpu_create_multi): this context is the leader (share 0 + the one final exponentiation),
     // peers[k-1] owns share k on its own device; the 576-byte partials and the flags are gathered into the leader
@@ -120,10 +136,10 @@ struct blsgpu_ctx {
     cudaEvent_t ev_share = nullptr;                          // "this share's partial is ready" (recorded on the share's stream)
     size_t multi_cap = 0;                                    // capacity of the whole multi-device context (leader only)
     // CUDA graphs for the small-batch route: a block-sized batch is ~35 launches on three streams, i.e. ~40 driver calls
-    // per batch from the host thread; the second call with the same (sets pointer, n, chunks) captures the whole
+    // per batch from the host thread; the second call with the same (sets pointer, n, chunks, input format) captures the whole
     // sequence (fork / join included) and every later one replays it with ONE launch.  The 32 random bytes reach the
     // scalar kernel through device memory (d_srb), refreshed by a copy node from a fixed pinned address.
-    struct graph_entry { const void *sets; size_t n; uint32_t chunks; int seen; cudaGraphExec_t exec; };
+    struct graph_entry { const void *sets; size_t n; uint32_t chunks; bool comp; int seen; cudaGraphExec_t exec; };
     std::vector<graph_entry> graphs;
     bool use_graph = true;
     bool srb_from_dev = false;                               // launch_scalars: read the random bytes from d_srb
@@ -182,8 +198,9 @@ static void destroy_slices(blsgpu_ctx *ctx) {
         if (ctx->slice_stream[k]) cudaStreamDestroy(ctx->slice_stream[k]);
         if (ctx->ev_copy[k]) cudaEventDestroy(ctx->ev_copy[k]);
         if (ctx->ev_slice[k]) cudaEventDestroy(ctx->ev_slice[k]);
+        if (ctx->ev_spread[k]) cudaEventDestroy(ctx->ev_spread[k]);
         ctx->slice_stream[k] = nullptr;
-        ctx->ev_copy[k] = ctx->ev_slice[k] = nullptr;
+        ctx->ev_copy[k] = ctx->ev_slice[k] = ctx->ev_spread[k] = nullptr;
     }
 }
 
@@ -194,8 +211,33 @@ static cudaError_t create_slices(blsgpu_ctx *ctx) {
         e = cudaStreamCreateWithFlags(&ctx->slice_stream[k], cudaStreamNonBlocking);
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_copy[k], cudaEventDisableTiming);
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_slice[k], cudaEventDisableTiming);
+        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_spread[k], cudaEventDisableTiming);
     }
     if (e != cudaSuccess) destroy_slices(ctx);
+    return e;
+}
+
+static void comp_free(comp_ws &w) {
+    cudaFree(w.recs); cudaFree(w.sig); cudaFree(w.status); cudaFree(w.check);
+    if (w.h_status) cudaFreeHost(w.h_status);
+    if (w.stream) cudaStreamDestroy(w.stream);
+    if (w.decoded) cudaEventDestroy(w.decoded);
+    if (w.checked) cudaEventDestroy(w.checked);
+    w = comp_ws();
+}
+
+// the compressed-set staging for `cap` sets; all or none: on failure w is left empty
+static cudaError_t comp_alloc(comp_ws &w, size_t cap) {
+    const size_t nchk = cap < route::SMALL_ROUTE_CAP ? cap : route::SMALL_ROUTE_CAP;
+    cudaError_t e = cudaMalloc((void **)&w.recs, cap * BLSGPU_COMPRESSED_SET_BYTES);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&w.sig, cap * sizeof(g2_aff));
+    if (e == cudaSuccess) e = cudaMalloc((void **)&w.status, cap);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&w.check, (12 * nchk + 64) * sizeof(fp));
+    if (e == cudaSuccess) e = cudaMallocHost((void **)&w.h_status, cap);
+    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&w.stream, cudaStreamNonBlocking);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&w.decoded, cudaEventDisableTiming);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&w.checked, cudaEventDisableTiming);
+    if (e != cudaSuccess) comp_free(w);
     return e;
 }
 
@@ -210,6 +252,7 @@ extern "C" void blsgpu_destroy(blsgpu_ctx *ctx) {
     for (auto &g : ctx->graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
     if (ctx->ev_share) cudaEventDestroy(ctx->ev_share);
     destroy_slices(ctx);
+    comp_free(ctx->comp);
     if (ctx->ev_scratch_valid) for (int i = 0; i < 8; i++) cudaEventDestroy(ctx->ev_scratch[i]);
     cudaFree(ctx->d_sets); cudaFree(ctx->d_r); cudaFree(ctx->d_H); cudaFree(ctx->d_Pj); cudaFree(ctx->d_Q);
     cudaFree(ctx->d_P); cudaFree(ctx->d_S); cudaFree(ctx->d_partials); cudaFree(ctx->d_gtb);
@@ -656,6 +699,7 @@ static int run_partial(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, size_t f
         cudaStreamSynchronize(ctx->chain);
         cudaStreamSynchronize(ctx->side);
         cudaStreamSynchronize(ctx->side2);
+        if (ctx->comp.stream) cudaStreamSynchronize(ctx->comp.stream);
         if (ctx->copy_stream) {
             cudaStreamSynchronize(ctx->copy_stream);
             for (int k = 0; k < H2D_SLICES; k++) cudaStreamSynchronize(ctx->slice_stream[k]);
@@ -684,7 +728,17 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
     // the hash kernel over that piece on its own stream, so the copy (and, for pageable memory, the host-side staging
     // that blocks the calling thread piece by piece) hides behind H(m_i) of the earlier pieces.
     const bool sliced = plan.sliced;
-    if (ctx->h_src && !sliced) CK(cudaMemcpyAsync(ctx->d_sets, ctx->h_src, n * sizeof(sigset), cudaMemcpyHostToDevice, s));
+    // Compressed sets: the records land in comp.recs (copied here, or ahead of the call by the caller); their keys and
+    // messages are spread into d_sets ahead of the hash (per slice when the copy is sliced), their signatures are decoded
+    // on the signature side stream and subgroup-checked on a stream of their own (below)
+    const bool comp = ctx->comp_call;
+    const size_t rec = comp ? BLSGPU_COMPRESSED_SET_BYTES : sizeof(sigset);
+    uint8_t *d_recs = comp ? ctx->comp.recs : (uint8_t *)ctx->d_sets;
+    if (ctx->h_src && !sliced) CK(cudaMemcpyAsync(d_recs, ctx->h_src, n * rec, cudaMemcpyHostToDevice, s));
+    if (comp && !sliced) {
+        k_comp_spread<<<nblk(8 * n), 128, 0, s>>>(ctx->comp.recs, n, ctx->d_sets);
+        ctx->launches++;
+    }
     if (sliced && !ctx->copy_stream) CK(create_slices(ctx));
     CK(cudaMemsetAsync(ctx->d_flags, 0, 4 * sizeof(int), s));
     // fork: the scalar chain (strictly sequential SHA-256 per reference chunk: tens of milliseconds for a large batch
@@ -700,10 +754,7 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
     int rc = launch_scalars(ctx, srb, n, first, total_n, chunks, scalars, plan.chain_hog, cs);
     if (rc) return rc;
     END(ST_SCALARS, cs);
-    if (ctx->use_side) {
-        CK(cudaEventRecord(ctx->ev[EV_SC], cs));
-        CK(cudaStreamWaitEvent(g, ctx->ev[EV_SC], 0));
-    }
+    if (ctx->use_side) CK(cudaEventRecord(ctx->ev[EV_SC], cs));   // the signature side waits for it below
     if (plan.chain_wait) {
         // the main stream (whose next kernel fills the machine) waits until the chains' block is placed: ~10 us when the
         // device is idle, at most 0.2 ms (400 000 cycles) when it is not
@@ -725,14 +776,23 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
         const size_t per = ((n + H2D_SLICES - 1) / H2D_SLICES + 127) & ~(size_t)127;      // whole thread blocks per piece
         for (int k = 0; k < H2D_SLICES; k++) {
             const size_t off = (size_t)k * per;
-            if (off >= n) { CK(cudaEventRecord(ctx->ev_copy[k], ctx->copy_stream)); CK(cudaEventRecord(ctx->ev_slice[k], ctx->copy_stream)); continue; }
+            if (off >= n) {
+                CK(cudaEventRecord(ctx->ev_copy[k], ctx->copy_stream));
+                CK(cudaEventRecord(ctx->ev_slice[k], ctx->copy_stream));
+                if (comp) CK(cudaEventRecord(ctx->ev_spread[k], ctx->copy_stream));
+                continue;
+            }
             const size_t len = n - off < per ? n - off : per;
             if (k == 0) CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev[EV_FORK], 0));     // after whatever preceded on s
-            CK(cudaMemcpyAsync(ctx->d_sets + off, ctx->h_src + off * sizeof(sigset), len * sizeof(sigset), cudaMemcpyHostToDevice,
-                               ctx->copy_stream));
+            CK(cudaMemcpyAsync(d_recs + off * rec, ctx->h_src + off * rec, len * rec, cudaMemcpyHostToDevice, ctx->copy_stream));
             CK(cudaEventRecord(ctx->ev_copy[k], ctx->copy_stream));
             cudaStream_t sk = ctx->slice_stream[k];
             CK(cudaStreamWaitEvent(sk, ctx->ev_copy[k], 0));
+            if (comp) {
+                k_comp_spread<<<nblk(8 * len), 128, 0, sk>>>(ctx->comp.recs + off * rec, len, ctx->d_sets + off);
+                ctx->launches++;
+                CK(cudaEventRecord(ctx->ev_spread[k], sk));
+            }
             if (plan.hash == route::HASH_LANES2) k_hash_sets_lanes2<<<nblk(2 * len), 128, 0, sk>>>(d_sets + off, len, ctx->d_H + off);
             else k_hash_sets<<<nblk(len), 128, 0, sk>>>(d_sets + off, len, ctx->d_H + off);
             ctx->launches++;
@@ -740,17 +800,47 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
         }
         for (int k = 0; k < H2D_SLICES; k++) CK(cudaStreamWaitEvent(s, ctx->ev_slice[k], 0));
         END(ST_HASH, s);
-        CK(cudaStreamWaitEvent(g, ctx->ev_copy[H2D_SLICES - 1], 0));    // the signature-side MSM reads every set
+        CK(cudaStreamWaitEvent(g, ctx->ev_copy[H2D_SLICES - 1], 0));    // the signature side reads every set
     }
     if (plan.g1_aside) {
         cudaStream_t g1s = ctx->side2;
         CK(cudaStreamWaitEvent(g1s, ctx->ev[EV_SC], 0));
-        if (sliced) CK(cudaStreamWaitEvent(g1s, ctx->ev_copy[H2D_SLICES - 1], 0));   // the keys of every slice are in place
+        if (sliced && comp) {                                            // the keys of every slice are in place
+            for (int k = 0; k < H2D_SLICES; k++) CK(cudaStreamWaitEvent(g1s, ctx->ev_spread[k], 0));
+        } else if (sliced) {
+            CK(cudaStreamWaitEvent(g1s, ctx->ev_copy[H2D_SLICES - 1], 0));
+        }
         BEGIN(ST_G1MUL, g1s);
         k_g1_mul<<<nblk(n), 128, 0, g1s>>>(d_sets, ctx->d_r, n, ctx->d_Pj, ctx->d_flags);
         END(ST_G1MUL, g1s);
         CK(cudaEventRecord(ctx->ev[EV_G1], g1s));
     }
+    // Compressed sets: decode the signatures on the signature side stream ahead of the scalars, which the decode does not
+    // need; the subgroup check gates only the verdict, so it runs on a stream of its own beside the signature sum and the
+    // main stream waits for it only before the partial is complete (end of this function).  Small batches run it as the
+    // per-set [|z|]P program, one warp per set; larger ones a thread per set.
+    if (comp) {
+        k_sig_decode<<<nblk(n), 128, 0, g>>>(ctx->comp.recs, n, ctx->comp.sig, ctx->comp.status, ctx->d_flags);
+        ctx->launches++;
+        CK(cudaEventRecord(ctx->comp.decoded, g));
+        cudaStream_t ks = ctx->comp.stream;
+        CK(cudaStreamWaitEvent(ks, ctx->comp.decoded, 0));
+        if (plan.small) {
+            fp *hom_in = ctx->comp.check, *hom_out = hom_in + 6 * n, *zbits = hom_out + 6 * n;
+            k_sig_check_prep<<<nblk(n), 128, 0, ks>>>(ctx->comp.sig, n, hom_in, zbits);
+            launch_prog_many(ctx, p_mul, ks, n, hom_in, 6, zbits, 0, hom_out, 6);
+            k_sig_check_cmp<<<nblk(n), 128, 0, ks>>>(ctx->comp.sig, hom_out, n, ctx->comp.status, ctx->d_flags);
+            ctx->launches += 2;
+        } else {
+            k_sig_subgroup<<<nblk(n), 128, 0, ks>>>(ctx->comp.sig, n, ctx->comp.status, ctx->d_flags);
+            ctx->launches++;
+        }
+        CK(cudaEventRecord(ctx->comp.checked, ks));
+    }
+    if (ctx->use_side) CK(cudaStreamWaitEvent(g, ctx->ev[EV_SC], 0));
+    // the signatures S sums: in place in the 320-byte sets, or decoded from compressed ones
+    const uint8_t *sigs = comp ? (const uint8_t *)ctx->comp.sig : (const uint8_t *)d_sets + offsetof(sigset, sig);
+    const size_t sstride = comp ? sizeof(g2_aff) : sizeof(sigset);
     // H(m_i) on the main stream (already launched piece by piece when the host copy is sliced)
     auto launch_hash = [&]() -> int {
         if (sliced) return 0;
@@ -775,19 +865,18 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
     BEGIN(ST_G2MUL, g);
     // S = sum_i [r_i] sig_i
     if (plan.sig == route::SIG_MSM) {
-        rc = run_msm<fp2>(ctx, (const uint8_t *)d_sets + offsetof(sigset, sig), sizeof(sigset), (const uint8_t *)ctx->d_r, 8, n, 64,
-                          g, ctx->d_S, nullptr);
+        rc = run_msm<fp2>(ctx, sigs, sstride, (const uint8_t *)ctx->d_r, 8, n, 64, g, ctx->d_S, nullptr);
         if (rc) return rc;
         END(ST_G2MUL, g);
         BEGIN(ST_G2SUM, g);
     } else {
         if (plan.sig == route::SIG_PROGRAM) {
-            k_g2_mul_prep<<<nblk(64 * n), 128, 0, g>>>(d_sets, ctx->d_r, n, sb.sig_in, sb.bits);
+            k_g2_mul_prep<<<nblk(64 * n), 128, 0, g>>>(sigs, sstride, ctx->d_r, n, sb.sig_in, sb.bits);
             launch_prog_many(ctx, p_mul, g, n, sb.sig_in, 6, sb.bits, 64, sb.sig_out, 6);
             k_g2_hom_to_jac<<<nblk(n), 128, 0, g>>>(sb.sig_out, n, ctx->d_S);
             ctx->launches += 2;
         } else {
-            k_g2_mul<<<nblk(n), 128, 0, g>>>(d_sets, ctx->d_r, n, ctx->d_S);
+            k_g2_mul<<<nblk(n), 128, 0, g>>>(sigs, sstride, ctx->d_r, n, ctx->d_S);
             ctx->launches++;
         }
         END(ST_G2MUL, g);
@@ -831,19 +920,22 @@ static int run_partial_impl(blsgpu_ctx *ctx, const sigset *d_sets, size_t n, siz
     ctx->launches += 3;
     if (!plan.defer_sig) {
         if (ctx->use_side) CK(cudaStreamWaitEvent(s, ctx->ev[EV_JOIN], 0));   // join: pair number n is in place
-        return run_miller(ctx, ctx->ml, n + 1, slot);
+        rc = run_miller(ctx, ctx->ml, n + 1, slot);
+        if (rc) return rc;
+    } else {
+        rc = run_miller(ctx, ctx->ml, n, slot);              // the n set pairs; (S, -G1) is being done on the side stream
+        if (rc) return rc;
+        CK(cudaStreamWaitEvent(s, ctx->ev[EV_JOIN], 0));
+        blsgpu_ctx::dev_prog p2;
+        rc = get_prog(ctx, PROG_PRODUCT, 2, p2, s);
+        if (rc) return rc;
+        // in place: the program loads all 24 inputs into its slot file before the first round and stores at the end
+        rc = launch_prog(ctx, p2, s, (const fp *)(ctx->d_partials + slot), (fp *)(ctx->d_partials + slot));
+        if (rc) return rc;
+        END(ST_PARTIAL, s);
+        CK(cudaGetLastError());
     }
-    rc = run_miller(ctx, ctx->ml, n, slot);                  // the n set pairs; (S, -G1) is being done on the side stream
-    if (rc) return rc;
-    CK(cudaStreamWaitEvent(s, ctx->ev[EV_JOIN], 0));
-    blsgpu_ctx::dev_prog p2;
-    rc = get_prog(ctx, PROG_PRODUCT, 2, p2, s);
-    if (rc) return rc;
-    // in place: the program loads all 24 inputs into its slot file before the first round and stores at the end
-    rc = launch_prog(ctx, p2, s, (const fp *)(ctx->d_partials + slot), (fp *)(ctx->d_partials + slot));
-    if (rc) return rc;
-    END(ST_PARTIAL, s);
-    CK(cudaGetLastError());
+    if (comp) CK(cudaStreamWaitEvent(s, ctx->comp.checked, 0));   // its verdict is in d_flags[0] before anyone reads it
     return 0;
 }
 
@@ -963,13 +1055,14 @@ extern "C" int blsgpu_rlc_scalars(blsgpu_ctx *ctx, const uint8_t srb[32], size_t
 static int verify_graphed(blsgpu_ctx *ctx, const void *d_sets, size_t n, const uint8_t srb[32], uint32_t chunks, bool &done) {
     done = false;
     blsgpu_ctx::graph_entry *e = nullptr;
-    for (auto &g : ctx->graphs) if (g.sets == d_sets && g.n == n && g.chunks == chunks) { e = &g; break; }
+    for (auto &g : ctx->graphs)
+        if (g.sets == d_sets && g.n == n && g.chunks == chunks && g.comp == ctx->comp_call) { e = &g; break; }
     if (!e) {
         if (ctx->graphs.size() >= 16) {                      // bounded cache: drop the oldest entry
             if (ctx->graphs.front().exec) cudaGraphExecDestroy(ctx->graphs.front().exec);
             ctx->graphs.erase(ctx->graphs.begin());
         }
-        ctx->graphs.push_back({d_sets, n, chunks, 1, nullptr});
+        ctx->graphs.push_back({d_sets, n, chunks, ctx->comp_call, 1, nullptr});
         return 0;
     }
     const words8 w = words_of(srb);
@@ -1044,13 +1137,15 @@ static void share_range(size_t total, size_t parts, size_t k, size_t &first, siz
 // caller's buffer on that device's stream), every device leaves its 576-byte partial + flag in its own memory, the
 // leader's stream waits for each share's event and pulls them over NVLink (cudaMemcpyPeerAsync), then runs the one final
 // exponentiation.  Scalars come from the GLOBAL (n, chunks) derivation, so verdict and GT equal the one-device result.
+// comp: the sets are 224-byte compressed records (blsgpu_batch_verify_compressed); every share decodes and checks its own
+// slice, and status (nullable) receives the statuses of all shares at their global indices.
 static int batch_verify_multi(blsgpu_ctx *lead, const uint8_t *sets, size_t n, const uint8_t srb[32], uint32_t chunks,
-                              const uint64_t *scalars, uint8_t gt_out[576]) {
+                              const uint64_t *scalars, uint8_t gt_out[576], bool comp = false, uint8_t *status = nullptr) {
     blsgpu_ctx *ctx = lead;                                  // CK() reports into the leader
     std::vector<blsgpu_ctx *> all;
     all.push_back(lead);
     for (blsgpu_ctx *p : lead->peers) all.push_back(p);
-    const size_t ndev = all.size();
+    const size_t ndev = all.size(), rec = comp ? BLSGPU_COMPRESSED_SET_BYTES : sizeof(sigset);
     int rc = 0, total_launches = 0;
     size_t issued = 0;
     for (size_t k = 0; k < ndev && rc == 0; k++) {
@@ -1064,10 +1159,16 @@ static int batch_verify_multi(blsgpu_ctx *lead, const uint8_t *sets, size_t n, c
             k_partial_one<<<1, 32, 0, c->stream>>>(c->d_partials, c->d_flags);
             c->launches = 1;
         } else {
-            e = cudaMemcpyAsync(c->d_sets, sets + first * sizeof(sigset), len * sizeof(sigset), cudaMemcpyHostToDevice, c->stream);
+            uint8_t *dst = comp ? c->comp.recs : (uint8_t *)c->d_sets;
+            e = cudaMemcpyAsync(dst, sets + first * rec, len * rec, cudaMemcpyHostToDevice, c->stream);
             if (e != cudaSuccess) { rc = fail(lead, BLSGPU_ERR_CUDA, "cudaMemcpyAsync(share)", e); break; }
+            c->comp_call = comp;
             rc = run_partial(c, c->d_sets, len, first, n, srb, chunks, scalars ? scalars + first : nullptr, 0);
+            c->comp_call = false;
             if (rc && c != lead) lead->err = c->err;
+            if (rc == 0 && comp && status &&
+                (e = cudaMemcpyAsync(c->comp.h_status, c->comp.status, len, cudaMemcpyDeviceToHost, c->stream)) != cudaSuccess)
+                rc = fail(lead, BLSGPU_ERR_CUDA, "cudaMemcpyAsync(share status)", e);
         }
         total_launches += c->launches;
         if (rc == 0 && (e = cudaEventRecord(c->ev_share, c->stream)) != cudaSuccess) rc = fail(lead, BLSGPU_ERR_CUDA, "cudaEventRecord", e);
@@ -1088,8 +1189,16 @@ static int batch_verify_multi(blsgpu_ctx *lead, const uint8_t *sets, size_t n, c
     rc = run_final(lead, (int)ndev, gt_out, &bad, lead->d_gather, lead->d_gather_flags);
     lead->launches = total_launches + lead->launches;
     collect_stage_times(lead, true);
-    // the H2D copies of the other devices read the caller's buffer: they are complete (their partials were consumed)
+    // the H2D copies of the other devices read the caller's buffer: they are complete (their partials were consumed), and
+    // so are the status copies queued ahead of each share's event
     if (rc < 0) return rc;
+    if (comp && status) {
+        for (size_t k = 0; k < ndev; k++) {
+            size_t first, len;
+            share_range(n, ndev, k, first, len);
+            if (len) memcpy(status + first, all[k]->comp.h_status, len);
+        }
+    }
     if (bad) { if (gt_out) memset(gt_out, 0, 576); return 0; }
     return rc;
 }
@@ -1115,6 +1224,66 @@ extern "C" int blsgpu_batch_verify(blsgpu_ctx *ctx, const void *sets, size_t n, 
     ctx->h_src = (const uint8_t *)sets;                      // run_partial_impl issues the copy (whole, or in overlapped pieces)
     int rc = blsgpu_batch_verify_dev(ctx, ctx->d_sets, n, srb, chunks, scalars, gt_out);
     ctx->h_src = nullptr;
+    return rc;
+}
+
+// One device: the records are copied ahead of the pipeline and small batches replay a captured graph (keyed apart from
+// the 320-byte format), or run_partial_impl issues the copy itself; the statuses come back after the graph or the
+// pipeline on the same stream, fresh on every call.
+static int batch_verify_compressed_one(blsgpu_ctx *ctx, const void *sets224, size_t n, const uint8_t srb[32], uint32_t chunks,
+                                       const uint64_t *scalars, uint8_t gt_out[576], uint8_t *status) {
+    cudaStream_t s = ctx->stream;
+    const route::batch_plan plan = batch_plan_of(ctx, n, n, chunks, true, scalars != nullptr);
+    bool done = false;
+    int rc = 0;
+    if (plan.copy_ahead) {
+        CK(cudaMemcpyAsync(ctx->comp.recs, sets224, n * BLSGPU_COMPRESSED_SET_BYTES, cudaMemcpyHostToDevice, s));
+        if (srb && plan.graph) rc = verify_graphed(ctx, ctx->d_sets, n, srb, chunks, done);
+    } else {
+        ctx->h_src = (const uint8_t *)sets224;
+    }
+    if (!rc && !done) {
+        rc = run_partial(ctx, ctx->d_sets, n, 0, n, srb, chunks, scalars, 0);
+        if (!rc) rc = run_final_enqueue(ctx, 1);
+    }
+    ctx->h_src = nullptr;
+    if (rc) return rc;
+    if (status) CK(cudaMemcpyAsync(ctx->comp.h_status, ctx->comp.status, n, cudaMemcpyDeviceToHost, s));
+    int pk_inf = 0;
+    rc = run_final_finish(ctx, gt_out, &pk_inf, false);
+    if (done) for (int i = 0; i < ST_COUNT; i++) ctx->stage_ms[i] = 0.f;     // no event timing inside a graph
+    else collect_stage_times(ctx, true);
+    if (rc < 0) return rc;
+    if (status) memcpy(status, ctx->comp.h_status, n);
+    if (pk_inf) { if (gt_out) memset(gt_out, 0, 576); return 0; }           // a bad signature, or an infinite key
+    return rc;
+}
+
+extern "C" int blsgpu_batch_verify_compressed(blsgpu_ctx *ctx, const void *sets224, size_t n, const uint8_t srb[32],
+                                              uint32_t chunks, const uint64_t *scalars, uint8_t gt_out[576], uint8_t *status) {
+    if (!ctx) return BLSGPU_ERR_ARG;
+    if (gt_out) memset(gt_out, 0, 576);
+    if (n == 0) return 0;
+    if (!sets224) return fail(ctx, BLSGPU_ERR_ARG, "sets is NULL");
+    if (n > blsgpu_capacity(ctx)) return fail(ctx, BLSGPU_ERR_CAPACITY, "batch larger than context capacity");
+    // argument errors are reported before any copy is queued: no transfer from the caller's buffer outlives the call
+    if (!scalars && !srb) return fail(ctx, BLSGPU_ERR_ARG, "secureRandomBytes is NULL");
+    if (scalars)
+        for (size_t i = 0; i < n; i++) if (scalars[i] == 0) return fail(ctx, BLSGPU_ERR_ARG, "explicit RLC scalar is zero");
+    // the staging of every share, on the first such call
+    std::vector<blsgpu_ctx *> all(1, ctx);
+    for (blsgpu_ctx *p : ctx->peers) all.push_back(p);
+    for (blsgpu_ctx *c : all) {
+        if (c->comp.recs) continue;
+        cudaError_t e = cudaSetDevice(c->device);
+        if (e == cudaSuccess) e = comp_alloc(c->comp, c->cap);
+        if (e != cudaSuccess) { cudaSetDevice(ctx->device); return fail(ctx, BLSGPU_ERR_CUDA, "compressed-set staging", e); }
+    }
+    if (!ctx->peers.empty()) return batch_verify_multi(ctx, (const uint8_t *)sets224, n, srb, chunks, scalars, gt_out, true, status);
+    CK(cudaSetDevice(ctx->device));
+    ctx->comp_call = true;
+    int rc = batch_verify_compressed_one(ctx, sets224, n, srb, chunks, scalars, gt_out, status);
+    ctx->comp_call = false;
     return rc;
 }
 

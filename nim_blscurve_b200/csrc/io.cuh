@@ -108,16 +108,23 @@ BLS_NOINLINE bool g1_in_subgroup(const g1_aff &p) {
     return pt_eq_affine(t, bx, ny);
 }
 
+// psi(P) == -T for the finite affine P and T = [|z|]P computed by the caller
+BLS_FN bool g2_psi_is_neg(const g2_aff &p, const g2_jac &t) {
+    g2_jac q;
+    pt_from_affine(q, p);
+    g2_psi(q, q);                      // affine in, Z stays 1
+    fp2 ny;
+    fp2_neg(ny, q.y);
+    return pt_eq_affine(t, q.x, ny);
+}
+
 // P in G2  <=>  psi(P) == [z]P = -[|z|]P
 BLS_NOINLINE bool g2_in_subgroup(const g2_aff &p) {
     if (aff_is_inf(p)) return true;
     g2_jac t, q;
     pt_from_affine(q, p);
     pt_mul_by_zabs(t, q);
-    g2_psi(q, q);                      // affine in, Z stays 1
-    fp2 ny;
-    fp2_neg(ny, q.y);
-    return pt_eq_affine(t, q.x, ny);
+    return g2_psi_is_neg(p, t);
 }
 
 // one compressed G1 point (48 bytes, flags already inspected by the caller: compressed, not infinity)

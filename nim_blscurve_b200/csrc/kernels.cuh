@@ -331,9 +331,15 @@ __global__ void k_g2_hom_to_jac(const fp *hom, size_t n, g2_jac *out) {
     pt_hom_to_jac(j, (const fp2 *)hom + 3 * i);
     out[i] = j;
 }
+// signature i of an array of affine signatures `sstride` bytes apart: the sig field of the 320-byte sets, or the
+// decoded signatures of compressed sets
+__device__ __forceinline__ const g2_aff &sig_at(const uint8_t *sigs, size_t sstride, size_t i) {
+    return *(const g2_aff *)(sigs + i * sstride);
+}
+
 // inputs of the [r_i] sig_i program (build_g2_mul64): the signature as (x : y : 1) (infinity (0 : 1 : 0)) and the 64
 // scalar bits as field elements 0 / 1
-__global__ void k_g2_mul_prep(const sigset *sets, const uint64_t *r, size_t n, fp *hom, fp *bits) {
+__global__ void k_g2_mul_prep(const uint8_t *sigs, size_t sstride, const uint64_t *r, size_t n, fp *hom, fp *bits) {
     const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     const size_t i = t >> 6;
     const int b = (int)(t & 63);
@@ -342,7 +348,7 @@ __global__ void k_g2_mul_prep(const sigset *sets, const uint64_t *r, size_t n, f
     if ((r[i] >> b) & 1) v = FP_ONE; else fp_set_zero(v);
     bits[64 * i + b] = v;
     if (b == 0) {
-        g2_aff a = sets[i].sig;
+        g2_aff a = sig_at(sigs, sstride, i);
         g2_jac j;
         pt_from_affine(j, a);
         pt_jac_to_hom((fp2 *)hom + 3 * i, j);
@@ -460,10 +466,10 @@ __global__ void BLS_LB k_pairs_affine(const g2_jac *H, const g1_jac *Pj, size_t 
     }
 }
 
-__global__ void BLS_LB k_g2_mul(const sigset *sets, const uint64_t *r, size_t n, g2_jac *S) {
+__global__ void BLS_LB k_g2_mul(const uint8_t *sigs, size_t sstride, const uint64_t *r, size_t n, g2_jac *S) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    g2_aff sig = sets[i].sig;
+    g2_aff sig = sig_at(sigs, sstride, i);
     g2_jac j;
     pt_mul_u64(j, sig, r[i]);                           // infinite signature contributes nothing (aggregate.c:261)
     S[i] = j;
@@ -1003,6 +1009,81 @@ __global__ void BLS_LB k_pt_from_bytes(const uint8_t *in, size_t n, int len, int
     status[i] = (uint8_t)err;
     if (err) atomicAdd(nfail, 1);
 }
+// ---- batch verification of compressed sets (blsgpu_batch_verify_compressed) ----
+// A record is blst_p1_affine (96 B) | 32 B message | Zcash-compressed signature (96 B), no padding.
+enum { COMP_SIG_OFF = 128 };
+static_assert(BLSGPU_COMPRESSED_SET_BYTES == COMP_SIG_OFF + 96 && BLSGPU_COMPRESSED_SET_BYTES % 16 == 0, "compressed set layout");
+
+// public key and message of every record into the 320-byte set that the hash and [r_i]pk_i read: 16 bytes per thread
+__global__ void k_comp_spread(const uint8_t *comp, size_t n, sigset *sets) {
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x, i = t >> 3;
+    if (i >= n) return;
+    const int w = (int)(t & 7);
+    ((uint4 *)(sets + i))[w] = ((const uint4 *)(comp + i * BLSGPU_COMPRESSED_SET_BYTES))[w];
+}
+
+// The signature of every record decoded (blst_p2_uncompress; the subgroup check runs apart, beside the signature sum):
+// the affine point, all-zero on failure (skipped by the sum like an infinite signature), its BLST_ERROR in status, and
+// flags[0] raised on failure, which fails the batch as an infinite public key does.
+__global__ void BLS_LB k_sig_decode(const uint8_t *comp, size_t n, g2_aff *sig, uint8_t *status, int *flags) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    uint4 raw[6];
+    const uint4 *src = (const uint4 *)(comp + i * BLSGPU_COMPRESSED_SET_BYTES + COMP_SIG_OFF);
+#pragma unroll
+    for (int k = 0; k < 6; k++) raw[k] = src[k];
+    g2_aff p;
+    const int err = g2_from_bytes(p, (const uint8_t *)raw, 96);
+    if (err != IO_SUCCESS) {
+        fp2_set_zero(p.x);
+        fp2_set_zero(p.y);
+        atomicOr(flags, 1);
+    }
+    sig[i] = p;
+    status[i] = (uint8_t)err;
+}
+
+// The subgroup check of the decoded signatures, a thread per set: status 3 and flags[0] for a signature outside G2
+__global__ void BLS_LB k_sig_subgroup(const g2_aff *sig, size_t n, uint8_t *status, int *flags) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n || status[i] != IO_SUCCESS) return;
+    const g2_aff p = sig[i];
+    if (!g2_in_subgroup(p)) {
+        status[i] = IO_NOT_IN_GROUP;
+        atomicOr(flags, 1);
+    }
+}
+
+// The same check as the per-set program build_g2_mul64 with the constant scalar |z| (small batches, where one thread
+// per set would run the 63 dependent doublings at lone-thread latency).  Inputs: the signature as (x : y : 1) (infinity
+// (0 : 1 : 0)), and the 64 bits of |z| as field elements 0 / 1, one copy that every set reads (stride 0).
+__global__ void k_sig_check_prep(const g2_aff *sig, size_t n, fp *hom, fp *zbits) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < 64) {
+        fp v;
+        if ((BLS_Z_ABS >> i) & 1) v = FP_ONE; else fp_set_zero(v);
+        zbits[i] = v;
+    }
+    if (i >= n) return;
+    const g2_aff a = sig[i];
+    g2_jac j;
+    pt_from_affine(j, a);
+    pt_jac_to_hom((fp2 *)hom + 3 * i, j);
+}
+// hom: [|z|]P from the program; P is in G2 iff psi(P) == -[|z|]P
+__global__ void k_sig_check_cmp(const g2_aff *sig, const fp *hom, size_t n, uint8_t *status, int *flags) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n || status[i] != IO_SUCCESS) return;
+    const g2_aff p = sig[i];
+    if (aff_is_inf(p)) return;
+    g2_jac t;
+    pt_hom_to_jac(t, (const fp2 *)hom + 3 * i);
+    if (!g2_psi_is_neg(p, t)) {
+        status[i] = IO_NOT_IN_GROUP;
+        atomicOr(flags, 1);
+    }
+}
+
 // Zcash compressed encoding: sizeof(F) bytes per point
 template <class F>
 __global__ void k_pt_compress(const aff_t<F> *in, size_t n, uint8_t *out) {

@@ -31,6 +31,9 @@ const
 type
   SignatureSet* = tuple[pubkey: PublicKey, message: array[32, byte], signature: Signature]
 
+  SignatureSetCompressed* = tuple[pubkey: PublicKey, message: array[32, byte], signature: array[96, byte]]
+    ## a set as it comes off the network: the signature still in its Zcash compressed encoding (bls_sig_io.nim:20-36)
+
   MultiSignatureSet* = object                                # bls_batch_verifier.nim:47-62
     pubkeys: seq[PublicKey]
     message: array[32, byte]
@@ -42,6 +45,7 @@ type
     numThreads: int
 
 static: doAssert sizeof(SignatureSet) == 320   # pk 96 | msg 32 | sig 192, no padding
+static: doAssert sizeof(SignatureSetCompressed) == 224   # pk 96 | msg 32 | compressed sig 96, no padding
 
 # ---- context lifetime --------------------------------------------------------------------------------------
 proc createCtx(maxSets: int): BlsGpuCtx =
@@ -192,6 +196,24 @@ when compileOption("threads"):
       tp.batchVerifyParallel(input, secureRandomBytes)
     else:
       batchVerifySerial(input, secureRandomBytes)
+
+  # ---- Signature.fromBytes (bls_sig_io.nim:42-60) of every set + batchVerify, decoded and checked on the device -----
+  proc batchVerifyCompressed*(
+        tp: Taskpool,
+        cache: var BatchedBLSVerifierCache,
+        input: openArray[SignatureSetCompressed],
+        secureRandomBytes: array[32, byte],
+        status: var openArray[byte]
+      ): bool =
+    ## status[i] receives the BLST_ERROR of signature i (0 success, 1 bad encoding, 2 not on curve, 3 not in group);
+    ## any failure makes the batch false.  Scalar chunking as batchVerify (:420-495).
+    doAssert status.len == input.len
+    if input.len == 0: return false
+    ensureCapacity(cache.ctx, input.len)
+    let chunks = if tp.numThreads > 1 and input.len >= 3: uint32 tp.numThreads else: 0'u32
+    check(cache.ctx, blsgpu_batch_verify_compressed(cache.ctx, unsafeAddr input[0], input.len.csize_t,
+                                                    unsafeAddr secureRandomBytes, chunks, nil, nil, addr status[0]),
+          "blsgpu_batch_verify_compressed")
 
 # ---- MultiSignatureSet (:73-106) --------------------------------------------------------------------------
 func init*(

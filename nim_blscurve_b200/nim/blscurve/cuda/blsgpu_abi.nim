@@ -24,6 +24,9 @@ proc blsgpu_rlc_scalars*(ctx: BlsGpuCtx, srb: ptr array[32, byte], n: csize_t, c
                          dst: ptr uint64): cint
 proc blsgpu_batch_verify*(ctx: BlsGpuCtx, sets: pointer, n: csize_t, srb: ptr array[32, byte],
                           chunks: uint32, scalars: ptr uint64, gtOut: ptr array[576, byte]): cint
+proc blsgpu_batch_verify_compressed*(ctx: BlsGpuCtx, sets: pointer, n: csize_t, srb: ptr array[32, byte],
+                                     chunks: uint32, scalars: ptr uint64, gtOut: ptr array[576, byte],
+                                     status: ptr byte): cint
 proc blsgpu_batch_verify_dev*(ctx: BlsGpuCtx, dSets: pointer, n: csize_t, srb: ptr array[32, byte],
                               chunks: uint32, scalars: ptr uint64, gtOut: ptr array[576, byte]): cint
 proc blsgpu_partial*(ctx: BlsGpuCtx, sets: pointer, setsOnDevice: cint, n, first, totalN: csize_t,
